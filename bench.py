@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo (CUDA, sm_100a)
     python bench.py --impl reference --gpus N --steps K ...  # CPU arm: the oracle port on host cores
+    python bench.py ... --dump-outputs DIR                   # + the last timed step's outputs as DIR/<name>.npy
 
 Workload (config.workload): the FSTR command line of the reference's README.md:63 (BASELINE
 configs[1] knobs) driven with synthetic U(-1,1)^2 actions, env-step only, ``--num-envs`` envs per
@@ -198,6 +199,26 @@ def timed_steps(env, lib, pool, steps, use_graph):
     return launch, s, start, end
 
 
+def dump_outputs(env, out_dir, max_bytes=64e6):
+    """Write what a caller of ``env.step()`` receives after the last timed step -- clamped observations, rewards, resets
+    and time-outs -- as float32 ``<out_dir>/<name>.npy``, one row per env, with the env ids of the rows in ``env_ids.npy``
+    (float64).  Above ``max_bytes`` in all, the rows are a fixed seeded sample of the envs, so that two builds run with
+    the same arguments can be compared output for output."""
+    import numpy as np
+    import torch
+    arrays = {"obs": env._obs_clamped, "rew": env.rew_buf, "reset": env.reset_buf, "time_outs": env.timeout_buf}
+    n = env.num_envs
+    row_bytes = 4 * sum(a[0].numel() for a in arrays.values()) + 8
+    ids = np.arange(n)
+    if n * row_bytes > max_bytes - 4096:              # 4096: room for the .npy headers
+        ids = np.sort(np.random.default_rng(0).choice(n, int((max_bytes - 4096) // row_bytes), replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    rows = torch.from_numpy(ids).to(env.device)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a[rows].float().cpu().numpy())
+    np.save(os.path.join(out_dir, "env_ids.npy"), (ids + env._global_env_offset).astype(np.float64))
+
+
 def run_ours(args, rank, world, local_rank):
     import numpy as np
     import torch
@@ -259,6 +280,8 @@ def run_ours(args, rank, world, local_rank):
     sampler.start()
     env, cfg, ms, window = measure(n, args.steps, args.warmup)
     clocks = sampler.summary(*window)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(env, args.dump_outputs)           # before the e2e steps below advance the same env
     value = n * world * args.steps / (ms * 1e-3)
     ms_per_step = ms / args.steps
 
@@ -555,7 +578,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-ppo", action="store_true")
     ap.add_argument("--ppo-iters", type=int, default=20)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step (rank 0's envs) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to the CUDA arm (--impl ours)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -1,9 +1,10 @@
-"""Generate the golden fixtures in tests/golden/*.npz by EXECUTING THE REFERENCE.
+"""Generate the golden fixtures in tests/golden/ by EXECUTING THE REFERENCE.
 
 Run in the build container only (needs /root/reference):
     python tests/golden/generate_golden.py
 
-Two families:
+Fixtures:
+  reference_cfg.json    the reference's cfg/ YAML files, composed and resolved (compose(cfg_dir=...))
   step_<scenario>.npz   whole ``VecTask.step`` rollouts of the reference's unmodified task under
                         ref_harness.FakeGym (dynamics = oracle f64, RNG = product Philox streams)
   fn_<name>.npz         single calls of the reference's own functions on synthetic inputs:
@@ -275,7 +276,22 @@ def gen_fn_pre_and_actuation(name, overrides, n=256, T=6, seed=11):
     print("fn_pre_act_%-12s T=%d |efforts|max=%.3g" % (name, T, float(np.abs(out["dof_efforts"]).max())))
 
 
+REFERENCE_CFG_UNCOMPARED = ("wandb_entity", "wandb_project", "wandb_group", "wandb_name", "wandb_tags", "wandb_logcode_dir")
+
+
+def gen_reference_cfg():
+    """reference_cfg.json: the reference's own cfg/ YAML files (config.yaml + task + train), composed and resolved, minus the
+    author's wandb settings."""
+    cfg = vcfg.compose(["task=Vine5LinkMovingBase", "train=Vine5LinkMovingBasePPO"],
+                       cfg_dir=os.path.join(H.REF_ROOT, "isaacgymenvs", "cfg"))
+    cfg = {k: v for k, v in cfg.items() if k not in REFERENCE_CFG_UNCOMPARED}
+    with open(os.path.join(HERE, "reference_cfg.json"), "w") as f:
+        json.dump(cfg, f, indent=1, sort_keys=True)
+        f.write("\n")
+
+
 def main():
+    gen_reference_cfg()
     for name, (ov, n, T, mode) in STEP_SCENARIOS.items():
         gen_step(name, ov, n, T, mode)
     gen_fn_post_physics("default28", NO_OBST)

@@ -5,6 +5,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -28,9 +29,37 @@ def test_reference_arm_line():
     assert "workload" in d["config"] and d["gpu_launches"] == 0
 
 
+def test_dump_outputs_above_the_cap_is_a_fixed_sample_of_envs(tmp_path):
+    import types
+
+    import torch
+    import bench
+    n, cap = 1000, 4096 + 100 * (4 * 21 + 8)          # room for the .npy headers + 100 rows of 18 obs, rew, reset, time-out, id
+    env = types.SimpleNamespace(num_envs=n, device="cpu", _global_env_offset=5000,
+                                _obs_clamped=torch.arange(n * 18, dtype=torch.float32).reshape(n, 18),
+                                rew_buf=torch.arange(n, dtype=torch.float32), reset_buf=torch.arange(n) % 2,
+                                timeout_buf=torch.arange(n) % 3 == 0)
+    for d in ("a", "b"):
+        bench.dump_outputs(env, str(tmp_path / d), max_bytes=cap)
+    names = ("obs", "rew", "reset", "time_outs", "env_ids")
+    a, b = ({k: np.load(tmp_path / d / f"{k}.npy") for k in names} for d in ("a", "b"))
+    assert all(np.array_equal(a[k], b[k]) for k in names) and sum(f.stat().st_size for f in (tmp_path / "a").iterdir()) <= cap
+    rows = a["rew"].astype(np.int64)
+    assert len(rows) == 100 and np.all(np.diff(rows) > 0) and np.array_equal(a["env_ids"], rows + 5000)
+    assert np.array_equal(a["obs"], env._obs_clamped.numpy()[rows]) and np.array_equal(a["reset"], rows % 2)
+    assert np.array_equal(a["time_outs"], rows % 3 == 0) and all(v.dtype in (np.float32, np.float64) for v in a.values())
+
+
 @pytest.mark.gpu
-def test_cuda_arm_line():
-    d = run_bench("--steps", "5", "--warmup", "3", "--no-sweep", "--ppo-iters", "3", "--num-envs", "65536", "--e2e-steps", "3")
+def test_cuda_arm_line(tmp_path):
+    d = run_bench("--steps", "5", "--warmup", "3", "--no-sweep", "--ppo-iters", "3", "--num-envs", "65536", "--e2e-steps", "3",
+                  "--dump-outputs", str(tmp_path))
+    # the outputs of the last timed step, every env (65,536 x 84 B is under the 64 MB cap, so no sampling)
+    out = {k: np.load(tmp_path / f"{k}.npy") for k in ("obs", "rew", "reset", "time_outs", "env_ids")}
+    assert out["obs"].shape == (65536, 18) and all(out[k].shape == (65536,) for k in ("rew", "reset", "time_outs", "env_ids"))
+    assert all(a.dtype in (np.float32, np.float64) and np.isfinite(a).all() for a in out.values())
+    assert np.array_equal(out["env_ids"], np.arange(65536)) and np.abs(out["obs"]).max() <= 5.0 and out["obs"].std() > 0
+    assert set(np.unique(out["reset"])) <= {0.0, 1.0} and set(np.unique(out["time_outs"])) <= {0.0, 1.0}
     assert BASE | {"roofline", "clocks", "gpu_launches", "ppo", "ppo_frames_per_s"} <= set(d)
     assert d["n_gpus"] == 1 and d["steps"] == 5 and d["warmup"] >= 3 and d["gpu_launches"] == 5 and d["scaling"] == "weak"
     assert d["value"] > 1e8 and d["e2e"]["value"] > 1e7 and d["e2e"]["h2d_bytes_per_step"] == 65536 * 8

@@ -8,7 +8,8 @@ rl-games 1.5.2's published structure (``ModelBuilder.load -> network.build(confi
 sub-modules ``a2c_network`` / ``running_mean_std`` / ``value_mean_std``; ``torch_ext.load_checkpoint``; ``torch_runner._restore``).
 The stub network is built ONLY from the pickled config and restores with a strict ``load_state_dict``: a missing, surplus or
 mis-shaped key in our file fails the test.  Its forward is plain torch (no code of this repo), and its deterministic action
-must equal ``player.PolicyPlayer``'s on the same file.  Runs only where /root/reference exists (the build container).
+must equal ``player.PolicyPlayer``'s on the same file.  The script's part runs only where the reference checkout exists; the
+stub network restoring our checkpoint from the pickled config alone runs everywhere.
 """
 import ast
 import os
@@ -22,7 +23,6 @@ import torch
 import torch.nn as nn
 
 REF = "/root/reference/isaacgymenvs/vine_robot_test_model.py"
-pytestmark = pytest.mark.skipif(not os.path.exists(REF), reason="needs the reference checkout (build container only)")
 
 
 # ---------------------------------------------------------------- stand-ins for the three rl_games names the script imports
@@ -116,10 +116,9 @@ def _reference_classes(n_obs, n_actions):
     return ns
 
 
-@pytest.mark.parametrize("rnn", [True, False], ids=["reference_network", "mlp_only"])
-def test_reference_deployment_script_restores_and_runs_our_checkpoint(tmp_path, rnn):
+def _write_checkpoint(tmp_path, rnn):
+    """A checkpoint + run config written by this trainer's code -> (path of the pickled config, path of the .pth)."""
     from vine_robot_isaacgymenvs_b200 import config as vcfg
-    from vine_robot_isaacgymenvs_b200.player import PolicyPlayer
     from vine_robot_isaacgymenvs_b200.ppo.ppo import ActorCritic, RunningMeanStd, rlgames_model_state
     from vine_robot_isaacgymenvs_b200.train import write_run_config
     cfg = vcfg.compose(vcfg.FSTR_OVERRIDES + ([] if rnn else ["train.params.network.rnn=null"]) + ["rl_device=cpu"])
@@ -140,7 +139,38 @@ def test_reference_deployment_script_restores_and_runs_our_checkpoint(tmp_path, 
     os.makedirs(exp_dir / "nn", exist_ok=True)
     path = str(exp_dir / "nn" / "last_Vine5LinkMovingBase_ep_7_rew_1.pth")
     torch.save(ckpt, path)
+    return pkl, path
 
+
+@pytest.mark.parametrize("rnn", [True, False], ids=["reference_network", "mlp_only"])
+def test_rl_games_network_built_from_the_pickled_config_restores_and_runs_our_checkpoint(tmp_path, rnn):
+    """What rl_games' player does with the two files, minus the script: network from the pickled config, strict load, act."""
+    from vine_robot_isaacgymenvs_b200.player import PolicyPlayer
+    pkl, path = _write_checkpoint(tmp_path, rnn)
+    O, A = 18, 2
+    with open(pkl, "rb") as f:
+        params = pickle.load(f)["params"]
+    model = _Model(params, {"actions_num": A, "input_shape": (O,), "normalize_input": params["config"]["normalize_input"],
+                            "normalize_value": params["config"]["normalize_value"], "value_size": 1})
+    model.load_state_dict(torch.load(path, map_location="cpu")["model"])     # strict
+    model.eval()
+    ours = PolicyPlayer(O, device="cpu").restore(path)
+    torch.manual_seed(0)
+    states = None
+    with torch.no_grad():
+        for step in range(5):                                    # the LSTM state is carried across calls in both
+            obs = torch.randn(1, O) * 2
+            out = model({"obs": obs, "rnn_states": states})
+            states = out["rnn_states"]
+            assert torch.allclose(torch.clamp(out["mus"], -1.0, 1.0), ours.get_action(obs, is_deterministic=True), atol=1e-5), step
+
+
+@pytest.mark.skipif(not os.path.exists(REF), reason="needs the reference checkout")
+@pytest.mark.parametrize("rnn", [True, False], ids=["reference_network", "mlp_only"])
+def test_reference_deployment_script_restores_and_runs_our_checkpoint(tmp_path, rnn):
+    from vine_robot_isaacgymenvs_b200.player import PolicyPlayer
+    pkl, path = _write_checkpoint(tmp_path, rnn)
+    O, A = 18, 2
     ns = _reference_classes(O, A)
     control = ns["VineRobotControlModel"](pkl, path, x_range=(-10.0, 10.0), u_range=(-0.1, 3.0))   # strict load_state_dict inside
     player = control.rl_games_player
