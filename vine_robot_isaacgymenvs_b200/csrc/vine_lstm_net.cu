@@ -932,18 +932,28 @@ __global__ void vine_lstm_adam_kernel(const float* __restrict__ flat, float scal
     state[2] = st4[2] * scale;
     state[3] = 1.f;
   }
-  if (p < PL) {
-  const float lr = state[0], step = state[1];
-  const float g = (ch ? s_g[threadIdx.x] : flat[p]) * scale;
-  const float mn = beta1 * m[p] + (1.f - beta1) * g;
-  const float vn = beta2 * v[p] + (1.f - beta2) * g * g;
-  m[p] = mn;
-  v[p] = vn;
-  const float bc1 = 1.f - powf(beta1, step), bc2 = 1.f - powf(beta2, step);
-  const float w_old = params[p];
-  const float w = w_old - (lr / bc1) * mn / (sqrtf(vn) / sqrtf(bc2) + eps);
-  params[p] = w;
   const LstmSeg sg = lstm_segments(O);
+  // b_hh[tr] is updated by the thread of b_ih[tr] (below), so that one thread writes the packed sum b_ih + b_hh
+  if (p < PL && !(p >= sg.bhh && p < sg.lng)) {
+  const float lr = state[0], step = state[1];
+  const float bc1 = 1.f - powf(beta1, step), bc2 = 1.f - powf(beta2, step);
+  auto adam = [&](float g, float& mq, float& vq, float& wq) {
+    mq = beta1 * mq + (1.f - beta1) * g;
+    vq = beta2 * vq + (1.f - beta2) * g * g;
+    wq = wq - (lr / bc1) * mq / (sqrtf(vq) / sqrtf(bc2) + eps);
+  };
+  const bool bias = p >= sg.bih && p < sg.bhh;
+  const int q = p + GATES;   // bias: b_hh of the same gate row
+  const float g = (ch ? s_g[threadIdx.x] : flat[p]) * scale;
+  float mp = m[p], vp = v[p], w = params[p], g2 = 0.f, mq = 0.f, vq = 0.f, w_hh = 0.f;
+  if (bias) {   // the partner's operands are loaded with the thread's own: these blocks run last, one memory round trip
+    g2 = (ch ? p2p_sum(ch, seq, q) : flat[q]) * scale;
+    mq = m[q], vq = v[q], w_hh = params[q];
+  }
+  adam(g, mp, vp, w);
+  m[p] = mp;
+  v[p] = vp;
+  params[p] = w;
   if (p < sg.whh) {
     const int tr = p / (H3 + O), c = p % (H3 + O), R = packed_gate_row(tr);
     *reinterpret_cast<__nv_bfloat16*>(packed + LP_WIH + (R / PIECE_ROWS) * PIECE_BYTES + tile_offset(R % PIECE_ROWS, c, UK)) = __float2bfloat16_rn(w);
@@ -951,10 +961,15 @@ __global__ void vine_lstm_adam_kernel(const float* __restrict__ flat, float scal
     const int q = p - sg.whh, tr = q / HID, c = q % HID, R = packed_gate_row(tr);
     *reinterpret_cast<__nv_bfloat16*>(packed + LP_WHH + ((c / UK) * NPIECE + R / PIECE_ROWS) * PIECE_BYTES + tile_offset(R % PIECE_ROWS, c % UK, UK)) =
         __float2bfloat16_rn(w);
-  } else if (p < sg.lng) {
-    // the kernels use b_ih + b_hh: each of the two parameters adds its own update to the packed sum
-    const int tr = (p - sg.bih) % GATES;
-    atomicAdd(reinterpret_cast<float*>(packed + LP_BIAS) + packed_gate_row(tr), w - w_old);
+  } else if (bias) {
+    // the kernels use b_ih + b_hh: this thread also updates b_hh[tr] and stores the sum as vine_lstm_pack computes it, so the
+    // packed bias is fl(b_ih + b_hh) of the new parameters and the same bits on every run and every rank (the partner's
+    // gradient is summed over the ranks in the same order as p2p_sum_block)
+    adam(g2, mq, vq, w_hh);
+    m[q] = mq;
+    v[q] = vq;
+    params[q] = w_hh;
+    reinterpret_cast<float*>(packed + LP_BIAS)[packed_gate_row(p - sg.bih)] = w + w_hh;
   }
   if (p >= sg.lng) {
     float* f32 = nullptr;
