@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define VINE_ABI_VERSION 2
+#define VINE_ABI_VERSION 3
 
 #define VINE_NUM_DOFS 6          /* 1 prismatic rail cart + 5 revolute links (V5:54,83) */
 #define VINE_NUM_ACTIONS 2       /* u_rail_velocity, u_fpam (V5:171) */
@@ -653,6 +653,10 @@ int vine_lstm_reduce(const float* workspace, int splits, float* head_grads, int 
                      void* p2p_channel, void* stream);
 int vine_lstm_adam(const float* flat, float grad_scale, float* params, float* exp_avg, float* exp_avg_sq, void* packed,
                    float* state, int num_obs, float beta1, float beta2, float eps, void* p2p_channel, void* stream);
+/* the same with the gradient-clipping coefficient clip_coef (device, NULL = none), see vine_grad_clip */
+int vine_lstm_adam_clipped(const float* flat, float grad_scale, float* params, float* exp_avg, float* exp_avg_sq, void* packed,
+                           float* state, int num_obs, float beta1, float beta2, float eps, const float* clip_coef,
+                           void* p2p_channel, void* stream);
 
 /*
  * Pointwise half of the LSTM layer of the reference's network (Vine5LinkMovingBasePPO.yaml:32-38; rl_games
@@ -685,7 +689,8 @@ int vine_lstm_cell_bwd(const void* acts_bf16, const float* c_prev, const float* 
  * done by the caller once per iteration), obs is raw and normalised inside like vine_mlp_forward.
  *
  * state (device, >= 16 floats): [0] learning rate, [1] Adam step count, [2] KL of the last minibatch,
- * [3] "KL pending" flag, [4..7] running sums of a_loss, c_loss, kl, b_loss, [8] minibatches summed.
+ * [3] "KL pending" flag, [4..7] running sums of a_loss, c_loss, kl, b_loss, [8] minibatches summed,
+ * [9] gradient-clipping coefficient and [10] gradient norm of the last vine_grad_clip call (untouched without clipping).
  * With adaptive_lr the `legacy` schedule of rl_games (lr /= 1.5 if kl > 2 kl_threshold, lr *= 1.5 if
  * kl < kl_threshold / 2, clamped to [lr_min, lr_max]) is applied on the device between optimiser steps:
  * no host synchronisation anywhere, the whole update is CUDA-graph capturable.
@@ -730,6 +735,28 @@ int vine_ppo_reduce(const float* workspace, int n_partials, int num_obs, float* 
 int vine_ppo_adam(const float* flat, float grad_scale, float* params, float* exp_avg, float* exp_avg_sq,
                   void* packed, float* state, int num_obs, float beta1, float beta2, float eps, int bookkeeping,
                   void* p2p_channel, void* stream);
+/* the same with g = flat * grad_scale * clip_coef[0]: clip_coef (device, NULL = no clipping) is the coefficient
+ * vine_grad_clip writes to state + 9 */
+int vine_ppo_adam_clipped(const float* flat, float grad_scale, float* params, float* exp_avg, float* exp_avg_sq,
+                          void* packed, float* state, int num_obs, float beta1, float beta2, float eps, int bookkeeping,
+                          const float* clip_coef, void* p2p_channel, void* stream);
+
+/*
+ * Gradient-norm clipping before Adam (rl_games truncate_grads / grad_norm: torch.nn.utils.clip_grad_norm_ over the model's
+ * parameters).  One or two flat gradient vectors (flat2 = NULL, count2 = length2 = 0 for one); entries [0, count) of each
+ * count towards the norm, all `length` floats (gradient + loss statistics) are carried: with the reference network, flat =
+ * the MLP half with count = vine_ppo_num_params(O) - 197 (its unused head slots excluded), flat2 = the recurrent half with
+ * count2 = vine_lstm_num_params(O); length = count of floats of each vector (P + 4).  With g = flat * grad_scale:
+ *   state[10] = total = sqrt(sum g^2) (f32, fixed summation order: the same bits on every rank holding the same sum),
+ *   state[9]  = min(max_norm / (total + 1e-6), 1) (NaN stays NaN),
+ * which vine_ppo_adam_clipped / vine_lstm_adam_clipped multiply in (pass state + 9).  workspace: device,
+ * VINE_GRAD_CLIP_WS_FLOATS floats, zeroed once before the first call (the kernel leaves it ready for the next one; one
+ * workspace per stream).  Multi-GPU over peer memory, this call is the consumer of the channels (one per vector): it writes
+ * the rank-order sum over the ranks into flat / flat2, and the Adam launches then run without a channel.
+ */
+#define VINE_GRAD_CLIP_WS_FLOATS 1024
+int vine_grad_clip(float* flat, int count, int length, float* flat2, int count2, int length2, float grad_scale,
+                   float max_norm, float* state, float* workspace, void* p2p_channel, void* p2p_channel2, void* stream);
 
 /*
  * Gradient all-reduce over peer memory (multi-GPU PPO; replaces the per-minibatch all-reduce of the flattened gradients the

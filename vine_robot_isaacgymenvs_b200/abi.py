@@ -12,7 +12,7 @@ NUM_ACTIONS = 2
 NUM_REWARDS = 13
 NUM_OBJECT_INFO = 2
 MAX_ACTION_DELAY = 8
-ABI_VERSION = 2
+ABI_VERSION = 3
 
 OK = 0
 ERR_INVALID_ARG = -1
@@ -143,6 +143,7 @@ EXPORTED_SYMBOLS = [
     "vine_policy_act", "vine_rollout_post", "vine_ppo_moments", "vine_ppo_finalize",
     "vine_lstm_cell_fwd", "vine_lstm_cell_bwd", "vine_lstm_pack", "vine_lstm_step", "vine_lstm_mask", "vine_lstm_head", "vine_lstm_head_train", "vine_lstm_cell_bwd_tiles", "vine_lstm_bwd_gemm",
     "vine_set_programmatic_launch", "vine_lstm_gather", "vine_abi_struct_size", "vine_lstm_num_params", "vine_lstm_wgrad", "vine_lstm_reduce", "vine_lstm_adam",
+    "vine_grad_clip", "vine_ppo_adam_clipped", "vine_lstm_adam_clipped",
 ]
 METRIC_SUMS, METRIC_MAXES = 45, 30
 METRIC_SCALARS = ["dist_tip_to_target", "target_reached", "limit_hit", "tip_limit_hit", "abs_tip_y", "tip_z", "tip_velocities",
@@ -156,6 +157,8 @@ LSTM_WGRAD_BLOCK_FLOATS = 12 * 128 * 256      # per K split
 LSTM_TILE_BYTES = 32768          # one [128 x 128] bf16 activation tile
 PPO_WS_FLOATS = 49664
 PPO_STATE_FLOATS = 16
+PPO_STATE_CLIP_COEF, PPO_STATE_GRAD_NORM = 9, 10   # slots of the state block written by vine_grad_clip
+GRAD_CLIP_WS_FLOATS = 1024
 
 
 class VinePolicyAct(C.Structure):
@@ -293,6 +296,9 @@ def _declare(lib):
     lib.vine_ppo_minibatch.argtypes = [C.POINTER(VinePpoMinibatch), vp]
     lib.vine_ppo_reduce.argtypes = [vp, C.c_int, C.c_int, vp, vp, vp, vp, vp]
     lib.vine_ppo_adam.argtypes = [vp, C.c_float, vp, vp, vp, vp, vp, C.c_int, C.c_float, C.c_float, C.c_float, C.c_int, vp, vp]
+    lib.vine_ppo_adam_clipped.argtypes = [vp, C.c_float, vp, vp, vp, vp, vp, C.c_int, C.c_float, C.c_float, C.c_float, C.c_int, vp, vp, vp]
+    lib.vine_lstm_adam_clipped.argtypes = [vp, C.c_float, vp, vp, vp, vp, vp, C.c_int, C.c_float, C.c_float, C.c_float, vp, vp, vp]
+    lib.vine_grad_clip.argtypes = [vp, C.c_int, C.c_int, vp, C.c_int, C.c_int, C.c_float, C.c_float, vp, vp, vp, vp, vp]
     lib.vine_p2p_alloc.argtypes = [C.c_int64, C.POINTER(C.c_void_p), vp]
     lib.vine_p2p_open.argtypes = [vp, C.POINTER(C.c_void_p)]
     lib.vine_p2p_close.argtypes = [vp]

@@ -909,7 +909,7 @@ __global__ void __launch_bounds__(256) vine_lstm_reduce_kernel(const float* __re
 
 __global__ void vine_lstm_adam_kernel(const float* __restrict__ flat, float scale, float* __restrict__ params, float* __restrict__ m,
                                       float* __restrict__ v, uint8_t* __restrict__ packed, float* __restrict__ state, int O, float beta1,
-                                      float beta2, float eps, VineP2PChannel* ch) {
+                                      float beta2, float eps, const float* __restrict__ clip, VineP2PChannel* ch) {
   vine_launch::grid_dependency_sync();
   const int PL = lstm_num_params(O);
   const int p = blockIdx.x * blockDim.x + threadIdx.x;
@@ -944,10 +944,13 @@ __global__ void vine_lstm_adam_kernel(const float* __restrict__ flat, float scal
   };
   const bool bias = p >= sg.bih && p < sg.bhh;
   const int q = p + GATES;   // bias: b_hh of the same gate row
-  const float g = (ch ? s_g[threadIdx.x] : flat[p]) * scale;
+  const float cf = clip ? *clip : 1.f;   // vine_grad_clip's coefficient (exactly 1 below the threshold; g * 1 == g)
+  float g = (ch ? s_g[threadIdx.x] : flat[p]) * scale;
+  if (clip) g *= cf;
   float mp = m[p], vp = v[p], w = params[p], g2 = 0.f, mq = 0.f, vq = 0.f, w_hh = 0.f;
   if (bias) {   // the partner's operands are loaded with the thread's own: these blocks run last, one memory round trip
     g2 = (ch ? p2p_sum(ch, seq, q) : flat[q]) * scale;
+    if (clip) g2 *= cf;
     mq = m[q], vq = v[q], w_hh = params[q];
   }
   adam(g, mp, vp, w);
@@ -1164,13 +1167,19 @@ int vine_lstm_reduce(const float* workspace, int splits, float* head_grads, int 
   return cudaGetLastError() == cudaSuccess ? VINE_OK : VINE_ERR_CUDA;
 }
 
-int vine_lstm_adam(const float* flat, float grad_scale, float* params, float* exp_avg, float* exp_avg_sq, void* packed, float* state,
-                   int num_obs, float beta1, float beta2, float eps, void* p2p_channel, void* stream) {
+int vine_lstm_adam_clipped(const float* flat, float grad_scale, float* params, float* exp_avg, float* exp_avg_sq, void* packed, float* state,
+                           int num_obs, float beta1, float beta2, float eps, const float* clip_coef, void* p2p_channel, void* stream) {
   if ((!flat && !p2p_channel) || !params || !exp_avg || !exp_avg_sq || !packed || !state || num_obs < 1 || num_obs >= K1) return VINE_ERR_INVALID_ARG;
   const int n = lstm_num_params(num_obs) + 1;
   vine_launch::launch(vine_lstm_adam_kernel, (n + 255) / 256, 256, 0, (cudaStream_t)stream, flat, grad_scale, params, exp_avg, exp_avg_sq, (uint8_t*)packed,
-                      state, num_obs, beta1, beta2, eps, (VineP2PChannel*)p2p_channel);
+                      state, num_obs, beta1, beta2, eps, clip_coef, (VineP2PChannel*)p2p_channel);
   return cudaGetLastError() == cudaSuccess ? VINE_OK : VINE_ERR_CUDA;
+}
+
+int vine_lstm_adam(const float* flat, float grad_scale, float* params, float* exp_avg, float* exp_avg_sq, void* packed, float* state,
+                   int num_obs, float beta1, float beta2, float eps, void* p2p_channel, void* stream) {
+  return vine_lstm_adam_clipped(flat, grad_scale, params, exp_avg, exp_avg_sq, packed, state, num_obs, beta1, beta2, eps, nullptr,
+                                p2p_channel, stream);
 }
 
 int vine_lstm_head_train(const VineLstmHeadTrain* a, void* stream) {

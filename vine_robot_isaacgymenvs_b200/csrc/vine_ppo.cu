@@ -451,10 +451,93 @@ __global__ void __launch_bounds__(RED_SLOTS* RED_SPLIT) vine_ppo_reduce_kernel(c
   if (ch) p2p_producer_done(const_cast<VineP2PChannel*>(ch));
 }
 
+// Gradient-norm clipping (torch.nn.utils.clip_grad_norm_ over the whole model) for one or two flat gradient vectors:
+// total = sqrt(sum of (flat[i] * scale)^2 over i < count of each vector), coef = min(max_norm / (total + 1e-6), 1) with a NaN
+// kept (torch's clamp(max=1)), both written to the state block; the Adam kernels multiply the coefficient in.  The sum of
+// squares has a fixed order -- per block a fixed tree, then the last block to finish (self-resetting ticket in the workspace)
+// sums the block partials in a fixed tree -- so every rank that holds the same summed gradient computes the same bits.
+// No block waits for another block of the grid.  Multi-GPU (peer memory), this kernel is the consumer of each channel: it
+// writes the rank-order sum of all `len` floats (gradient + loss statistics) into the local `flat`, which Adam then reads
+// without a channel.
+constexpr int CLIP_THREADS = 256, CLIP_CHUNK = 4 * CLIP_THREADS, CLIP_MAX_BLOCKS = VINE_GRAD_CLIP_WS_FLOATS - 1;
+constexpr int ST_CLIP_COEF = 9, ST_GRAD_NORM = 10;
+struct ClipArgs {
+  float* flat[2];
+  VineP2PChannel* ch[2];
+  int count[2], len[2], chunks0, chunks;   // chunks0 = chunks of vector 0; blocks stride over all chunks of both
+  float scale, max_norm;
+  float *state, *ws;                      // ws[0]: ticket (u32 bits), ws[1 + b]: partial of block b
+};
+
+// deterministic sum over the block (every thread gets the result; CLIP_THREADS / 32 warps added in warp order)
+__device__ __forceinline__ float clip_block_sum(float v, float* red) {
+  v = warp_sum_f(v);
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = v;
+  __syncthreads();
+  float s = 0.f;
+#pragma unroll
+  for (int w = 0; w < CLIP_THREADS / 32; ++w) s += red[w];
+  __syncthreads();   // red is reused
+  return s;
+}
+
+__global__ void __launch_bounds__(CLIP_THREADS) vine_grad_clip_kernel(const ClipArgs a) {
+  vine_launch::grid_dependency_sync();
+  __shared__ __align__(16) float s_g[CLIP_CHUNK];
+  __shared__ float red[CLIP_THREADS / 32];
+  __shared__ int s_last;
+  // vine_ppo_reduce / vine_lstm_reduce have published this rank's flags
+  const unsigned seq0 = a.ch[0] ? p2p_exchange_begin(a.ch[0], false) : 0u, seq1 = a.ch[1] ? p2p_exchange_begin(a.ch[1], false) : 0u;
+  float acc = 0.f;
+  for (int c = blockIdx.x; c < a.chunks; c += gridDim.x) {   // (selects instead of a[v]: no local-memory copy of the arguments)
+    const bool second = c >= a.chunks0;
+    const int base = (second ? c - a.chunks0 : c) * CLIP_CHUNK, n = min(CLIP_CHUNK, (second ? a.len[1] : a.len[0]) - base);
+    const int count = second ? a.count[1] : a.count[0];
+    float* flat = second ? a.flat[1] : a.flat[0];
+    VineP2PChannel* ch = second ? a.ch[1] : a.ch[0];
+    if (ch) p2p_sum_block(ch, second ? seq1 : seq0, base, n, s_g);
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+      const int i = threadIdx.x + k * CLIP_THREADS;
+      if (i < n) {
+        float x;
+        if (ch) flat[base + i] = x = s_g[i];
+        else x = flat[base + i];
+        const float g = x * a.scale;
+        if (base + i < count) acc = fmaf(g, g, acc);
+      }
+    }
+    if (ch) __syncthreads();   // s_g is refilled by the next chunk
+  }
+  if (a.ch[0]) p2p_exchange_end(a.ch[0]);
+  if (a.ch[1]) p2p_exchange_end(a.ch[1]);
+  const float part = clip_block_sum(acc, red);
+  unsigned* ticket = reinterpret_cast<unsigned*>(a.ws);
+  if (threadIdx.x == 0) {
+    a.ws[1 + blockIdx.x] = part;
+    __threadfence();
+    s_last = atomicAdd(ticket, 1u) + 1u == gridDim.x;
+  }
+  __syncthreads();
+  if (!s_last) return;
+  __threadfence();
+  float t = 0.f;
+  for (int b = threadIdx.x; b < (int)gridDim.x; b += CLIP_THREADS) t += __ldcg(a.ws + 1 + b);
+  const float sumsq = clip_block_sum(t, red);
+  if (threadIdx.x == 0) {
+    const float total = sqrtf(sumsq);
+    const float coef = a.max_norm / (total + 1e-6f);
+    a.state[ST_CLIP_COEF] = coef > 1.f ? 1.f : coef;   // NaN stays NaN, as with torch.clamp(max=1.0)
+    a.state[ST_GRAD_NORM] = total;
+    *ticket = 0u;                                      // ready for the next call (and the next replay of a graph)
+  }
+}
+
 // torch.optim.Adam (no weight decay, no amsgrad) on the flat parameter vector + re-pack for the tensor cores
 __global__ void vine_ppo_adam_kernel(const float* __restrict__ flat, float scale, float* __restrict__ params, float* __restrict__ m,
                                      float* __restrict__ v, uint8_t* __restrict__ packed, float* __restrict__ state, int O,
-                                     float beta1, float beta2, float eps, int bookkeeping, VineP2PChannel* ch) {
+                                     float beta1, float beta2, float eps, int bookkeeping, const float* __restrict__ clip,
+                                     VineP2PChannel* ch) {
   vine_launch::grid_dependency_sync();
   const int P = num_params(O);
   const int p = blockIdx.x * blockDim.x + threadIdx.x;
@@ -479,7 +562,8 @@ __global__ void vine_ppo_adam_kernel(const float* __restrict__ flat, float scale
   }
   if (p < P) {
     const float lr = state[ST_LR], step = state[ST_STEP];
-    const float g = (ch ? s_g[threadIdx.x] : flat[p]) * scale;
+    float g = (ch ? s_g[threadIdx.x] : flat[p]) * scale;
+    if (clip) g *= *clip;   // vine_grad_clip's coefficient: exactly 1 when the norm is below max_norm, and g * 1 == g
     const float mn = beta1 * m[p] + (1.f - beta1) * g;
     const float vn = beta2 * v[p] + (1.f - beta2) * g * g;
     m[p] = mn;
@@ -559,13 +643,37 @@ int vine_ppo_reduce(const float* workspace, int n_partials, int num_obs, float* 
   return cudaGetLastError() == cudaSuccess ? VINE_OK : VINE_ERR_CUDA;
 }
 
-int vine_ppo_adam(const float* flat, float grad_scale, float* params, float* exp_avg, float* exp_avg_sq, void* packed,
-                  float* state, int num_obs, float beta1, float beta2, float eps, int bookkeeping, void* p2p_channel, void* stream) {
+int vine_ppo_adam_clipped(const float* flat, float grad_scale, float* params, float* exp_avg, float* exp_avg_sq, void* packed,
+                          float* state, int num_obs, float beta1, float beta2, float eps, int bookkeeping, const float* clip_coef,
+                          void* p2p_channel, void* stream) {
   if ((!flat && !p2p_channel) || !params || !exp_avg || !exp_avg_sq || !packed || !state || num_obs < 1 || num_obs >= K1)
     return VINE_ERR_INVALID_ARG;
   const int n = num_params(num_obs) + 1;
   vine_launch::launch(vine_ppo_adam_kernel, (n + 127) / 128, 128, 0, (cudaStream_t)stream, flat, grad_scale, params, exp_avg, exp_avg_sq,
-                      (uint8_t*)packed, state, num_obs, beta1, beta2, eps, bookkeeping, (VineP2PChannel*)p2p_channel);
+                      (uint8_t*)packed, state, num_obs, beta1, beta2, eps, bookkeeping, clip_coef, (VineP2PChannel*)p2p_channel);
+  return cudaGetLastError() == cudaSuccess ? VINE_OK : VINE_ERR_CUDA;
+}
+
+int vine_ppo_adam(const float* flat, float grad_scale, float* params, float* exp_avg, float* exp_avg_sq, void* packed,
+                  float* state, int num_obs, float beta1, float beta2, float eps, int bookkeeping, void* p2p_channel, void* stream) {
+  return vine_ppo_adam_clipped(flat, grad_scale, params, exp_avg, exp_avg_sq, packed, state, num_obs, beta1, beta2, eps, bookkeeping,
+                               nullptr, p2p_channel, stream);
+}
+
+int vine_grad_clip(float* flat, int count, int length, float* flat2, int count2, int length2, float grad_scale, float max_norm,
+                   float* state, float* workspace, void* p2p_channel, void* p2p_channel2, void* stream) {
+  if (!flat || !state || !workspace || count < 1 || count > length || !isfinite(max_norm)) return VINE_ERR_INVALID_ARG;
+  if (flat2 ? (count2 < 1 || count2 > length2) : (count2 != 0 || length2 != 0 || p2p_channel2)) return VINE_ERR_INVALID_ARG;
+  const int64_t chunks0 = ((int64_t)length + CLIP_CHUNK - 1) / CLIP_CHUNK;
+  const int64_t chunks = chunks0 + (flat2 ? ((int64_t)length2 + CLIP_CHUNK - 1) / CLIP_CHUNK : 0);
+  ClipArgs a;
+  a.flat[0] = flat, a.flat[1] = flat2;
+  a.ch[0] = (VineP2PChannel*)p2p_channel, a.ch[1] = (VineP2PChannel*)p2p_channel2;
+  a.count[0] = count, a.count[1] = count2, a.len[0] = length, a.len[1] = length2;
+  a.chunks0 = (int)chunks0, a.chunks = (int)chunks;
+  a.scale = grad_scale, a.max_norm = max_norm, a.state = state, a.ws = workspace;
+  const int grid = (int)(chunks < CLIP_MAX_BLOCKS ? chunks : CLIP_MAX_BLOCKS);
+  vine_launch::launch(vine_grad_clip_kernel, grid, CLIP_THREADS, 0, (cudaStream_t)stream, a);
   return cudaGetLastError() == cudaSuccess ? VINE_OK : VINE_ERR_CUDA;
 }
 

@@ -4,7 +4,8 @@ this module only owns the HBM buffers (activation tiles, cell states, gradient w
 
 One minibatch (S sequences x L steps, rows ordered [step][sequence]) = 1 MLP forward launch (U tiles), L LSTM steps,
 1 head forward/loss/backward, L x (cell backward + backward-data GEMM), 1 MLP backward launch (recompute + weight
-gradients), 1 LSTM weight-gradient GEMM, 2 reductions, [all-reduce], 2 Adam launches.
+gradients), 1 LSTM weight-gradient GEMM, 2 reductions, [all-reduce], [gradient-norm clip over both vectors, with
+truncate_grads], 2 Adam launches.
 """
 import ctypes as C
 

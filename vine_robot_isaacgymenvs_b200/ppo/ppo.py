@@ -295,8 +295,6 @@ class PPOAgent:
             why.append(f"{self.O} observations (kernels: <= {30 if self.has_rnn else 31})")
         if not (self.normalize_input and self.normalize_value):
             why.append("normalize_input / normalize_value must both be True")
-        if update and self.truncate_grads:
-            why.append("truncate_grads=True (gradient-norm clipping is not in the kernel update)")
         if self.has_rnn:
             if int(rnn_cfg.get("units", 0)) != 256 or not rnn_cfg.get("concat_input") or not rnn_cfg.get("layer_norm"):
                 why.append("network.rnn must be the reference's block: units 256, concat_input True, layer_norm True")
@@ -336,6 +334,7 @@ class PPOAgent:
         self._rng_counter = torch.zeros(1, dtype=torch.int32, device=dev)
         self._moments = torch.zeros(2 * self.O + 4, dtype=torch.float64, device=dev)
         self._adv_stats = torch.zeros(2, device=dev)
+        self._clip_ws = torch.zeros(abi.GRAD_CLIP_WS_FLOATS, device=dev) if self.truncate_grads else None
 
     # ------------------------------------------------------------------ reference network on kernels only
     def _lstm_param_order(self):
@@ -378,6 +377,7 @@ class PPOAgent:
         self._rng_counter = torch.zeros(1, dtype=torch.int32, device=dev)
         self._moments = torch.zeros(2 * self.O + 4, dtype=torch.float64, device=dev)
         self._adv_stats = z(2)
+        self._clip_ws = z(abi.GRAD_CLIP_WS_FLOATS) if self.truncate_grads else None
         L, chunks, tiles_n = self.seq_len, self.T // self.seq_len, self.n // 128
         hyper = dict(e_clip=self.e_clip, critic_coef=self.critic_coef, entropy_coef=self.entropy_coef,
                      bounds_loss_coef=self.bounds_coef, adaptive_lr=int(self.adaptive), kl_threshold=self.kl_threshold)
@@ -492,10 +492,29 @@ class PPOAgent:
                 if self.grad_allreduce == "nccl":   # baseline: ONE NCCL all-reduce per minibatch (gradients + loss statistics)
                     torch.distributed.all_reduce(path.flat_g)
                 sc = 1.0 / self.world                # p2p: the Adam kernels add the ranks' buffers themselves (vine_p2p.cuh)
+                if self.truncate_grads:
+                    self._clip_and_adam_native_lstm(path, sc, pm, pl, stream)
+                    continue
                 assert lib.vine_ppo_adam(p(path.flat_g_mlp), sc, p(self.flat), p(self.adam_m), p(self.adam_v), p(self._packed),
                                          p(self.ppo_state), self.O, 0.9, 0.999, 1e-8, 0, pm, stream) == 0
                 assert lib.vine_lstm_adam(p(path.flat_g_lstm), sc, p(self.flat_l), p(self.adam_ml), p(self.adam_vl), p(self._lpacked),
                                           p(self.ppo_state), self.O, 0.9, 0.999, 1e-8, pl, stream) == 0
+
+    def _clip_and_adam_native_lstm(self, path, sc, pm, pl, stream):
+        """truncate_grads: ONE norm over both gradient vectors (the MLP half without its unused head slots, the whole
+        recurrent half), then both Adam launches with the coefficient.  With peer memory the clip kernel consumes both
+        channels and leaves the rank sums in flat_g_*, so Adam runs without a channel."""
+        lib = self._lib
+        p = lambda x: C.c_void_p(x.data_ptr())  # noqa: E731
+        P, PL = path.P_mlp, path.P_lstm
+        counted = P - sum(t.numel() for t in self._mlp_dummy)
+        assert lib.vine_grad_clip(p(path.flat_g_mlp), counted, P + 4, p(path.flat_g_lstm), PL, PL + 4, sc, self.grad_norm,
+                                  p(self.ppo_state), p(self._clip_ws), pm, pl, stream) == 0
+        coef = C.c_void_p(self.ppo_state.data_ptr() + abi.PPO_STATE_CLIP_COEF * 4)
+        assert lib.vine_ppo_adam_clipped(p(path.flat_g_mlp), sc, p(self.flat), p(self.adam_m), p(self.adam_v), p(self._packed),
+                                         p(self.ppo_state), self.O, 0.9, 0.999, 1e-8, 0, coef, None, stream) == 0
+        assert lib.vine_lstm_adam_clipped(p(path.flat_g_lstm), sc, p(self.flat_l), p(self.adam_ml), p(self.adam_vl), p(self._lpacked),
+                                          p(self.ppo_state), self.O, 0.9, 0.999, 1e-8, coef, None, stream) == 0
 
     def _allreduce_moments(self, stream):
         """Sum over the ranks of the f64 running-statistics moments (observations, values, advantages), once per iteration:
@@ -799,6 +818,15 @@ class PPOAgent:
                                            p(self._logstd_old[slot]), pm, stream) == 0
                 if self.grad_allreduce == "nccl":   # baseline: ONE NCCL all-reduce per minibatch (gradients + loss statistics)
                     torch.distributed.all_reduce(self._flat_grads)
+                if self.truncate_grads:   # the norm of the mean gradient, then Adam with the coefficient (state slot 9)
+                    P = self.flat.numel()  # p2p: the clip kernel consumes the channel and leaves the rank sum in _flat_grads
+                    assert lib.vine_grad_clip(p(self._flat_grads), P, P + 4, None, 0, 0, 1.0 / self.world, self.grad_norm,
+                                              p(self.ppo_state), p(self._clip_ws), pm, None, stream) == 0
+                    coef = C.c_void_p(self.ppo_state.data_ptr() + abi.PPO_STATE_CLIP_COEF * 4)
+                    assert lib.vine_ppo_adam_clipped(p(self._flat_grads), 1.0 / self.world, p(self.flat), p(self.adam_m),
+                                                     p(self.adam_v), p(self._packed), p(self.ppo_state), self.O, 0.9, 0.999, 1e-8,
+                                                     1, coef, None, stream) == 0
+                    continue
                 # p2p: the Adam kernel waits for every rank's buffer and adds them in rank order itself (vine_p2p.cuh)
                 assert lib.vine_ppo_adam(p(self._flat_grads), 1.0 / self.world, p(self.flat), p(self.adam_m), p(self.adam_v),
                                          p(self._packed), p(self.ppo_state), self.O, 0.9, 0.999, 1e-8, 1, pm, stream) == 0
