@@ -143,7 +143,7 @@ __device__ __forceinline__ void env_begin(const VineParams& p, const StepArgs& a
   E.rail_force = 0.f;
 #pragma unroll
   for (int i = 0; i < VINE_MAX_CFI; ++i) E.contact[i] = 0.f;
-  rel_to_abs(p, q, qd, d);
+  rel_to_abs(q, qd, d);
 }
 
 // head of sim step i (VT:338-351): dynamics-scaling draws, rail controller, contact sample, integrator constants
@@ -223,7 +223,7 @@ __device__ __forceinline__ void env_end(const VineParams& p, const StepArgs& a, 
     if (p.stale) {                                                       // V5:796-797 stale rigid-body views
       in.prev_tip[1] = E.tipb_y; in.prev_tip[2] = E.tipb_z;
     } else {                                                             // "as if FK were done": clean episode boundary
-      Dyn dn; rel_to_abs(p, q, qd, dn);
+      Dyn dn; rel_to_abs(q, qd, dn);
       tip_fk(dn, tip_y, tip_z, tipvel_y, tipvel_z);
       in.prev_tip[1] = tip_y; in.prev_tip[2] = tip_z;
       cart_y_body = q[0]; cart_body_vy = 0.f; E.lip = 0.f; E.prev_cart_vel = 0.f;
@@ -350,9 +350,6 @@ vine_step_kernel(const __grid_constant__ VineParams p, const StepArgs a) {
       // ---- controlFrequencyInv x {forces, contact sample, simulate}  VT:338-356 ----
 #pragma unroll 1
       for (int i = 0; i < p.C; ++i) {
-        // exact sin/cos: once per control step in free space (the incremental rotation drifts < 1e-6 over the 40 substeps at
-        // |w| < 36 rad/s), once per sim step with obstacles (impacts can spin a link an order of magnitude faster)
-        if (CONTACT && i > 0) refresh_trig(p, d);
         JointImp J;
         env_sim_step_begin(p, a, i, E, d, J);
 #pragma unroll 1
@@ -378,7 +375,7 @@ vine_step_kernel(const __grid_constant__ VineParams p, const StepArgs a) {
 // bounding box last had a gap to the obstacles' (7 instructions per substep).  An env whose boxes come to overlap is given up
 // -- nothing has been written for it -- and appended to the redo list, which the contact variant runs afterwards.  An env
 // that finishes here never had a contact candidate, so it computed exactly what the contact variant would have (same
-// explicit round-to-nearest arithmetic, same per-sim-step trig refresh): results do not depend on the routing.
+// explicit round-to-nearest arithmetic, same link_trig of the same x): results do not depend on the routing.
 // ------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(VINE_BLOCK) vine_step_far_kernel(const __grid_constant__ VineParams p, const StepArgs a) {
   __shared__ float s_obs[VINE_BLOCK * (VINE_MAX_OBS + 1)];
@@ -399,7 +396,6 @@ __global__ void __launch_bounds__(VINE_BLOCK) vine_step_far_kernel(const __grid_
     const float m00 = fmaf(p.h, p.damping, p.mtot), m00inv = rcp_approx(m00);
 #pragma unroll 1
     for (int i = 0; i < p.C && !given_up; ++i) {
-      if (i > 0) refresh_trig(p, d);        // like the contact variant: exact sin/cos once per sim step
       JointImp J;
       env_sim_step_begin(p, a, i, E, d, J);
 #pragma unroll 1
@@ -541,7 +537,7 @@ __global__ void vine_reset_idx_kernel(const __grid_constant__ VineParams p, cons
   s3.z = 0.f;  // prev_cart_vel_error, V5:799
   s4.w = 0.f;  // aggregated_rew_buf, V5:810
   if (!p.stale) {
-    Dyn d; rel_to_abs(p, q, qd, d);
+    Dyn d; rel_to_abs(q, qd, d);
     float vy, vz; tip_fk(d, s4.x, s4.y, vy, vz);
     s4.z = 0.f; s3.w = 0.f; s3.y = 0.f;
   }
@@ -710,7 +706,7 @@ __global__ void __launch_bounds__(VINE_BLOCK) vine_simulate_kernel(const __grid_
   ContactCache cc = {0u, ghost ? -1e30f : 1e30f, 0u};
   if (CONTACT) build_obstacles(p, io.target_positions[3 * e + 1], io.target_positions[3 * e + 2],
                                io.object_info[2 * e], io.object_info[2 * e + 1], cs, ob);
-  Dyn d; rel_to_abs(p, q, qd, d);
+  Dyn d; rel_to_abs(q, qd, d);
   JointImp J; joint_implicit_consts(p, law, u_use, efforts, J);
   float lip = 0.f;
   const float m00 = fmaf(p.h, p.damping, p.mtot), m00inv = rcp_approx(m00);

@@ -29,6 +29,10 @@ VDEV uint4 philox4x32(uint32_t k0, uint32_t k1, uint32_t c0, uint32_t c1, uint32
 // 1/x as one MUFU.RCP (__fdividef(1, x) adds a range check and a scaling multiply per call; the pivots of the SPD system
 // matrix and squared edge lengths are far inside the normal range)
 VDEV float rcp_approx(float x) { float r; asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x)); return r; }
+// sin/cos as MUFU.SIN / MUFU.COS on the XU pipe behind one shared FMUL by 1/(2 pi), whatever the compiler flags (absolute
+// error <= 2^-20.5 for |x| <= 100 pi, PTX ISA)
+VDEV float sin_approx(float x) { float r; asm("sin.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x)); return r; }
+VDEV float cos_approx(float x) { float r; asm("cos.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x)); return r; }
 // IEEE a / b (round to nearest) for the task logic that must match torch bit for bit. div.rn's fast path (FCHK) sends the whole
 // warp through a ~50-instruction subroutine whenever one lane's numerator is zero, and the observation row is full of exact
 // zeros (x components, depth and angle without an obstacle): ncu showed 20 such calls per warp and step, 17 % of the stall
@@ -199,8 +203,8 @@ VDEV void obstacle_bbox(const VineParams& p, float ty, float tz, float depth, fl
 // ------------------------------------------------------------------------------------------
 // Dynamics state in absolute coordinates: x = (cart y, phi'_0..4), v = d/dt.
 // ------------------------------------------------------------------------------------------
-// S/C = sin/cos of the absolute link angles phi_k = 3.1415 + phi'_k, carried in registers: refreshed
-// exactly once per sim step (refresh_trig) and rotated incrementally by h*w_k in every substep.
+// S/C = sin/cos of the absolute link angles phi_k = 3.1415 + phi'_k, always link_trig of the current x: evaluated by
+// rel_to_abs and again after the position update of every substep.
 template <typename T> struct DynT { T x[6], v[6], S[VINE_NL], C[VINE_NL]; };
 typedef DynT<float> Dyn;
 
@@ -220,6 +224,7 @@ template <> struct Ops<float> {
   static VDEV float sub(float a, float b) { return __fsub_rn(a, b); }
   static VDEV float neg(float a) { return -a; }
   static VDEV float rcp(float a) { return rcp_approx(a); }
+  static VDEV void sincos(float a, float& s, float& c) { s = sin_approx(a); c = cos_approx(a); }
 };
 template <> struct Ops<float2> {
   static VDEV float2 bc(float a) { return make_float2(a, a); }
@@ -229,22 +234,24 @@ template <> struct Ops<float2> {
   static VDEV float2 neg(float2 a) { return make_float2(-a.x, -a.y); }
   static VDEV float2 sub(float2 a, float2 b) { return __fadd2_rn(a, neg(b)); }
   static VDEV float2 rcp(float2 a) { return make_float2(rcp_approx(a.x), rcp_approx(a.y)); }
+  static VDEV void sincos(float2 a, float2& s, float2& c) {
+    s = make_float2(sin_approx(a.x), sin_approx(a.y)); c = make_float2(cos_approx(a.x), cos_approx(a.y));
+  }
 };
 
-VDEV void refresh_trig(const VineParams& p, Dyn& d) {
-#pragma unroll
-  for (int j = 0; j < VINE_NL; ++j) {
-    float s, c; vine_sincos(d.x[j + 1], s, c);
-    d.S[j] = fmaf(p.s0, c, p.c0 * s); d.C[j] = fmaf(p.c0, c, -p.s0 * s);
-  }
+// sin/cos of the absolute angle 3.1415 + x of one link (URDF:289): one FADD, one FMUL and two MUFU. Every kernel takes S/C
+// from here, so they are one function of x whichever kernel integrated it (the routed step equals a single launch).
+template <typename T> VDEV void link_trig(T x, T& s, T& c) {
+  Ops<T>::sincos(Ops<T>::add(x, Ops<T>::bc(VINE_BASE_ANGLE)), s, c);
 }
 
-VDEV void rel_to_abs(const VineParams& p, const float q[6], const float qd[6], Dyn& d) {
+VDEV void rel_to_abs(const float q[6], const float qd[6], Dyn& d) {
   d.x[0] = q[0]; d.v[0] = qd[0];
   float a = 0.f, b = 0.f;
 #pragma unroll
   for (int j = 0; j < VINE_NL; ++j) { a += q[j + 1]; b += qd[j + 1]; d.x[j + 1] = a; d.v[j + 1] = b; }
-  refresh_trig(p, d);
+#pragma unroll
+  for (int j = 0; j < VINE_NL; ++j) link_trig(d.x[j + 1], d.S[j], d.C[j]);
 }
 
 VDEV void abs_to_rel(const Dyn& d, float q[6], float qd[6]) {
@@ -634,16 +641,8 @@ VDEV void substep(const VineParams& p, const JointImpT<T>& J, float m00, float m
 #pragma unroll
   for (int j = 0; j < VINE_NL; ++j) {
     d.v[j + 1] = O::fma(O::bc(p.h), f[j + 1], d.v[j + 1]);
-    const T dl = O::mul(O::bc(p.h), d.v[j + 1]);
-    d.x[j + 1] = O::add(d.x[j + 1], dl);
-    // rotate (S,C) by dl: sin dl ~ dl (1 - dl^2/6), cos dl ~ 1 - dl^2/2. |dl| = h |w| < 0.03 for |w| < 36 rad/s, where the
-    // dropped dl^4/24 < 3.4e-8 is below half an ulp of 1; the exact sin/cos is re-evaluated every sim step (refresh_trig)
-    const T d2 = O::mul(dl, dl);
-    const T sd = O::mul(dl, O::fma(O::bc(-0.16666667f), d2, O::bc(1.f)));
-    const T cd = O::fma(O::bc(-0.5f), d2, O::bc(1.f));
-    const T s = d.S[j], c = d.C[j];
-    d.S[j] = O::fma(s, cd, O::mul(c, sd));
-    d.C[j] = O::fma(c, cd, O::neg(O::mul(s, sd)));
+    d.x[j + 1] = O::fma(O::bc(p.h), d.v[j + 1], d.x[j + 1]);
+    link_trig(d.x[j + 1], d.S[j], d.C[j]);   // evaluated afresh: no drift and no bound on the link rate
   }
 }
 

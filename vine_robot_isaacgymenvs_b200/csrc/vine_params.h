@@ -48,7 +48,6 @@ struct VineParams {
   float kc, dc, rest;            // penalty contact
   float beta[VINE_NL], alpha[VINE_NL], mtot;
   float Lbeta[VINE_NL], gbeta[VINE_NL], inv_L;  // L*beta_j, g*beta_j, 1/L (hoisted products)
-  float s0, c0;                  // sin/cos of the URDF base angle 3.1415 (URDF:289)
   float tip0_y, tip0_z;          // tip pose at q = 0
 };
 
@@ -58,6 +57,7 @@ static const double kPivotZ = 1.0 - 0.025 - 0.01;
 static const double kLinkMass[VINE_NL] = {0.005, 0.005, 0.005, 0.005, 0.1};
 static const double kLinkInertia[VINE_NL] = {6.89246e-6, 6.89246e-6, 6.89246e-6, 6.89246e-6, 1.01559e-4};
 #define VINE_LINK_LEN 0.0885f
+#define VINE_BASE_ANGLE 3.1415f   // kBaseAngle
 #define VINE_PIVOT_Z 0.965f
 #define VINE_LINK_RADIUS 0.0381f
 #define VINE_FPAM_RADIUS 0.0169f
@@ -144,7 +144,6 @@ static inline int vine_derive_params(const VineConfig* c, VineParams* p, const c
   p->mtot = (float)(kCartMass + tail);
   for (int j = 0; j < VINE_NL; ++j) { p->Lbeta[j] = (float)kLinkLen * p->beta[j]; p->gbeta[j] = p->g * p->beta[j]; }
   p->inv_L = (float)(1.0 / kLinkLen);
-  p->s0 = (float)sin(kBaseAngle); p->c0 = (float)cos(kBaseAngle);
   p->tip0_y = (float)(-5.0 * kLinkLen * sin(kBaseAngle)); p->tip0_z = (float)(kPivotZ + 5.0 * kLinkLen * cos(kBaseAngle));
   return VINE_OK;
 }
