@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define VINE_ABI_VERSION 3
+#define VINE_ABI_VERSION 4
 
 #define VINE_NUM_DOFS 6          /* 1 prismatic rail cart + 5 revolute links (V5:54,83) */
 #define VINE_NUM_ACTIONS 2       /* u_rail_velocity, u_fpam (V5:171) */
@@ -141,16 +141,7 @@ typedef struct VineConfig {
                                           rectangle) pairs are re-culled; <= 0 selects the default 0.01 */
   int32_t contact_binning;             /* obstacle variants: order envs by "had contact candidates" before launches of
                                           >= 98,304 envs (1 = default) or keep the identity order (0) */
-  int32_t step_kernel_variant;         /* free space: VINE_STEP_KERNEL_AUTO, _ONE_ENV_PER_THREAD or _TWO_ENVS_PACKED */
 } VineConfig;
-
-/* free-space step kernel: one env per thread (scalar FFMA) or two envs per thread in the two lanes of Blackwell's
- * packed FP32 instructions (fma/mul/add.rn.f32x2); bit-identical results, AUTO picks the faster one measured on B200. */
-typedef enum VineStepKernelVariant {
-  VINE_STEP_KERNEL_AUTO = 0,
-  VINE_STEP_KERNEL_ONE_ENV_PER_THREAD = 1,
-  VINE_STEP_KERNEL_TWO_ENVS_PACKED = 2
-} VineStepKernelVariant;
 
 typedef struct VineEnv VineEnv;
 

@@ -104,7 +104,7 @@ void oracle_config_defaults(VineConfig* c) { /* YT:7-134 */
   c->revolute_lower = -3.4e38; c->revolute_upper = 3.4e38;
   c->prismatic_lower = -3.4e38; c->prismatic_upper = 3.4e38;
   c->contact_stiffness = 2000.0; c->contact_damping = 2.0; c->contact_rest_offset = 0.001;
-  c->contact_cull_slack = 0.01; c->contact_binning = 1; c->step_kernel_variant = 0;  /* launch tuning of the CUDA library: unused here */
+  c->contact_cull_slack = 0.01; c->contact_binning = 1;  /* launch tuning of the CUDA library: unused here */
 }
 
 /* ------------------------------------------------------------------------------------------

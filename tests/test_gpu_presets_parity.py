@@ -177,32 +177,6 @@ def test_dynamics_uniform_halves_are_the_raw_philox_words(lib, oracle_lib):
         assert halves[20] == np.float32(w[10] & 0xFFFF) * np.float32(2.0 ** -16)   # vine_b200.cu: u[10] & 0xffff
 
 
-@pytest.mark.parametrize("n", [1, 129, 1000, 4096 + 77])
-def test_packed_two_env_kernel_equals_one_env_per_thread_kernel_bit_for_bit(n):
-    """Free space: vine_step2_kernel (two envs per thread in the lanes of FFMA2/FMUL2/FADD2) and vine_step_kernel<false>
-    (scalar) run the same explicit round-to-nearest arithmetic per env -> every buffer and every state plane identical,
-    including ragged tails (odd env counts, a lone env in lane A)."""
-    import vine_robot_isaacgymenvs_b200 as vine
-    envs = []
-    for variant in ("one_env_per_thread", "two_envs_packed"):
-        cfg = vcfg.compose(vcfg.FSTR_OVERRIDES + [f"num_envs={n}", "headless=True", "task.env.maxEpisodeLength=20",
-                                                  f"+task.sim.vine_step_kernel={variant}"])
-        env = vine.make(cfg=cfg)
-        env.enable_debug_outputs(True)
-        envs.append(env)
-    g = torch.Generator(device="cuda").manual_seed(n)
-    for t in range(45):   # crosses two episode boundaries: the in-kernel reset branch is exercised
-        a = torch.rand(n, 2, device="cuda", generator=g) * 2.6 - 1.3
-        outs = [e.step(a.clone()) for e in envs]
-        for k in ("obs_buf", "rew_buf", "reset_buf", "progress_buf", "timeout_buf"):
-            assert torch.equal(getattr(envs[0], k), getattr(envs[1], k)), f"{k} step {t}"
-        assert torch.equal(outs[0][0]["obs"], outs[1][0]["obs"])
-    s0, s1 = envs[0].get_state_dict(debug=True), envs[1].get_state_dict(debug=True)
-    for k in s0:
-        assert torch.equal(s0[k], s1[k]), k
-    assert int(envs[0].progress_buf.max()) < 45    # resets did happen
-
-
 @pytest.mark.parametrize("name", ["c2_fstr", "c3_shelf"])
 def test_wandb_dict_matches_the_reference_key_by_key(name, oracle_lib):
     """tests/golden/metrics_<name>.npz holds what the reference's own compute_reward put into ``self.wandb_dict`` at every

@@ -32,7 +32,6 @@ import sys
 LIB = os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "vine_robot_isaacgymenvs_b200", "csrc", "libvine_b200.so")
 KERNELS = {  # mangled name -> short name
     "_Z16vine_step_kernelILb0EEv10VineParams8StepArgs": "vine_step_kernel<false>",
-    "_Z17vine_step2_kernel10VineParams8StepArgs": "vine_step2_kernel",
     "_Z20vine_step_far_kernel10VineParams8StepArgs": "vine_step_far_kernel",
     "_Z16vine_step_kernelILb1EEv10VineParams8StepArgs": "vine_step_kernel<true>",
     "_Z20vine_simulate_kernelILb0EEv10VineParamsl14VineSimulateIO": "vine_simulate_kernel<false>",

@@ -12,7 +12,7 @@ NUM_ACTIONS = 2
 NUM_REWARDS = 13
 NUM_OBJECT_INFO = 2
 MAX_ACTION_DELAY = 8
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 OK = 0
 ERR_INVALID_ARG = -1
@@ -32,7 +32,6 @@ OBSERVATION_TYPES = {
 }
 NUM_OBSERVATIONS = {0: 14, 1: 26, 2: 26, 3: 26, 4: 28, 5: 18}
 TORQUE_LAW_INTEGRATION = {"zoh": 0, "implicit": 1}
-STEP_KERNEL_VARIANT = {"auto": 0, "one_env_per_thread": 1, "two_envs_packed": 2}
 
 # REWARD_NAMES order (reference: Vine5LinkMovingBase.py:78-81) -> cfg["env"] weight keys (:186-200)
 REWARD_NAMES = ["Position", "Const Negative", "Position Success", "Velocity Success", "Velocity",
@@ -83,7 +82,7 @@ class VineConfig(C.Structure):
         ("revolute_lower", _f64), ("revolute_upper", _f64),
         ("prismatic_lower", _f64), ("prismatic_upper", _f64),
         ("contact_stiffness", _f64), ("contact_damping", _f64), ("contact_rest_offset", _f64),
-        ("contact_cull_slack", _f64), ("contact_binning", _i32), ("step_kernel_variant", _i32),
+        ("contact_cull_slack", _f64), ("contact_binning", _i32),
     ]
 
     def copy(self):

@@ -524,5 +524,4 @@ def task_cfg_to_vine_config(cfg):
     c.contact_cull_slack = float(vc.get("cull_slack", 0.01))
     b = vc.get("binning", 1)                    # 0 = one launch in identity order, 1 = routed from 4096 envs, 2 = always routed
     c.contact_binning = int(b) if not isinstance(b, bool) else int(b)
-    c.step_kernel_variant = abi.STEP_KERNEL_VARIANT[str(sim.get("vine_step_kernel", "auto")).lower()]
     return c

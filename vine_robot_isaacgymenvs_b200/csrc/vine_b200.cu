@@ -23,9 +23,6 @@
 #ifndef VINE_STEP_MIN_BLOCKS_CONTACT
 #define VINE_STEP_MIN_BLOCKS_CONTACT 12  // contact variant (1-warp blocks): 160 registers (no spills) instead of 200 -> 12 warps/SM; measured
 #endif                                   // +14 % (shelf) / +11 % (pipe): hides the per-warp load imbalance of the narrow phase
-#ifndef VINE_STEP2_MIN_BLOCKS
-#define VINE_STEP2_MIN_BLOCKS 0  // two-envs-per-thread kernel: the compiler's own register choice
-#endif
 #define VINE_DBG_W 28  // u_rail,u_fpam,prev_u_rail,rail_force,tipvel y,z, reward_matrix[13], pad, fd dof vel[6], fd tip vel y,z
 
 struct StepArgs {
@@ -76,16 +73,16 @@ static char g_create_err[256] = "";
 // ------------------------------------------------------------------------------------------
 // coalesced store of a block's observation rows staged in shared memory
 // ------------------------------------------------------------------------------------------
-template <int ROWS, int THREADS>
+template <int BLOCK>   // one row per thread
 __device__ __forceinline__ void store_obs_block(const float* s_obs, int O, int64_t first, int64_t end, float clip,
                                                 float* __restrict__ obs, float* __restrict__ obs_clamped) {
-  const int64_t row0 = first + (int64_t)blockIdx.x * ROWS;
-  const int rows = (int)min((int64_t)ROWS, end - row0);
+  const int64_t row0 = first + (int64_t)blockIdx.x * BLOCK;
+  const int rows = (int)min((int64_t)BLOCK, end - row0);
   const int count2 = rows * O / 2;  // O is even for every ObservationType
   float2* g = reinterpret_cast<float2*>(obs + row0 * O);
   float2* gc = obs_clamped ? reinterpret_cast<float2*>(obs_clamped + row0 * O) : nullptr;
   const float inv_O = 1.0f / (float)O;
-  for (int i = threadIdx.x; i < count2; i += THREADS) {
+  for (int i = threadIdx.x; i < count2; i += BLOCK) {
     // r0 = e0 / O without the 20-instruction integer division (exact: e0 < 256 * 32, the quotient is far from a rounding boundary)
     const int e0 = 2 * i, r0 = (int)(((float)e0 + 0.5f) * inv_O), c0 = e0 - r0 * O;  // c0 even, c0+1 < O
     float2 v;
@@ -100,8 +97,8 @@ __device__ __forceinline__ void store_obs_block(const float* s_obs, int O, int64
 }
 
 // ------------------------------------------------------------------------------------------
-// The control step of ONE environment, cut at the points where the integrator runs, so that the one-env-per-thread
-// kernel (contact variant) and the two-envs-per-thread kernel (free space, packed FP32) share every line of task logic.
+// The control step of ONE environment, cut at the points where the integrator runs, so that the step kernel (free space and
+// contact variant) and the far pass of the obstacle variants share every line of task logic.
 // ------------------------------------------------------------------------------------------
 struct EnvStep {   // what one env carries in registers across the sim steps of a control step
   float smoothed, prev_cart_vel, prev_err, lip, cart_body_vy;
@@ -346,14 +343,14 @@ vine_step_kernel(const __grid_constant__ VineParams p, const StepArgs a) {
       Obstacles ob = {0, -1, 0.f, 0.f, 0.f, 0.f};
       ContactCache cc = {0u, ghost ? -1e30f : 1e30f, 0u};   // no candidate pairs yet: the first substep culls
       if (CONTACT) { const float4 s5 = a.S5[e]; build_obstacles(p, s5.x, s5.y, s5.z, s5.w, cs, ob); }
-      const float m00 = fmaf(p.h, p.damping, p.mtot), m00inv = rcp_approx(m00);
+      const float m00inv = rcp_approx(fmaf(p.h, p.damping, p.mtot));
       // ---- controlFrequencyInv x {forces, contact sample, simulate}  VT:338-356 ----
 #pragma unroll 1
       for (int i = 0; i < p.C; ++i) {
         JointImp J;
         env_sim_step_begin(p, a, i, E, d, J);
 #pragma unroll 1
-        for (int s = 0; s < p.S; ++s) substep<CONTACT, float>(p, J, m00, m00inv, E.rail_force, ob, cs, cc, d, E.lip, ghost);
+        for (int s = 0; s < p.S; ++s) substep<CONTACT>(p, J, m00inv, E.rail_force, ob, cs, cc, d, E.lip, ghost);
       }
       if (!ghost) {
         env_end(p, a, e, E, d, s_obs + threadIdx.x * (VINE_MAX_OBS + 1));
@@ -362,7 +359,7 @@ vine_step_kernel(const __grid_constant__ VineParams p, const StepArgs a) {
     }
     __syncthreads();
     if (CONTACT && a.list) store_obs_rows_scattered(p, a, s_obs, live ? e : -1);
-    else store_obs_block<BLOCK, BLOCK>(s_obs, p.O, a.first + base - (int64_t)blockIdx.x * BLOCK, a.end, p.clip_obs, a.obs, a.obs_clamped);   // unlisted: lanes == BLOCK
+    else store_obs_block<BLOCK>(s_obs, p.O, a.first + base - (int64_t)blockIdx.x * BLOCK, a.end, p.clip_obs, a.obs, a.obs_clamped);   // unlisted: lanes == BLOCK
     __syncthreads();
   }
 }
@@ -393,14 +390,14 @@ __global__ void __launch_bounds__(VINE_BLOCK) vine_step_far_kernel(const __grid_
     bool given_up = !(gap > 0.f);
     float disp = -gap;
     ContactCache cc = {0u, 0.f, 0u};
-    const float m00 = fmaf(p.h, p.damping, p.mtot), m00inv = rcp_approx(m00);
+    const float m00inv = rcp_approx(fmaf(p.h, p.damping, p.mtot));
 #pragma unroll 1
     for (int i = 0; i < p.C && !given_up; ++i) {
       JointImp J;
       env_sim_step_begin(p, a, i, E, d, J);
 #pragma unroll 1
       for (int s = 0; s < p.S; ++s) {
-        substep<false, float>(p, J, m00, m00inv, E.rail_force, ob, nullptr, cc, d, E.lip);
+        substep<false>(p, J, m00inv, E.rail_force, ob, nullptr, cc, d, E.lip);
         disp += chain_displacement_bound(p, d);
         if (disp > p.cull_slack) {          // the chain may have reached the boxes' gap: measure it again
           gap = chain_obstacle_gap(p, ob, d);
@@ -422,55 +419,6 @@ __global__ void __launch_bounds__(VINE_BLOCK) vine_step_far_kernel(const __grid_
   }
   __syncthreads();
   store_obs_rows_scattered(p, a, s_obs, e);
-}
-
-// ------------------------------------------------------------------------------------------
-// The free-space control step with TWO environments per thread: thread t of a block owns envs base + t and
-// base + VINE_BLOCK2 + t (both coalesced), integrates them in the two lanes of FFMA2/FMUL2/FADD2 (substep<false, float2>)
-// and runs the scalar task logic (bit-exact to the reference's torch kernels) once per env.
-// ------------------------------------------------------------------------------------------
-#define VINE_BLOCK2 128
-__global__ void __launch_bounds__(VINE_BLOCK2, VINE_STEP2_MIN_BLOCKS)
-vine_step2_kernel(const __grid_constant__ VineParams p, const StepArgs a) {
-  __shared__ float s_obs[2 * VINE_BLOCK2 * (VINE_MAX_OBS + 1)];
-  const int64_t eA = a.first + (int64_t)blockIdx.x * (2 * VINE_BLOCK2) + threadIdx.x;
-  const int64_t eB0 = eA + VINE_BLOCK2;
-  const bool liveA = eA < a.end, liveB = eB0 < a.end;
-  const int64_t eB = liveB ? eB0 : eA;   // a ragged tail integrates env A in both lanes and stores it once
-  if (liveA) {
-    EnvStep EA, EB;
-    DynT<float2> d2;
-    {
-      Dyn dA, dB;
-      env_begin(p, a, eA, EA, dA);
-      env_begin(p, a, eB, EB, dB);
-      pack2(dA, dB, d2);
-    }
-    Obstacles ob = {0, -1, 0.f, 0.f, 0.f, 0.f};
-    ContactCache cc = {0u, 1e30f, 0u};
-    float lip_unused = 0.f;
-    const float m00 = fmaf(p.h, p.damping, p.mtot), m00inv = rcp_approx(m00);
-#pragma unroll 1
-    for (int i = 0; i < p.C; ++i) {
-      JointImpT<float2> J2;
-      float2 rail;
-      {
-        Dyn dA, dB; unpack2(d2, dA, dB);
-        JointImp JA, JB;
-        env_sim_step_begin(p, a, i, EA, dA, JA);
-        env_sim_step_begin(p, a, i, EB, dB, JB);
-        pack2(JA, JB, J2);
-        rail = make_float2(EA.rail_force, EB.rail_force);
-      }
-#pragma unroll 1
-      for (int s = 0; s < p.S; ++s) substep<false, float2>(p, J2, m00, m00inv, rail, ob, nullptr, cc, d2, lip_unused);
-    }
-    Dyn dA, dB; unpack2(d2, dA, dB);
-    env_end(p, a, eA, EA, dA, s_obs + threadIdx.x * (VINE_MAX_OBS + 1));
-    if (liveB) env_end(p, a, eB, EB, dB, s_obs + (VINE_BLOCK2 + threadIdx.x) * (VINE_MAX_OBS + 1));
-  }
-  __syncthreads();
-  store_obs_block<2 * VINE_BLOCK2, VINE_BLOCK2>(s_obs, p.O, a.first, a.end, p.clip_obs, a.obs, a.obs_clamped);
 }
 
 // Env order of a binned launch of the contact variant: envs that had contact candidates in their last step first, the others
@@ -709,9 +657,9 @@ __global__ void __launch_bounds__(VINE_BLOCK) vine_simulate_kernel(const __grid_
   Dyn d; rel_to_abs(q, qd, d);
   JointImp J; joint_implicit_consts(p, law, u_use, efforts, J);
   float lip = 0.f;
-  const float m00 = fmaf(p.h, p.damping, p.mtot), m00inv = rcp_approx(m00);
+  const float m00inv = rcp_approx(fmaf(p.h, p.damping, p.mtot));
 #pragma unroll 1
-  for (int s = 0; s < p.S; ++s) substep<CONTACT, float>(p, J, m00, m00inv, efforts[0], ob, cs, cc, d, lip, ghost);
+  for (int s = 0; s < p.S; ++s) substep<CONTACT>(p, J, m00inv, efforts[0], ob, cs, cc, d, lip, ghost);
   if (ghost) return;
   float ty, tz, vy, vz; tip_fk(d, ty, tz, vy, vz);
   abs_to_rel(d, q, qd);
@@ -802,7 +750,7 @@ int vine_config_defaults(VineConfig* c) {  // YT:7-134
   c->revolute_lower = -3.4e38; c->revolute_upper = 3.4e38;
   c->prismatic_lower = -3.4e38; c->prismatic_upper = 3.4e38;
   c->contact_stiffness = 2000.0; c->contact_damping = 2.0; c->contact_rest_offset = 0.001;
-  c->contact_cull_slack = 0.01; c->contact_binning = 1; c->step_kernel_variant = VINE_STEP_KERNEL_AUTO;
+  c->contact_cull_slack = 0.01; c->contact_binning = 1;
   return VINE_OK;
 }
 
@@ -833,9 +781,6 @@ int vine_create(const VineConfig* cfg, int64_t num_envs, int64_t global_env_offs
   memset(env, 0, sizeof(*env));
   // contact variant: re-cull slack in metres (measured on B200: 0.005-0.01 best, 0.04 is 5-10 % slower)
   p.cull_slack = cfg->contact_cull_slack > 0.0 ? (float)cfg->contact_cull_slack : 0.01f;
-  if (cfg->step_kernel_variant < VINE_STEP_KERNEL_AUTO || cfg->step_kernel_variant > VINE_STEP_KERNEL_TWO_ENVS_PACKED) {
-    snprintf(g_create_err, 256, "unknown step_kernel_variant"); return VINE_ERR_INVALID_ARG;
-  }
   env->p = p; env->cfg = *cfg; env->device = device;
   StepArgs& a = env->a;
   a.n = num_envs; a.first = 0; a.end = num_envs; a.gid0 = global_env_offset; a.k0 = (uint32_t)seed; a.k1 = (uint32_t)(seed >> 32);
@@ -1016,16 +961,6 @@ int vine_metrics(VineEnv* env, double* sums, float* maxes, void* stream) {
   return VINE_OK;
 }
 
-// free space: one env per thread (AUTO: as fast at 1 M envs and 1.5x faster at 4096, see DESIGN.md) unless the config asks for
-// the packed two-envs-per-thread kernel
-static void launch_free_step(const VineEnv* env, const StepArgs& a, cudaStream_t st) {
-  const int64_t count = a.end - a.first;
-  if (env->cfg.step_kernel_variant == VINE_STEP_KERNEL_TWO_ENVS_PACKED)
-    vine_step2_kernel<<<grid_for(count, 2 * VINE_BLOCK2), VINE_BLOCK2, 0, st>>>(env->p, a);
-  else
-    vine_launch::launch(vine_step_kernel<false>, grid_for(count, VINE_BLOCK), VINE_BLOCK, 0, st, env->p, a);
-}
-
 // Routed step of the obstacle variants (contact_binning != 0), per control step:
 //   1. vine_bin_kernel          orders the envs: "near" (chain box overlapped the obstacles' box in the last step) first, the
 //                               rest from the back; the near count stays on the device
@@ -1080,7 +1015,7 @@ int vine_step(VineEnv* env, void* stream) {
       vine_launch::launch(vine_step_kernel<true>, grid_for(a.n, VINE_BLOCK_CONTACT), VINE_BLOCK_CONTACT, 0, st, env->p, a);
     }
   } else {
-    launch_free_step(env, env->a, st);
+    vine_launch::launch(vine_step_kernel<false>, grid_for(env->a.n, VINE_BLOCK), VINE_BLOCK, 0, st, env->p, env->a);
   }
   CUDA_TRY(env, cudaGetLastError());
   return VINE_OK;
@@ -1109,7 +1044,7 @@ int vine_step_range(VineEnv* env, int64_t first, int64_t count, void* stream) {
   a.first = first; a.end = first + count;
   a.perm = nullptr;   // chunked launches keep the identity order (the near flags are still maintained)
   if (env->p.shelf || env->p.pipe) vine_step_kernel<true><<<grid_for(count, VINE_BLOCK_CONTACT), VINE_BLOCK_CONTACT, 0, (cudaStream_t)stream>>>(env->p, a);
-  else launch_free_step(env, a, (cudaStream_t)stream);
+  else vine_launch::launch(vine_step_kernel<false>, grid_for(count, VINE_BLOCK), VINE_BLOCK, 0, (cudaStream_t)stream, env->p, a);
   CUDA_TRY(env, cudaGetLastError());
   return VINE_OK;
 }

@@ -205,44 +205,13 @@ VDEV void obstacle_bbox(const VineParams& p, float ty, float tz, float depth, fl
 // ------------------------------------------------------------------------------------------
 // S/C = sin/cos of the absolute link angles phi_k = 3.1415 + phi'_k, always link_trig of the current x: evaluated by
 // rel_to_abs and again after the position update of every substep.
-template <typename T> struct DynT { T x[6], v[6], S[VINE_NL], C[VINE_NL]; };
-typedef DynT<float> Dyn;
-
-// Arithmetic of the integrator, written once for two value types:
-//   float  : one environment per thread (contact variant, function-level entry points)
-//   float2 : TWO environments per thread on Blackwell's packed FP32 instructions (fma/mul/add.rn.f32x2 -> SASS
-//            FFMA2/FMUL2/FADD2): lane .x = env A, .y = env B, half the issue slots per environment. Scalar constants
-//            enter as broadcast operands (`R.F32` / `UR.F32` / immediates in SASS), negations as operand modifiers.
-// Every operation is an explicit round-to-nearest intrinsic (nvcc cannot contract or re-associate them), so both
-// instantiations compute bit-identical results per environment.
-template <typename T> struct Ops;
-template <> struct Ops<float> {
-  static VDEV float bc(float a) { return a; }
-  static VDEV float fma(float a, float b, float c) { return __fmaf_rn(a, b, c); }
-  static VDEV float mul(float a, float b) { return __fmul_rn(a, b); }
-  static VDEV float add(float a, float b) { return __fadd_rn(a, b); }
-  static VDEV float sub(float a, float b) { return __fsub_rn(a, b); }
-  static VDEV float neg(float a) { return -a; }
-  static VDEV float rcp(float a) { return rcp_approx(a); }
-  static VDEV void sincos(float a, float& s, float& c) { s = sin_approx(a); c = cos_approx(a); }
-};
-template <> struct Ops<float2> {
-  static VDEV float2 bc(float a) { return make_float2(a, a); }
-  static VDEV float2 fma(float2 a, float2 b, float2 c) { return __ffma2_rn(a, b, c); }
-  static VDEV float2 mul(float2 a, float2 b) { return __fmul2_rn(a, b); }
-  static VDEV float2 add(float2 a, float2 b) { return __fadd2_rn(a, b); }
-  static VDEV float2 neg(float2 a) { return make_float2(-a.x, -a.y); }
-  static VDEV float2 sub(float2 a, float2 b) { return __fadd2_rn(a, neg(b)); }
-  static VDEV float2 rcp(float2 a) { return make_float2(rcp_approx(a.x), rcp_approx(a.y)); }
-  static VDEV void sincos(float2 a, float2& s, float2& c) {
-    s = make_float2(sin_approx(a.x), sin_approx(a.y)); c = make_float2(cos_approx(a.x), cos_approx(a.y));
-  }
-};
+struct Dyn { float x[6], v[6], S[VINE_NL], C[VINE_NL]; };
 
 // sin/cos of the absolute angle 3.1415 + x of one link (URDF:289): one FADD, one FMUL and two MUFU. Every kernel takes S/C
 // from here, so they are one function of x whichever kernel integrated it (the routed step equals a single launch).
-template <typename T> VDEV void link_trig(T x, T& s, T& c) {
-  Ops<T>::sincos(Ops<T>::add(x, Ops<T>::bc(VINE_BASE_ANGLE)), s, c);
+VDEV void link_trig(float x, float& s, float& c) {
+  const float a = __fadd_rn(x, VINE_BASE_ANGLE);
+  s = sin_approx(a); c = cos_approx(a);
 }
 
 VDEV void rel_to_abs(const float q[6], const float qd[6], Dyn& d) {
@@ -507,8 +476,7 @@ VDEV float contact_forces(const VineParams& p, const Obstacles& ob, ContactScrat
 // per-sim-step joint constants for the implicit integrator:
 //   t_j = tc_j - kk_j theta_j - ek_j thetadot_j  (ek = dd + h kk),  gam_j = h dd_j + h^2 kk_j + armature,
 //   diag_j = alpha_j + gam_j + gam_{j+1} (constant part of the system matrix diagonal)
-template <typename T> struct JointImpT { T kk[VINE_NL], ek[VINE_NL], tc[VINE_NL], gam[VINE_NL], diag[VINE_NL]; };
-typedef JointImpT<float> JointImp;
+struct JointImp { float kk[VINE_NL], ek[VINE_NL], tc[VINE_NL], gam[VINE_NL], diag[VINE_NL]; };
 
 VDEV void joint_implicit_consts(const VineParams& p, const JointLaw& law, float u_use, const float efforts[6], JointImp& J) {
 #pragma unroll
@@ -527,121 +495,100 @@ VDEV void joint_implicit_consts(const VineParams& p, const JointLaw& law, float 
   for (int j = 0; j < VINE_NL; ++j) J.diag[j] = p.alpha[j] + J.gam[j] + (j + 1 < VINE_NL ? J.gam[j + 1] : 0.f);
 }
 
-// (A, B) of two environments -> lanes (.x, .y)
-VDEV void pack2(const Dyn& A, const Dyn& B, DynT<float2>& d) {
-#pragma unroll
-  for (int i = 0; i < 6; ++i) { d.x[i] = make_float2(A.x[i], B.x[i]); d.v[i] = make_float2(A.v[i], B.v[i]); }
-#pragma unroll
-  for (int j = 0; j < VINE_NL; ++j) { d.S[j] = make_float2(A.S[j], B.S[j]); d.C[j] = make_float2(A.C[j], B.C[j]); }
-}
-VDEV void unpack2(const DynT<float2>& d, Dyn& A, Dyn& B) {
-#pragma unroll
-  for (int i = 0; i < 6; ++i) { A.x[i] = d.x[i].x; B.x[i] = d.x[i].y; A.v[i] = d.v[i].x; B.v[i] = d.v[i].y; }
-#pragma unroll
-  for (int j = 0; j < VINE_NL; ++j) { A.S[j] = d.S[j].x; B.S[j] = d.S[j].y; A.C[j] = d.C[j].x; B.C[j] = d.C[j].y; }
-}
-VDEV void pack2(const JointImp& A, const JointImp& B, JointImpT<float2>& J) {
-#pragma unroll
-  for (int j = 0; j < VINE_NL; ++j) {
-    J.kk[j] = make_float2(A.kk[j], B.kk[j]); J.ek[j] = make_float2(A.ek[j], B.ek[j]); J.tc[j] = make_float2(A.tc[j], B.tc[j]);
-    J.gam[j] = make_float2(A.gam[j], B.gam[j]); J.diag[j] = make_float2(A.diag[j], B.diag[j]);
-  }
-}
-
 // One substep of the semi-implicit integrator (equations of motion: DESIGN.md §4):
 //   (A + h D + h^2 K + armature) dv = h [ f - D v - K (x - x0) - h K v ],  v += dv,  x += h v
 // Velocity-product terms in O(n): with a_m = C_m w_m^2, b_m = S_m w_m^2,
 //   P_j = sum_{m>j} L beta_m a_m + L beta_j sum_{m<j} a_m  (Q_j likewise with b):
 //   f_j = S_j (g beta_j - P_j) + C_j Q_j ,   f_y = F - D v_y - (1/L) sum_m L beta_m b_m
-// m00 = M_tot + h D (cart row of the system matrix), m00inv its reciprocal: the same for every env and substep.
-template <bool CONTACT, typename T>
-VDEV void substep(const VineParams& p, const JointImpT<T>& J, float m00, float m00inv, T rail_force, const Obstacles& ob,
-                  ContactScratch* cs, ContactCache& cc, DynT<T>& d, float& lip, bool ghost = false) {
-  typedef Ops<T> O;
-  T a[VINE_NL], b[VINE_NL], As[VINE_NL], Bs[VINE_NL];
+// m00inv = 1 / (M_tot + h D), the reciprocal pivot of the cart row of the system matrix: the same for every env and substep.
+// Every operation is an explicit round-to-nearest intrinsic, which nvcc can neither contract nor re-associate: the far pass
+// and the contact variant therefore compute the same bits for an env without contact, and the routing changes no result.
+template <bool CONTACT>
+VDEV void substep(const VineParams& p, const JointImp& J, float m00inv, float rail_force, const Obstacles& ob,
+                  ContactScratch* cs, ContactCache& cc, Dyn& d, float& lip, bool ghost = false) {
+  float a[VINE_NL], b[VINE_NL], As[VINE_NL], Bs[VINE_NL];
 #pragma unroll
-  for (int j = 0; j < VINE_NL; ++j) { const T w2 = O::mul(d.v[j + 1], d.v[j + 1]); a[j] = O::mul(d.C[j], w2); b[j] = O::mul(d.S[j], w2); }
-  As[VINE_NL - 2] = O::mul(O::bc(p.Lbeta[VINE_NL - 1]), a[VINE_NL - 1]);
-  Bs[VINE_NL - 2] = O::mul(O::bc(p.Lbeta[VINE_NL - 1]), b[VINE_NL - 1]);
+  for (int j = 0; j < VINE_NL; ++j) { const float w2 = __fmul_rn(d.v[j + 1], d.v[j + 1]); a[j] = __fmul_rn(d.C[j], w2); b[j] = __fmul_rn(d.S[j], w2); }
+  As[VINE_NL - 2] = __fmul_rn(p.Lbeta[VINE_NL - 1], a[VINE_NL - 1]);
+  Bs[VINE_NL - 2] = __fmul_rn(p.Lbeta[VINE_NL - 1], b[VINE_NL - 1]);
 #pragma unroll
   for (int j = VINE_NL - 3; j >= 0; --j) {
-    As[j] = O::fma(O::bc(p.Lbeta[j + 1]), a[j + 1], As[j + 1]);
-    Bs[j] = O::fma(O::bc(p.Lbeta[j + 1]), b[j + 1], Bs[j + 1]);
+    As[j] = __fmaf_rn(p.Lbeta[j + 1], a[j + 1], As[j + 1]);
+    Bs[j] = __fmaf_rn(p.Lbeta[j + 1], b[j + 1], Bs[j + 1]);
   }
-  T f[6];
-  f[0] = O::fma(O::bc(-p.inv_L), O::fma(O::bc(p.Lbeta[0]), b[0], Bs[0]), O::fma(O::bc(-p.damping), d.v[0], rail_force));
+  float f[6];
+  f[0] = __fmaf_rn(-p.inv_L, __fmaf_rn(p.Lbeta[0], b[0], Bs[0]), __fmaf_rn(-p.damping, d.v[0], rail_force));
   {
-    T Ap = a[0], Bp = b[0];
-    f[1] = O::fma(d.C[0], Bs[0], O::mul(d.S[0], O::sub(O::bc(p.gbeta[0]), As[0])));
+    float Ap = a[0], Bp = b[0];
+    f[1] = __fmaf_rn(d.C[0], Bs[0], __fmul_rn(d.S[0], __fsub_rn(p.gbeta[0], As[0])));
 #pragma unroll
     for (int j = 1; j < VINE_NL; ++j) {
-      const T P = j == VINE_NL - 1 ? O::mul(O::bc(p.Lbeta[j]), Ap) : O::fma(O::bc(p.Lbeta[j]), Ap, As[j]);
-      const T Q = j == VINE_NL - 1 ? O::mul(O::bc(p.Lbeta[j]), Bp) : O::fma(O::bc(p.Lbeta[j]), Bp, Bs[j]);
-      f[j + 1] = O::fma(d.C[j], Q, O::mul(d.S[j], O::sub(O::bc(p.gbeta[j]), P)));
-      if (j + 1 < VINE_NL) { Ap = O::add(Ap, a[j]); Bp = O::add(Bp, b[j]); }
+      const float P = j == VINE_NL - 1 ? __fmul_rn(p.Lbeta[j], Ap) : __fmaf_rn(p.Lbeta[j], Ap, As[j]);
+      const float Q = j == VINE_NL - 1 ? __fmul_rn(p.Lbeta[j], Bp) : __fmaf_rn(p.Lbeta[j], Bp, Bs[j]);
+      f[j + 1] = __fmaf_rn(d.C[j], Q, __fmul_rn(d.S[j], __fsub_rn(p.gbeta[j], P)));
+      if (j + 1 < VINE_NL) { Ap = __fadd_rn(Ap, a[j]); Bp = __fadd_rn(Bp, b[j]); }
     }
   }
   // joint torques (relative coordinates) -> absolute: Q_j = t_j - t_{j+1}
   {
-    T tn = O::bc(0.f);
+    float tn = 0.f;
 #pragma unroll
     for (int j = VINE_NL - 1; j >= 0; --j) {
-      const T th = j == 0 ? d.x[1] : O::sub(d.x[j + 1], d.x[j]);
-      const T thd = j == 0 ? d.v[1] : O::sub(d.v[j + 1], d.v[j]);
-      const T t = O::fma(O::neg(J.ek[j]), thd, O::fma(O::neg(J.kk[j]), th, J.tc[j]));
-      f[j + 1] = O::add(f[j + 1], j == VINE_NL - 1 ? t : O::sub(t, tn));
+      const float th = j == 0 ? d.x[1] : __fsub_rn(d.x[j + 1], d.x[j]);
+      const float thd = j == 0 ? d.v[1] : __fsub_rn(d.v[j + 1], d.v[j]);
+      const float t = __fmaf_rn(-J.ek[j], thd, __fmaf_rn(-J.kk[j], th, J.tc[j]));
+      f[j + 1] = __fadd_rn(f[j + 1], j == VINE_NL - 1 ? t : __fsub_rn(t, tn));
       tn = t;
     }
   }
   if constexpr (CONTACT) lip = contact_forces(p, ob, cs, cc, d, f, ghost);   // ghost: a lane without an env of its own (see there)
   // lower triangle of the SPD system matrix; rows/cols: 0 = cart, 1..5 = links
-  T M[6][6];
+  float M[6][6];
 #pragma unroll
   for (int j = 0; j < VINE_NL; ++j) {
-    M[j + 1][0] = O::mul(O::bc(-p.beta[j]), d.C[j]);
+    M[j + 1][0] = __fmul_rn(-p.beta[j], d.C[j]);
     M[j + 1][j + 1] = J.diag[j];
 #pragma unroll
     for (int m = 0; m < j; ++m) {
-      const T c = O::fma(d.C[j], d.C[m], O::mul(d.S[j], d.S[m]));
-      M[j + 1][m + 1] = (m == j - 1) ? O::fma(O::bc(p.Lbeta[j]), c, O::neg(J.gam[j])) : O::mul(O::bc(p.Lbeta[j]), c);
+      const float c = __fmaf_rn(d.C[j], d.C[m], __fmul_rn(d.S[j], d.S[m]));
+      M[j + 1][m + 1] = (m == j - 1) ? __fmaf_rn(p.Lbeta[j], c, -J.gam[j]) : __fmul_rn(p.Lbeta[j], c);
     }
   }
   // LDL^T (row-wise): u_q = A_jq - sum_{r<q} u_r L_qr ; L_jq = u_q / d_q ; d_j = A_jj - sum_q u_q L_jq
-  T dinv[6];
-  dinv[0] = O::bc(m00inv);
+  float dinv[6];
+  dinv[0] = m00inv;
 #pragma unroll
   for (int j = 1; j < 6; ++j) {
-    T u[5];
-    T dj = M[j][j];
+    float u[5];
+    float dj = M[j][j];
 #pragma unroll
     for (int q = 0; q < j; ++q) {
-      T uq = M[j][q];
+      float uq = M[j][q];
 #pragma unroll
-      for (int r = 0; r < q; ++r) uq = O::fma(O::neg(u[r]), M[q][r], uq);
+      for (int r = 0; r < q; ++r) uq = __fmaf_rn(-u[r], M[q][r], uq);
       u[q] = uq;
-      const T l = O::mul(uq, dinv[q]);
+      const float l = __fmul_rn(uq, dinv[q]);
       M[j][q] = l;
-      dj = O::fma(O::neg(uq), l, dj);
+      dj = __fmaf_rn(-uq, l, dj);
     }
-    dinv[j] = O::rcp(dj);
+    dinv[j] = rcp_approx(dj);
   }
-  (void)m00;
   // solve M a = f (dv = h a is folded into the velocity update)
 #pragma unroll
   for (int i = 1; i < 6; ++i)
 #pragma unroll
-    for (int q = 0; q < i; ++q) f[i] = O::fma(O::neg(M[i][q]), f[q], f[i]);
+    for (int q = 0; q < i; ++q) f[i] = __fmaf_rn(-M[i][q], f[q], f[i]);
 #pragma unroll
-  for (int i = 0; i < 6; ++i) f[i] = O::mul(f[i], dinv[i]);
+  for (int i = 0; i < 6; ++i) f[i] = __fmul_rn(f[i], dinv[i]);
 #pragma unroll
   for (int i = 4; i >= 0; --i)
 #pragma unroll
-    for (int q = i + 1; q < 6; ++q) f[i] = O::fma(O::neg(M[q][i]), f[q], f[i]);
-  d.v[0] = O::fma(O::bc(p.h), f[0], d.v[0]); d.x[0] = O::fma(O::bc(p.h), d.v[0], d.x[0]);
+    for (int q = i + 1; q < 6; ++q) f[i] = __fmaf_rn(-M[q][i], f[q], f[i]);
+  d.v[0] = __fmaf_rn(p.h, f[0], d.v[0]); d.x[0] = __fmaf_rn(p.h, d.v[0], d.x[0]);
 #pragma unroll
   for (int j = 0; j < VINE_NL; ++j) {
-    d.v[j + 1] = O::fma(O::bc(p.h), f[j + 1], d.v[j + 1]);
-    d.x[j + 1] = O::fma(O::bc(p.h), d.v[j + 1], d.x[j + 1]);
+    d.v[j + 1] = __fmaf_rn(p.h, f[j + 1], d.v[j + 1]);
+    d.x[j + 1] = __fmaf_rn(p.h, d.v[j + 1], d.x[j + 1]);
     link_trig(d.x[j + 1], d.S[j], d.C[j]);   // evaluated afresh: no drift and no bound on the link rate
   }
 }
