@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define VINE_ABI_VERSION 4
+#define VINE_ABI_VERSION 5
 
 #define VINE_NUM_DOFS 6          /* 1 prismatic rail cart + 5 revolute links (V5:54,83) */
 #define VINE_NUM_ACTIONS 2       /* u_rail_velocity, u_fpam (V5:171) */
@@ -441,6 +441,9 @@ int vine_policy_act(const VinePolicyAct* args, void* stream);
  * After the env step (rl_games play_steps tail): shaped = reward * reward_scale (YP:58-59)
  * [+ gamma * value on time-outs, value_bootstrap YP:56], dones, per-env episode return/length and the
  * device-side episode statistics ep_stats f64[4] += {episodes, successes, sum return, sum length}.
+ * The whole rl_games DefaultRewardsShaper (without log_val): shaped = clamp((reward + reward_shift) * reward_scale,
+ * reward_min, reward_max), the shift added only when it is non-zero (reward + 0 would turn -0 into +0) and the clamp applied
+ * only with reward_clamp != 0; a NaN reward stays NaN, as with torch.clamp.
  */
 typedef struct VineRolloutPost {
   const float* rewards;          /* env rew_buf [n] */
@@ -458,6 +461,9 @@ typedef struct VineRolloutPost {
   int32_t value_bootstrap;
   float success_reward_threshold;
   float* not_done_next;          /* NULL or [n] out: 1 - dones_next (the mask of the recurrent state) */
+  float reward_shift;            /* reward_shaper.shift_value (0: none) */
+  float reward_min, reward_max;  /* reward_shaper.min_val / max_val, used when reward_clamp != 0 */
+  int32_t reward_clamp;
 } VineRolloutPost;
 int vine_rollout_post(const VineRolloutPost* args, void* stream);
 
@@ -561,6 +567,8 @@ typedef struct VineLstmHeadTrain {
    * stores this pass's mu into columns 2,3 of the source row of every minibatch row (rows = [step in chunk][chunk][env]) */
   float* mu_writeback;
   int64_t wb_seq_len, wb_chunks, wb_num_envs, wb_env_begin, wb_env_count;
+  int32_t value_loss_unclipped;  /* 0: clipped value loss (rl_games clip_value True); 1: c_loss = (return - v)^2 */
+  int32_t reserved2;             /* 0 */
 } VineLstmHeadTrain;
 int vine_lstm_head_train(const VineLstmHeadTrain* args, void* stream);
 
@@ -666,8 +674,8 @@ int vine_lstm_cell_bwd(const void* acts_bf16, const float* c_prev, const float* 
 
 /*
  * PPO minibatch update of the same network as ONE fused tcgen05/TMEM kernel: forward, the PPO losses of
- * Vine5LinkMovingBasePPO.yaml:46-81 (e_clip actor loss, clipped value loss x critic_coef / 2, bounds loss,
- * entropy), backward and weight gradients (rl_games A2CAgent.calc_gradients + autograd; in-repo analogue
+ * Vine5LinkMovingBasePPO.yaml:46-81 (e_clip actor loss, clipped -- with value_loss_unclipped plain -- value loss
+ * x critic_coef / 2, bounds loss, entropy), backward and weight gradients (rl_games A2CAgent.calc_gradients + autograd; in-repo analogue
  * learning/common_agent.py:319-435, 482-517), then the gradient reduction and torch.optim.Adam.
  *
  * Parameters live in ONE flat f32 vector in torch layouts, in this order:
@@ -681,10 +689,17 @@ int vine_lstm_cell_bwd(const void* acts_bf16, const float* c_prev, const float* 
  *
  * state (device, >= 16 floats): [0] learning rate, [1] Adam step count, [2] KL of the last minibatch,
  * [3] "KL pending" flag, [4..7] running sums of a_loss, c_loss, kl, b_loss, [8] minibatches summed,
- * [9] gradient-clipping coefficient and [10] gradient norm of the last vine_grad_clip call (untouched without clipping).
- * With adaptive_lr the `legacy` schedule of rl_games (lr /= 1.5 if kl > 2 kl_threshold, lr *= 1.5 if
- * kl < kl_threshold / 2, clamped to [lr_min, lr_max]) is applied on the device between optimiser steps:
- * no host synchronisation anywhere, the whole update is CUDA-graph capturable.
+ * [9] gradient-clipping coefficient and [10] gradient norm of the last vine_grad_clip call (untouched without clipping),
+ * [11] training iteration (rl_games epoch_num: +1 by every launch with epoch_begin), [12] sum and [13] count of the
+ * minibatch KLs of the current mini-epoch (schedule_standard).
+ * The learning-rate schedule runs on the device between optimiser steps, in block 0 of vine_ppo_minibatch: no host
+ * synchronisation anywhere, the whole update is CUDA-graph capturable.  One run of the rule (rl_games scheduler.update):
+ *   adaptive_lr: lr /= 1.5 if kl > 2 kl_threshold, lr *= 1.5 if kl < kl_threshold / 2, clamped to [lr_min, lr_max];
+ *   lr_linear:   lr = lr_min + (lr0 - lr_min) * max(0, max_epochs - epoch) / max_epochs (epoch = state[11]);
+ *   neither:     lr unchanged.
+ * When: schedule_standard = 0 (rl_games `legacy`): with the KL of every minibatch, before the next optimiser step;
+ * schedule_standard = 1 (`standard`): once per mini-epoch with the mean KL of its minibatches, applied by the first launch of
+ * the next mini-epoch (mini_epoch_begin).  A launch first applies what is pending, then counts epoch_begin.
  */
 #define VINE_PPO_WS_FLOATS 49664   /* floats per CTA gradient partial */
 typedef struct VinePpoMinibatch {
@@ -710,6 +725,14 @@ typedef struct VinePpoMinibatch {
   const float* dh3_ext;          /* NULL, or f32 [T*env_count, 64]: d(loss)/d(MLP output) supplied by the LSTM backward
                                     (vine_lstm_bwd_gemm); the heads and losses are skipped and the loss pointers may be
                                     NULL -- the kernel recomputes the MLP forward and back-propagates from there */
+  int32_t lr_linear;             /* 1: linear schedule (adaptive_lr must be 0; max_epochs > 0) */
+  int32_t schedule_standard;     /* 0: rl_games schedule_type legacy, 1: standard (see above) */
+  int32_t epoch_begin;           /* 1: this launch opens a training iteration */
+  int32_t mini_epoch_begin;      /* 1: this launch opens a mini-epoch */
+  int32_t max_epochs;            /* lr_linear: the schedule's length in iterations */
+  int32_t value_loss_unclipped;  /* 0: clipped value loss (rl_games clip_value True); 1: c_loss = (return - v)^2 */
+  float lr0;                     /* lr_linear: the initial learning rate */
+  float reserved_f2;             /* 0 */
 } VinePpoMinibatch;
 
 int vine_ppo_num_params(int num_obs);

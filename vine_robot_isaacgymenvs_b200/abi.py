@@ -12,7 +12,7 @@ NUM_ACTIONS = 2
 NUM_REWARDS = 13
 NUM_OBJECT_INFO = 2
 MAX_ACTION_DELAY = 8
-ABI_VERSION = 4
+ABI_VERSION = 5
 
 OK = 0
 ERR_INVALID_ARG = -1
@@ -157,6 +157,7 @@ LSTM_TILE_BYTES = 32768          # one [128 x 128] bf16 activation tile
 PPO_WS_FLOATS = 49664
 PPO_STATE_FLOATS = 16
 PPO_STATE_CLIP_COEF, PPO_STATE_GRAD_NORM = 9, 10   # slots of the state block written by vine_grad_clip
+PPO_STATE_EPOCH, PPO_STATE_EPOCH_KL_SUM, PPO_STATE_EPOCH_KL_COUNT = 11, 12, 13   # learning-rate schedule (vine_ppo_minibatch)
 GRAD_CLIP_WS_FLOATS = 1024
 
 
@@ -184,7 +185,8 @@ class VineLstmHeadTrain(C.Structure):
                 + [("n", C.c_int64)]
                 + [(n, C.c_float) for n in ("e_clip", "critic_coef", "entropy_coef", "bounds_loss_coef", "inv_B", "reserved_f")]
                 + [("mu_writeback", C.c_void_p)]
-                + [(n, C.c_int64) for n in ("wb_seq_len", "wb_chunks", "wb_num_envs", "wb_env_begin", "wb_env_count")])
+                + [(n, C.c_int64) for n in ("wb_seq_len", "wb_chunks", "wb_num_envs", "wb_env_begin", "wb_env_count")]
+                + [("value_loss_unclipped", C.c_int32), ("reserved2", C.c_int32)])
 
 
 class VineLstmCellBwd(C.Structure):
@@ -210,7 +212,8 @@ class VineRolloutPost(C.Structure):
         "rewards", "resets", "timeouts", "values", "shaped_rewards", "dones_next", "ep_return", "ep_length", "ep_stats",
         "rng_counter")]
         + [("n", C.c_int64), ("reward_scale", C.c_float), ("gamma", C.c_float), ("value_bootstrap", C.c_int32),
-           ("success_reward_threshold", C.c_float), ("not_done_next", C.c_void_p)])
+           ("success_reward_threshold", C.c_float), ("not_done_next", C.c_void_p),
+           ("reward_shift", C.c_float), ("reward_min", C.c_float), ("reward_max", C.c_float), ("reward_clamp", C.c_int32)])
 
 
 class VinePpoPrologue(C.Structure):
@@ -229,7 +232,10 @@ class VinePpoMinibatch(C.Structure):
                                     "adaptive_lr", "reserved")]
         + [(n, C.c_float) for n in ("e_clip", "critic_coef", "entropy_coef", "bounds_loss_coef", "kl_threshold",
                                     "lr_min", "lr_max", "reserved_f")]
-        + [("dh3_ext", C.c_void_p)])
+        + [("dh3_ext", C.c_void_p)]
+        + [(n, C.c_int32) for n in ("lr_linear", "schedule_standard", "epoch_begin", "mini_epoch_begin", "max_epochs",
+                                    "value_loss_unclipped")]
+        + [("lr0", C.c_float), ("reserved_f2", C.c_float)])
 
 # argument structs of the PPO entry points in the order of vine_abi_struct_size()
 PPO_STRUCTS = [VinePolicyAct, VineRolloutPost, VinePpoPrologue, VinePpoMinibatch, VineLstmStep, VineLstmHead, VineLstmHeadTrain,

@@ -390,6 +390,7 @@ __global__ void __launch_bounds__(256, 2) vine_lstm_head_train_kernel(const Vine
   const float klc0 = __logf(sigo0 / sig0 + 1e-5f) - 0.5f, klc1 = __logf(sigo1 / sig1 + 1e-5f) - 0.5f;
   const float klq0 = 1.f / (2.f * (sigo0 * sigo0 + 1e-5f)), klq1 = 1.f / (2.f * (sigo1 * sigo1 + 1e-5f));
   const float lo = 1.f - a.e_clip, hi = 1.f + a.e_clip;
+  const bool clip_value = !a.value_loss_unclipped;   // rl_games clip_value
   __syncthreads();
   auto load8 = [&](int arr, float* v) {
     const float4 x = prm[arr][0][lane], y = prm[arr][1][lane];
@@ -479,7 +480,7 @@ __global__ void __launch_bounds__(256, 2) vine_lstm_head_train_kernel(const Vine
       const float dvo = v - vo, vclip = vo + fminf(fmaxf(dvo, -a.e_clip), a.e_clip);
       const float r1 = v - ret, r2 = vclip - ret, c1 = r1 * r1, c2 = r2 * r2;
       const float pass2 = (fabsf(dvo) <= a.e_clip) ? 1.f : 0.f;
-      const float dvc = c1 > c2 ? 2.f * r1 : (c2 > c1 ? 2.f * r2 * pass2 : r1 + r2 * pass2);
+      const float dvc = !clip_value ? 2.f * r1 : c1 > c2 ? 2.f * r1 : (c2 > c1 ? 2.f * r2 * pass2 : r1 + r2 * pass2);
       float dv = 0.5f * a.critic_coef * dvc;
       const float bh0 = fmaxf(mu0 - 1.1f, 0.f), bl0 = fminf(mu0 + 1.1f, 0.f), bh1 = fmaxf(mu1 - 1.1f, 0.f), bl1 = fminf(mu1 + 1.1f, 0.f);
       dmu0 += a.bounds_loss_coef * 2.f * (bh0 + bl0);
@@ -491,7 +492,7 @@ __global__ void __launch_bounds__(256, 2) vine_lstm_head_train_kernel(const Vine
       gr[r][0] = dmu0, gr[r][1] = dmu1, gr[r][2] = dv;
       sc[0] += dmu0, sc[1] += dmu1, sc[2] += dv;
       sc[3] += dls0 * w, sc[4] += dls1 * w;
-      sc[5] += fmaxf(t1, t2) * w, sc[6] += fmaxf(c1, c2) * w, sc[7] += kl * w;
+      sc[5] += fmaxf(t1, t2) * w, sc[6] += (clip_value ? fmaxf(c1, c2) : c1) * w, sc[7] += kl * w;
       sc[8] += (bh0 * bh0 + bl0 * bl0 + bh1 * bh1 + bl1 * bl1) * w;
       if (lane == 0 && ok[r]) {
         const int64_t s = srow[r];

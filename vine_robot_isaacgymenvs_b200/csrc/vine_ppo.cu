@@ -53,6 +53,7 @@ constexpr int WS_FLOATS = 49664;
 static_assert(WS_STATS + 8 <= WS_FLOATS && WS_FLOATS == VINE_PPO_WS_FLOATS, "workspace layout");
 // device-resident optimiser state (floats): see include/vine_b200.h
 constexpr int ST_LR = 0, ST_STEP = 1, ST_KL = 2, ST_PENDING = 3, ST_SUMS = 4 /* a,c,kl,b */, ST_COUNT = 8;
+constexpr int ST_EPOCH = 11, ST_EKL_SUM = 12, ST_EKL_N = 13;   // iteration, KL sum / count of the current mini-epoch
 
 struct MbArgs {
   const uint8_t* packed;
@@ -61,9 +62,23 @@ struct MbArgs {
   float *ws, *state, *debug;
   const float* dh3_ext;   // recurrent network: d(loss)/d(h3) comes from the LSTM backward instead of the MLP heads
   int T, N, e0, E, O;
-  float e_clip, critic_coef, entropy_coef, bounds_coef, inv_B, kl_threshold, lr_min, lr_max;
-  int adaptive;
+  float e_clip, critic_coef, entropy_coef, bounds_coef, inv_B, kl_threshold, lr_min, lr_max, lr0;
+  int adaptive, linear, standard, epoch_begin, mini_epoch_begin, max_epochs, clip_value;
 };
+
+// One run of the learning-rate rule (rl_games scheduler.update) on the state block; `kl` is the rank-mean KL it acts on.
+__device__ __forceinline__ void lr_schedule_rule(const MbArgs& a, float kl) {
+  float lr = a.state[ST_LR];
+  if (a.adaptive) {   // AdaptiveScheduler
+    if (kl > 2.f * a.kl_threshold) lr = fmaxf(lr / 1.5f, a.lr_min);
+    if (kl < 0.5f * a.kl_threshold) lr = fminf(lr * 1.5f, a.lr_max);
+  } else if (a.linear) {   // LinearScheduler(use_epochs=True): in f64, one rounding to f32
+    const double left = fmax((double)a.max_epochs - (double)a.state[ST_EPOCH], 0.0);
+    lr = (float)((double)a.lr_min + ((double)a.lr0 - (double)a.lr_min) * (left / (double)a.max_epochs));
+  }
+  a.state[ST_LR] = lr;
+}
+
 
 // Q = epilogue threads per row (2 or 4): thread (row, part) owns the columns [part * N/Q, (part+1) * N/Q) of every N-wide
 // accumulator; with Q = 4 the SM has 4 warps per sub-partition to hide the TMEM/shared-memory latencies of the epilogues.
@@ -86,18 +101,24 @@ __global__ void __launch_bounds__(128 * Q, 1) vine_ppo_minibatch_kernel(const Mb
     mbar_expect_tx(bar_w, PACKED_BYTES);
     bulk_g2s(smem_u32(smem), a.packed, PACKED_BYTES, bar_w);   // ONE bulk TMA copy: all weights and biases
     if (blockIdx.x == 0) {
-      // the adaptive-KL learning-rate schedule (rl_games `legacy`) acts between optimiser steps: apply the KL of the
-      // previous minibatch now, then count this step.  The Adam kernel that follows in the stream reads both.
+      // the learning-rate schedule acts between optimiser steps: `legacy` applies the KL of the previous minibatch now;
+      // `standard` adds it to the mini-epoch's sum and applies the mean when a new mini-epoch opens.  Then count this
+      // iteration (if it opens one) and this step.  The Adam kernel that follows in the stream reads both.
       if (a.state[ST_PENDING] != 0.f) {
-        if (a.adaptive) {
-          const float kl = a.state[ST_KL];
-          float lr = a.state[ST_LR];
-          if (kl > 2.f * a.kl_threshold) lr = fmaxf(lr / 1.5f, a.lr_min);
-          if (kl < 0.5f * a.kl_threshold) lr = fminf(lr * 1.5f, a.lr_max);
-          a.state[ST_LR] = lr;
+        if (a.standard) {
+          a.state[ST_EKL_SUM] += a.state[ST_KL];
+          a.state[ST_EKL_N] += 1.f;
+        } else {
+          lr_schedule_rule(a, a.state[ST_KL]);
         }
         a.state[ST_PENDING] = 0.f;
       }
+      if (a.standard && a.mini_epoch_begin && a.state[ST_EKL_N] > 0.f) {
+        lr_schedule_rule(a, a.state[ST_EKL_SUM] / a.state[ST_EKL_N]);
+        a.state[ST_EKL_SUM] = 0.f;
+        a.state[ST_EKL_N] = 0.f;
+      }
+      if (a.epoch_begin) a.state[ST_EPOCH] += 1.f;
       a.state[ST_STEP] += 1.f;
     }
   }
@@ -196,11 +217,11 @@ __global__ void __launch_bounds__(128 * Q, 1) vine_ppo_minibatch_kernel(const Mb
         dmu0 = g_nlp * (-d0 * inv_sig0);
         dmu1 = g_nlp * (-d1 * inv_sig1);
         float dls0 = g_nlp * (1.f - d0 * d0) - a.entropy_coef, dls1 = g_nlp * (1.f - d1 * d1) - a.entropy_coef;
-        // clipped value loss (clip_value: True), both on normalised values
+        // clipped value loss (clip_value: True) or (ret - v)^2 (clip_value: False), both on normalised values
         const float dvo = v - vo, vclip = vo + fminf(fmaxf(dvo, -a.e_clip), a.e_clip);
         const float e1 = v - ret, e2 = vclip - ret, c1 = e1 * e1, c2 = e2 * e2;
         const float pass2 = (fabsf(dvo) <= a.e_clip) ? 1.f : 0.f;
-        const float dvc = c1 > c2 ? 2.f * e1 : (c2 > c1 ? 2.f * e2 * pass2 : e1 + e2 * pass2);
+        const float dvc = !a.clip_value ? 2.f * e1 : c1 > c2 ? 2.f * e1 : (c2 > c1 ? 2.f * e2 * pass2 : e1 + e2 * pass2);
         dv = 0.5f * a.critic_coef * dvc;
         // bound loss on mu (soft bound 1.1)
         const float bh0 = fmaxf(mu0 - 1.1f, 0.f), bl0 = fminf(mu0 + 1.1f, 0.f), bh1 = fmaxf(mu1 - 1.1f, 0.f), bl1 = fminf(mu1 + 1.1f, 0.f);
@@ -211,7 +232,7 @@ __global__ void __launch_bounds__(128 * Q, 1) vine_ppo_minibatch_kernel(const Mb
         // the next mini-epoch measures its KL against THIS pass (a2c_common train_epoch: dataset.update_mu_sigma(cmu, csigma))
         *reinterpret_cast<float2*>(a.mu_old + 2 * grow) = make_float2(mu0, mu1);
         st[0] += fmaxf(t1, t2) * a.inv_B;
-        st[1] += fmaxf(c1, c2) * a.inv_B;
+        st[1] += (a.clip_value ? fmaxf(c1, c2) : c1) * a.inv_B;
         st[2] += kl * a.inv_B;
         st[3] += (bh0 * bh0 + bl0 * bl0 + bh1 * bh1 + bl1 * bl1) * a.inv_B;
         st[4] += dls0 * a.inv_B;
@@ -603,6 +624,7 @@ int vine_ppo_minibatch(const VinePpoMinibatch* b, void* stream) {
   if (b->horizon < 1 || b->num_envs < 1 || b->env_count < 1 || b->env_begin < 0 || b->env_begin + b->env_count > b->num_envs ||
       b->num_obs < 1 || b->num_obs >= K1 || (((uintptr_t)b->packed) & 15u) || (((uintptr_t)b->workspace) & 15u))
     return VINE_ERR_INVALID_ARG;
+  if (b->lr_linear && (b->adaptive_lr || b->max_epochs < 1)) return VINE_ERR_INVALID_ARG;
   static int configured = -1, q4 = 1;
   int dev = 0, sms = 0;
   if (cudaGetDevice(&dev) != cudaSuccess) return VINE_ERR_CUDA;
@@ -627,6 +649,8 @@ int vine_ppo_minibatch(const VinePpoMinibatch* b, void* stream) {
   a.T = b->horizon, a.N = b->num_envs, a.e0 = b->env_begin, a.E = b->env_count, a.O = b->num_obs;
   a.e_clip = b->e_clip, a.critic_coef = b->critic_coef, a.entropy_coef = b->entropy_coef, a.bounds_coef = b->bounds_loss_coef;
   a.inv_B = 1.0f / (float)B, a.kl_threshold = b->kl_threshold, a.lr_min = b->lr_min, a.lr_max = b->lr_max, a.adaptive = b->adaptive_lr;
+  a.lr0 = b->lr0, a.linear = b->lr_linear, a.standard = b->schedule_standard, a.epoch_begin = b->epoch_begin;
+  a.mini_epoch_begin = b->mini_epoch_begin, a.max_epochs = b->max_epochs, a.clip_value = !b->value_loss_unclipped;
   if (q4) vine_launch::launch(vine_ppo_minibatch_kernel<4>, grid, 512, SMEM_BYTES, (cudaStream_t)stream, a);
   else vine_launch::launch(vine_ppo_minibatch_kernel<2>, grid, 256, SMEM_BYTES, (cudaStream_t)stream, a);
   if (cudaGetLastError() != cudaSuccess) return VINE_ERR_CUDA;

@@ -149,7 +149,12 @@ __global__ void __launch_bounds__(256) vine_rollout_post_kernel(const VineRollou
   if (i < a.n) {
     const float rew = a.rewards[i];
     const float d = a.resets[i] != 0 ? 1.f : 0.f;
-    float shaped = rew * a.reward_scale;
+    // rl_games DefaultRewardsShaper: (r + shift) * scale, clamped like torch.clamp (comparisons keep a NaN, fminf would not)
+    float shaped = (a.reward_shift != 0.f ? rew + a.reward_shift : rew) * a.reward_scale;
+    if (a.reward_clamp) {
+      if (shaped < a.reward_min) shaped = a.reward_min;
+      if (shaped > a.reward_max) shaped = a.reward_max;
+    }
     if (a.value_bootstrap && a.timeouts[i]) shaped += a.gamma * a.values[i];   // Vine5LinkMovingBasePPO.yaml:56
     a.shaped_rewards[i] = shaped;
     a.dones_next[i] = d;

@@ -68,13 +68,15 @@ class NativeLstmPath:
 
     # ------------------------------------------------------------------ forward + backward of one minibatch
     def gradients(self, packed_mlp, packed_lstm, obs, scalars, not_done, obs_mean, obs_inv_std, value_stats, logstd, logstd_old,
-                  state, debug_out=None, writeback=None, p2p=(None, None)):
+                  state, debug_out=None, writeback=None, p2p=(None, None), position=(0, 0)):
         """obs f32 [L, S, O], scalars f32 [L, S, 8], not_done f32 [L, S]; self.HM[0] (masked initial hidden state tiles) and
         self.C0 must already hold the initial LSTM state.  Leaves the gradients in flat_g_mlp / flat_g_lstm.
         ``writeback`` = (scalars_src [T, N, 8], seq_len, chunks, num_envs, env_begin, env_count): rl_games'
         dataset.update_mu_sigma -- this pass's mu goes back into the source rows and ``logstd_old`` receives ``logstd``.
         ``p2p`` = (MLP channel, LSTM channel) device pointers: multi-GPU, the two gradient sums go into this rank's peer-visible
-        buffers instead of flat_g_* (distributed.P2PChannel)."""
+        buffers instead of flat_g_* (distributed.P2PChannel).  ``position`` = (mini-epoch, minibatch slot) of this minibatch
+        in the iteration: what the learning-rate schedule of vine_ppo_minibatch needs to know, passed to hyper["schedule"]
+        (PPOAgent._schedule_fields); without that entry the launch runs the adaptive legacy schedule."""
         lib, L, S, tl, st = self.lib, self.L, self.S, self.tiles, self._stream()
         n = L * S
         act = abi.VinePolicyAct(packed=_ptr(packed_mlp), obs=_ptr(obs), obs_mean=_ptr(obs_mean), obs_inv_std=_ptr(obs_inv_std),
@@ -92,7 +94,7 @@ class NativeLstmPath:
                                    logstd_old=_ptr(logstd_old), dh=_ptr(self.DH), grads=_ptr(self.head_grads),
                                    debug_out=_ptr(debug_out) if debug_out is not None else None, n=n, inv_B=1.0 / n,
                                    e_clip=h["e_clip"], critic_coef=h["critic_coef"], entropy_coef=h["entropy_coef"],
-                                   bounds_loss_coef=h["bounds_loss_coef"])
+                                   bounds_loss_coef=h["bounds_loss_coef"], value_loss_unclipped=int(not h.get("clip_value", True)))
         if writeback is not None:
             src, wl, wc, wn, wb, we = writeback
             ht.mu_writeback, ht.wb_seq_len, ht.wb_chunks, ht.wb_num_envs, ht.wb_env_begin, ht.wb_env_count = _ptr(src), wl, wc, wn, wb, we
@@ -108,12 +110,13 @@ class NativeLstmPath:
             bg = abi.VineLstmBwdGemm(params=_ptr(packed_lstm), dg=_ptr(self.DG[t]), not_done=_ptr(not_done[t]), dh3=_ptr(self.DH3[t]),
                                      dh_rec=_ptr(self.DHREC[t - 1]) if t else None, n=S)
             assert lib.vine_lstm_bwd_gemm(C.byref(bg), st) == 0
+        sched = h["schedule"](*position) if "schedule" in h else dict(
+            adaptive_lr=int(h.get("adaptive_lr", 1)), kl_threshold=h.get("kl_threshold", 0.008), lr_min=1e-6, lr_max=1e-2)
         mb = abi.VinePpoMinibatch(packed=_ptr(packed_mlp), obs=_ptr(obs), obs_mean=_ptr(obs_mean), obs_inv_std=_ptr(obs_inv_std),
                                   logstd=_ptr(logstd), logstd_old=_ptr(logstd_old), workspace=_ptr(self.mlp_ws), state=_ptr(state),
                                   horizon=1, num_envs=n, env_begin=0, env_count=n, num_obs=self.O, workspace_ctas=self.mlp_ctas,
-                                  adaptive_lr=int(h.get("adaptive_lr", 1)), kl_threshold=h.get("kl_threshold", 0.008), lr_min=1e-6,
-                                  lr_max=1e-2, e_clip=h["e_clip"], critic_coef=h["critic_coef"], entropy_coef=h["entropy_coef"],
-                                  bounds_loss_coef=h["bounds_loss_coef"], dh3_ext=_ptr(self.DH3))
+                                  e_clip=h["e_clip"], critic_coef=h["critic_coef"], entropy_coef=h["entropy_coef"],
+                                  bounds_loss_coef=h["bounds_loss_coef"], dh3_ext=_ptr(self.DH3), **sched)
         n_part = lib.vine_ppo_minibatch(C.byref(mb), st)
         assert n_part > 0, n_part
         wb = writeback is not None   # sigma half of update_mu_sigma: after the last reader of logstd_old, before Adam

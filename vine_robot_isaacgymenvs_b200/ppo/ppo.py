@@ -3,8 +3,9 @@
 Restates what rl-games 1.5.2's ``A2CAgent`` does for ``cfg/train/Vine5LinkMovingBasePPO.yaml``
 (``a2c_continuous`` / ``continuous_a2c_logstd`` / ``actor_critic``): horizon-16 rollouts, GAE
 (``vine_gae`` CUDA kernel), running mean/std of observations and values, advantage normalisation,
-clipped actor loss, clipped critic loss x critic_coef, bound loss, Adam with the ``legacy``
-adaptive-KL learning-rate schedule, value bootstrap on ``time_outs``, reward shaper.
+clipped actor loss, clipped (``clip_value``) critic loss x critic_coef, bound loss, Adam with the adaptive-KL or linear
+learning-rate schedule (``lr_schedule``) run per minibatch or per mini-epoch (``schedule_type``), value bootstrap on
+``time_outs``, reward shaper (scale, shift, clamp).
 In-repo analogue of the same math: isaacgymenvs/learning/common_agent.py:257-314 (rollout),
 :319-435 (update), :482-517 (losses).  rl_games itself is not vendored in the reference
 (setup.py:22) and not installed here: PARITY UNPINNED, checked by learning curves only.
@@ -155,6 +156,9 @@ def policy_kl(p0_mu, p0_sigma, p1_mu, p1_sigma):
     return (c1 + c2 - 0.5).sum(-1).mean()
 
 
+LR_MIN, LR_MAX = 1e-6, 1e-2   # rl_games AdaptiveScheduler's bounds; LinearScheduler's min_lr is LR_MIN too
+
+
 def rlgames_model_state(model, obs_rms, val_rms):
     """The ``model`` entry of an rl-games 1.5.2 checkpoint (``A2CBase.get_full_state_weights`` -> ``model.state_dict()`` of
     ``ModelA2CContinuousLogStd.Network``): the network under ``a2c_network.*``, the input normaliser under
@@ -188,8 +192,12 @@ class PPOAgent:
         assert self.minibatch % self.T == 0, "minibatch_size must be a multiple of horizon_length"
         self.mb_envs = self.minibatch // self.T
         self.kl_threshold = float(c["kl_threshold"])
-        self.adaptive = c.get("lr_schedule") == "adaptive"
-        self.reward_scale = float(c.get("reward_shaper", {}).get("scale_value", 1.0))
+        opts = self.update_options(train_cfg)
+        self.adaptive, self.linear_lr, self.schedule_standard = opts["adaptive"], opts["linear"], opts["standard"]
+        self.max_epochs, self.clip_value, self.lr0 = opts["max_epochs"], opts["clip_value"], float(c["learning_rate"])
+        self.reward_scale, self.reward_shift = opts["reward_scale"], opts["reward_shift"]
+        self.reward_min, self.reward_max = opts["reward_min"], opts["reward_max"]
+        self.reward_clamp = self.reward_min > -math.inf or self.reward_max < math.inf
         self.value_bootstrap = bool(c.get("value_bootstrap", False))
         self.normalize_input, self.normalize_value = bool(c["normalize_input"]), bool(c["normalize_value"])
         self.normalize_advantage = bool(c["normalize_advantage"])
@@ -247,6 +255,7 @@ class PPOAgent:
             self._init_fused_update(float(c["learning_rate"]))
         else:
             self.lr_t = torch.tensor(float(c["learning_rate"]), device=dev)   # device-side: no sync in the schedule
+            self._epoch_t = torch.zeros((), dtype=torch.float64, device=dev)    # rl_games epoch_num, for the linear schedule
             self.opt = torch.optim.Adam(self.model.parameters(), lr=self.lr_t, eps=1e-8, capturable=True)
         if self.grad_allreduce == "p2p":
             self._p2p_mlp = vd.P2PChannel(self._lib, self._lib.vine_ppo_num_params(self.O) + 4, dev)
@@ -283,6 +292,45 @@ class PPOAgent:
             self._val_stats = f(2)
             self._mu_buf, self._val_buf = f(n, self.A), f(n)
             self._refresh_fused(pack=True)
+
+    @staticmethod
+    def update_options(train_cfg):
+        """The rl_games keys of ``train.params.config`` that select the learning-rate schedule, the value loss and the reward
+        shaper, parsed and checked on a plain train-config dict (rl-games 1.5.2 semantics as recalled, DESIGN §9).  Every
+        update path (both kernel paths and the torch baseline) implements all of them; a value they cannot honour raises
+        here instead of being ignored.  lr_schedule values other than adaptive / linear mean a constant learning rate."""
+        c = train_cfg["params"]["config"]
+        sched, stype = c.get("lr_schedule"), c.get("schedule_type", "legacy")
+        if stype not in ("legacy", "standard"):
+            raise ValueError(f"schedule_type {stype!r}: must be 'legacy' (the lr rule after every minibatch) or 'standard' "
+                             "(after every mini-epoch, on its mean KL); rl_games would silently keep the learning rate constant")
+        max_epochs = int(c.get("max_epochs", -1))
+        if sched == "linear" and max_epochs <= 0:
+            raise ValueError(f"lr_schedule 'linear' decays the learning rate over max_epochs iterations: max_epochs must be > 0, "
+                             f"got {max_epochs}")
+        if c.get("schedule_entropy", False):
+            raise NotImplementedError("schedule_entropy: True (a linear schedule of entropy_coef) is not implemented: the "
+                                      "kernels read entropy_coef as a constant. Set schedule_entropy: False")
+        shaper = c.get("reward_shaper") or {}
+        if shaper.get("log_val", False):
+            raise NotImplementedError("reward_shaper.log_val: True (log of the shifted reward) is not implemented by the rollout "
+                                      "kernels or the torch rollout. Remove log_val or set it to False")
+        return {"adaptive": sched == "adaptive", "linear": sched == "linear", "standard": stype == "standard",
+                "max_epochs": max_epochs, "clip_value": bool(c.get("clip_value", True)),
+                "reward_scale": float(shaper.get("scale_value", 1.0)), "reward_shift": float(shaper.get("shift_value", 0.0)),
+                "reward_min": float(shaper.get("min_val", -math.inf)), "reward_max": float(shaper.get("max_val", math.inf))}
+
+    def _shaper_fields(self):
+        """Reward-shaper fields of VineRolloutPost."""
+        return dict(reward_scale=self.reward_scale, reward_shift=self.reward_shift, reward_min=self.reward_min,
+                    reward_max=self.reward_max, reward_clamp=int(self.reward_clamp))
+
+    def _schedule_fields(self, mini_epoch, slot):
+        """Learning-rate schedule and value-loss fields of the vine_ppo_minibatch launch of (mini-epoch, minibatch slot)."""
+        return dict(adaptive_lr=int(self.adaptive), lr_linear=int(self.linear_lr), schedule_standard=int(self.schedule_standard),
+                    epoch_begin=int(mini_epoch == 0 and slot == 0), mini_epoch_begin=int(slot == 0),
+                    max_epochs=max(self.max_epochs, 0), lr0=self.lr0, kl_threshold=self.kl_threshold, lr_min=LR_MIN,
+                    lr_max=LR_MAX, value_loss_unclipped=int(not self.clip_value))
 
     def _kernel_path_gaps(self, units, rnn_cfg, update=True):
         """Why the hand-written kernel path cannot run this configuration (empty list: it can)."""
@@ -380,7 +428,7 @@ class PPOAgent:
         self._clip_ws = z(abi.GRAD_CLIP_WS_FLOATS) if self.truncate_grads else None
         L, chunks, tiles_n = self.seq_len, self.T // self.seq_len, self.n // 128
         hyper = dict(e_clip=self.e_clip, critic_coef=self.critic_coef, entropy_coef=self.entropy_coef,
-                     bounds_loss_coef=self.bounds_coef, adaptive_lr=int(self.adaptive), kl_threshold=self.kl_threshold)
+                     bounds_loss_coef=self.bounds_coef, clip_value=self.clip_value, schedule=self._schedule_fields)
         self._path = NativeLstmPath(self.O, L, chunks * self.mb_envs, dev, hyper)
         from .lstm_native import TB
         bf = lambda *s: torch.zeros(*s, dtype=torch.bfloat16, device=dev)  # noqa: E731
@@ -435,9 +483,9 @@ class PPOAgent:
             post = abi.VineRolloutPost(rewards=ptr(env.rew_buf), resets=ptr(env.reset_buf), timeouts=ptr(env.timeout_buf),
                                        values=ptr(self.b_val[t]), shaped_rewards=ptr(self.b_rew[t]), dones_next=ptr(self._done_ext[t + 1]),
                                        ep_return=ptr(self.ep_ret), ep_length=ptr(self.ep_len), ep_stats=ptr(self.ep_stats),
-                                       rng_counter=ptr(self._rng_counter), n=n, reward_scale=self.reward_scale, gamma=self.gamma,
+                                       rng_counter=ptr(self._rng_counter), n=n, gamma=self.gamma,
                                        value_bootstrap=int(self.value_bootstrap), success_reward_threshold=self.success_threshold,
-                                       not_done_next=ptr(self._nd_ext[t + 1]))
+                                       not_done_next=ptr(self._nd_ext[t + 1]), **self._shaper_fields())
             assert lib.vine_rollout_post(C.byref(post), stream) == 0
         if self._r_cur != 0:   # odd horizon: keep the persistent state in buffer 0 so a captured graph can be replayed
             self._r_HH[0].copy_(self._r_HH[1])
@@ -477,7 +525,7 @@ class PPOAgent:
         path = self._path
         pm = self._p2p_mlp.ptr if self._p2p_mlp is not None else None
         pl = self._p2p_lstm.ptr if self._p2p_lstm is not None else None
-        for _ in range(self.mini_epochs):
+        for k in range(self.mini_epochs):
             for e0 in range(0, n, E):
                 # rows of the minibatch ordered [step in chunk][chunk, env] + the initial LSTM state of every sequence: one launch
                 ga = abi.VineLstmGather(obs=ptr(self.b_obs), scalars=ptr(self._scal), not_done=ptr(self._nd_ext),
@@ -488,7 +536,7 @@ class PPOAgent:
                 assert lib.vine_lstm_gather(C.byref(ga), stream) == 0
                 path.gradients(self._packed, self._lpacked, self._mb_obs, self._mb_scal, self._mb_nd, self._obs_mean_f,
                                self._obs_inv_std_f, self._val_stats, self.model.sigma, self._logstd_old[e0 // E], self.ppo_state,
-                               writeback=(self._scal, L, chunks, n, e0, E), p2p=(pm, pl))
+                               writeback=(self._scal, L, chunks, n, e0, E), p2p=(pm, pl), position=(k, e0 // E))
                 if self.grad_allreduce == "nccl":   # baseline: ONE NCCL all-reduce per minibatch (gradients + loss statistics)
                     torch.distributed.all_reduce(path.flat_g)
                 sc = 1.0 / self.world                # p2p: the Adam kernels add the ranks' buffers themselves (vine_p2p.cuh)
@@ -589,9 +637,9 @@ class PPOAgent:
                                          values=ptr(self.b_val[t]), shaped_rewards=ptr(self.b_rew[t]),
                                          dones_next=ptr(self._done_ext[t + 1]), ep_return=ptr(self.ep_ret),
                                          ep_length=ptr(self.ep_len), ep_stats=ptr(self.ep_stats),
-                                         rng_counter=ptr(self._rng_counter), n=n, reward_scale=self.reward_scale,
-                                         gamma=self.gamma, value_bootstrap=int(self.value_bootstrap),
-                                         success_reward_threshold=self.success_threshold) for t in range(T)]
+                                         rng_counter=ptr(self._rng_counter), n=n, gamma=self.gamma,
+                                         value_bootstrap=int(self.value_bootstrap), success_reward_threshold=self.success_threshold,
+                                         **self._shaper_fields()) for t in range(T)]
             last = abi.VinePolicyAct(mu=ptr(self._mu_buf), value=ptr(self.last_value), **common)
             self._roll_structs = (acts, posts, last)
         acts, posts, last = self._roll_structs
@@ -634,7 +682,7 @@ class PPOAgent:
             env.actions.copy_(torch.clamp(action, -1.0, 1.0))                  # rl_games preprocess_actions
             env.step_device()                                                  # ONE fused kernel launch
             rew, dones, timeouts = env.rew_buf, env.reset_buf, env.timeout_buf
-            shaped = rew * self.reward_scale
+            shaped = self._shape_rewards(rew)
             if self.value_bootstrap:                                           # Vine5LinkMovingBasePPO.yaml:56
                 shaped = shaped + self.gamma * value * timeouts.float()
             self.b_rew[t] = shaped
@@ -685,14 +733,24 @@ class PPOAgent:
             sigma.copy_(keep)
         return self.pop_stats()
 
+    def _shape_rewards(self, rew):
+        """rl_games DefaultRewardsShaper without log_val: clamp((r + shift) * scale, min_val, max_val); the shift is added only
+        when non-zero and the clamp applied only with a finite bound, so the default is exactly r * scale."""
+        r = rew + self.reward_shift if self.reward_shift != 0.0 else rew
+        r = r * self.reward_scale
+        return torch.clamp(r, self.reward_min, self.reward_max) if self.reward_clamp else r
+
     # ------------------------------------------------------------------ learning
     def _update_lr(self, kl):
-        if not self.adaptive:
-            return
-        lr = self.lr_t
-        lr = torch.where(kl > 2.0 * self.kl_threshold, torch.clamp(lr / 1.5, min=1e-6), lr)
-        lr = torch.where(kl < 0.5 * self.kl_threshold, torch.clamp(lr * 1.5, max=1e-2), lr)
-        self.lr_t.copy_(lr)
+        """One run of the learning-rate rule (rl_games scheduler.update) on the device-side lr; kl = the rank-mean KL."""
+        if self.adaptive:
+            lr = self.lr_t
+            lr = torch.where(kl > 2.0 * self.kl_threshold, torch.clamp(lr / 1.5, min=LR_MIN), lr)
+            lr = torch.where(kl < 0.5 * self.kl_threshold, torch.clamp(lr * 1.5, max=LR_MAX), lr)
+            self.lr_t.copy_(lr)
+        elif self.linear_lr:   # LinearScheduler(use_epochs=True), epoch = rl_games epoch_num of this iteration
+            left = torch.clamp(self.max_epochs - self._epoch_t, min=0.0)
+            self.lr_t.copy_(LR_MIN + (self.lr0 - LR_MIN) * (left / self.max_epochs))
 
     def _update(self):
         T, n, L = self.T, self.n, self.seq_len
@@ -717,6 +775,7 @@ class PPOAgent:
             # sigma of the policy each row was last evaluated with, per minibatch slot (rl_games dataset.update_mu_sigma)
             sigma_old = torch.exp(self.model.sigma.detach()).clone().expand(n // self.mb_envs, -1).clone()
             not_done = 1.0 - self.b_done
+            self._epoch_t += 1.0
         params = [p for p in self.model.parameters()]
         E = self.mb_envs
 
@@ -727,6 +786,7 @@ class PPOAgent:
             return y.reshape(L, (T // L) * E, *x.shape[2:])
 
         for _ in range(self.mini_epochs):
+            ep_kls = []
             for e0 in range(0, n, E):
                 o_mb = mb(obs, e0)                                             # [L, S, O]
                 flat = lambda x: mb(x, e0).reshape(L * (T // L) * E, *x.shape[2:])  # noqa: E731
@@ -743,8 +803,11 @@ class PPOAgent:
                 ratio = torch.exp(flat(nlp_old) - nlp)
                 a, vo, r = flat(adv), flat(val_old), flat(ret)
                 a_loss = torch.max(-a * ratio, -a * torch.clamp(ratio, 1.0 - self.e_clip, 1.0 + self.e_clip)).mean()
-                v_clip = vo + (value - vo).clamp(-self.e_clip, self.e_clip)
-                c_loss = torch.max((value - r) ** 2, (v_clip - r) ** 2).mean()
+                if self.clip_value:
+                    v_clip = vo + (value - vo).clamp(-self.e_clip, self.e_clip)
+                    c_loss = torch.max((value - r) ** 2, (v_clip - r) ** 2).mean()
+                else:
+                    c_loss = ((value - r) ** 2).mean()
                 b_loss = (torch.clamp_min(mu - 1.1, 0.0) ** 2 + torch.clamp_max(mu + 1.1, 0.0) ** 2).sum(-1).mean()
                 entropy = (0.5 + 0.5 * math.log(2 * math.pi) + logstd).sum(-1).mean()
                 loss = a_loss + 0.5 * c_loss * self.critic_coef - self.entropy_coef * entropy + b_loss * self.bounds_coef
@@ -768,9 +831,15 @@ class PPOAgent:
                         nn.utils.clip_grad_norm_(params, self.grad_norm)
                 self.opt.step()
                 with torch.no_grad():
-                    self._update_lr(kl)
+                    if self.schedule_standard:
+                        ep_kls.append(kl)
+                    else:
+                        self._update_lr(kl)
                     self.loss_stats += torch.stack([a_loss.detach(), c_loss.detach(), kl,
                                                     torch.ones((), device=kl.device)]).double()
+            if self.schedule_standard:   # rl_games schedule_type standard: once per mini-epoch, on its mean KL
+                with torch.no_grad():
+                    self._update_lr(torch.stack(ep_kls).mean())
         if self.fused or self.native_lstm:
             self._refresh_fused(pack=True)
 
@@ -798,19 +867,20 @@ class PPOAgent:
         self._logstd_old.copy_(self.model.sigma.expand_as(self._logstd_old))
         if self._mb_structs is None:
             ptr = lambda x: x.data_ptr()  # noqa: E731
-            self._mb_structs = [abi.VinePpoMinibatch(
+            self._mb_structs = [[abi.VinePpoMinibatch(
                 packed=ptr(self._packed), obs=ptr(self.b_obs), actions=ptr(self.b_act), mu_old=ptr(self.b_mu),
                 neglogp_old=ptr(self.b_nlp), values_old=ptr(self._val_old_n), returns=ptr(self._ret_n),
                 advantages=ptr(self._adv_n), obs_mean=ptr(self._obs_mean_f), obs_inv_std=ptr(self._obs_inv_std_f),
                 logstd=ptr(self.model.sigma), logstd_old=ptr(self._logstd_old[e0 // self.mb_envs]), workspace=ptr(self._ws),
                 state=ptr(self.ppo_state), debug_out=None, horizon=T, num_envs=n, env_begin=e0, env_count=self.mb_envs,
-                num_obs=self.O, workspace_ctas=self._ctas, adaptive_lr=int(self.adaptive), e_clip=self.e_clip,
-                critic_coef=self.critic_coef, entropy_coef=self.entropy_coef, bounds_loss_coef=self.bounds_coef,
-                kl_threshold=self.kl_threshold, lr_min=1e-6, lr_max=1e-2) for e0 in range(0, n, self.mb_envs)]
+                num_obs=self.O, workspace_ctas=self._ctas, e_clip=self.e_clip, critic_coef=self.critic_coef,
+                entropy_coef=self.entropy_coef, bounds_loss_coef=self.bounds_coef, **self._schedule_fields(k, e0 // self.mb_envs))
+                for e0 in range(0, n, self.mb_envs)] for k in range(self.mini_epochs)]   # one per (mini-epoch, slot): the schedule
+                                                                                       # needs to know which launch opens what
         p = lambda x: C.c_void_p(x.data_ptr())  # noqa: E731
         pm = self._p2p_mlp.ptr if self._p2p_mlp is not None else None
-        for _ in range(self.mini_epochs):
-            for slot, mb in enumerate(self._mb_structs):
+        for k in range(self.mini_epochs):
+            for slot, mb in enumerate(self._mb_structs[k]):
                 # forward + losses + backward; writes this pass's mu over the rows' mu_old (rl_games dataset.update_mu_sigma)
                 n_part = lib.vine_ppo_minibatch(C.byref(mb), stream)
                 assert n_part > 0, n_part
@@ -957,5 +1027,10 @@ class PPOAgent:
             self._rng_counter.fill_(int(sd["vine_rng_counter"]))
         self.epoch, self.frames = sd.get("epoch", 0), sd.get("frame", 0)
         self.lr_t.fill_(float(sd.get("last_lr", self.lr)))
+        # the iteration counter of the linear schedule: a resumed run continues its learning-rate sequence
+        if self.fused_update:
+            self.ppo_state[abi.PPO_STATE_EPOCH] = float(self.epoch)
+        else:
+            self._epoch_t.fill_(float(self.epoch))
         if self.fused or self.native_lstm:
             self._refresh_fused(pack=True)
