@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define VINE_ABI_VERSION 5
+#define VINE_ABI_VERSION 6
 
 #define VINE_NUM_DOFS 6          /* 1 prismatic rail cart + 5 revolute links (V5:54,83) */
 #define VINE_NUM_ACTIONS 2       /* u_rail_velocity, u_fpam (V5:171) */
@@ -434,6 +434,9 @@ typedef struct VinePolicyAct {
   void* u_out;                   /* NULL, or [ceil(n/128)] tiles [128 x 128] bf16 (UMMA row-blocked): the LSTM input
                                     [MLP output (64) | normalised obs (32, col 31 == 1) | 0]; heads and sampling are
                                     skipped (they follow the LSTM: vine_lstm_step / vine_lstm_head) */
+  int32_t u_step_rows, u_step_seqs;   /* with u_out: rows come in groups of u_step_rows (one time step of a minibatch padded to
+                                    whole tiles), of which the first u_step_seqs are real; the rest read no observation and
+                                    get the U row of a zero input.  0, 0: every row is real */
 } VinePolicyAct;
 int vine_policy_act(const VinePolicyAct* args, void* stream);
 
@@ -518,6 +521,8 @@ typedef struct VineLstmStep {
   void* hm_next;                 /* NULL or like hh */
   void* act;                     /* NULL or [tiles][16][128 x 64] bf16 activated gates */
   int64_t n;
+  int64_t hm_next_rows;          /* 0, or n <= hm_next_rows <= tiles * 128: rows [n, hm_next_rows) of hm_next are written as
+                                    zeros (padded sequences of a minibatch); every other output row past n is left alone */
 } VineLstmStep;
 typedef struct VineLstmHead {
   const void* params;
@@ -562,20 +567,23 @@ typedef struct VineLstmHeadTrain {
   float* grads;                  /* [VINE_LSTM_HEAD_GRAD_PARTS][VINE_LSTM_HEAD_GRAD_FLOATS] per-block partials */
   float* debug_out;              /* NULL or [n, 4]: mu0, mu1, normalised value, neglogp */
   int64_t n;
-  float e_clip, critic_coef, entropy_coef, bounds_loss_coef, inv_B, reserved_f;
+  float e_clip, critic_coef, entropy_coef, bounds_loss_coef, inv_B;   /* inv_B = 1 / number of real rows */
+  int32_t step_rows;             /* rows per time step (sequences padded to whole tiles); 0: every row is real */
   /* rl_games dataset.update_mu_sigma: NULL, or the [T, N, 8] scalars buffer this minibatch was gathered from; the kernel
-   * stores this pass's mu into columns 2,3 of the source row of every minibatch row (rows = [step in chunk][chunk][env]) */
+   * stores this pass's mu into columns 2,3 of the source row of every real minibatch row (rows = [step in chunk][chunk][env]) */
   float* mu_writeback;
   int64_t wb_seq_len, wb_chunks, wb_num_envs, wb_env_begin, wb_env_count;
   int32_t value_loss_unclipped;  /* 0: clipped value loss (rl_games clip_value True); 1: c_loss = (return - v)^2 */
-  int32_t reserved2;             /* 0 */
+  int32_t step_seqs;             /* with step_rows: the real sequences at the start of every step; the other (padded) rows
+                                    add nothing to the losses, statistics and gradients, get dh = 0 and no mu write-back */
 } VineLstmHeadTrain;
 int vine_lstm_head_train(const VineLstmHeadTrain* args, void* stream);
 
 /*
  * Backward through one LSTM time step of a minibatch (truncated BPTT, steps visited in reverse):
  *   vine_lstm_cell_bwd_tiles : pointwise; from the activated gates, c_prev, c, dh (from the head) [+ dh_rec from the
- *       following step, already masked] and dc_next -> dG (bf16 tiles like act) and dc_prev.
+ *       following step, already masked] and dc_next -> dG (bf16 tiles like act) and dc_prev.  The rows of the last tile
+ *       past n get dG = 0 (padded sequences of a minibatch).
  *   vine_lstm_bwd_gemm : d[u(:, 0:64) | hm] = dG W (tcgen05; the 1024 gate rows streamed as 16 pieces through a 3-stage
  *       ring of bulk-TMA copies; the forward weight pieces are read as MN-major operands): dh3 f32 [n, 64] = gradient of
  *       the MLP output, dh_rec = not_done * d(hm) as bf16 tiles for the previous step (NULL at the first step).
@@ -596,9 +604,10 @@ typedef struct VineLstmBwdGemm {
   const void* params;
   const void* dg;
   const float* not_done;         /* [n] mask applied to dh_rec (NULL = 1) */
-  float* dh3;                    /* out [n, 64] */
+  float* dh3;                    /* out [dh3_rows, 64] */
   void* dh_rec;                  /* out tiles like hh, or NULL */
   int64_t n;
+  int64_t dh3_rows;              /* 0 (= n), or n <= dh3_rows <= tiles * 128: rows [n, dh3_rows) of dh3 are written as zeros */
 } VineLstmBwdGemm;
 int vine_lstm_cell_bwd_tiles(const VineLstmCellBwd* args, void* stream);
 int vine_lstm_bwd_gemm(const VineLstmBwdGemm* args, void* stream);
@@ -609,7 +618,9 @@ int vine_lstm_bwd_gemm(const VineLstmBwdGemm* args, void* stream);
  *   b_v[1] logstd[2]                                   (vine_lstm_num_params(O) floats)
  *   vine_lstm_wgrad : dW^T = in^T dG over all (step, sequence) rows of the minibatch (tcgen05, both operands MN-major,
  *       rows streamed through a 2-stage bulk-TMA ring); grid = 12 output blocks x `splits` K ranges; partials go to
- *       workspace f32 [splits][12][128][256].  ntiles = number of 128-row tiles of u / hm / dg (all steps).
+ *       workspace f32 [splits][12][128][256].  ntiles = number of 128-row tiles of u / hm / dg (all steps).  A padded row
+ *       adds exactly nothing: its dG is 0 (vine_lstm_cell_bwd_tiles) and its u / hm are finite (vine_policy_act
+ *       u_step_*, vine_lstm_step, vine_lstm_gather).
  *   vine_lstm_reduce : flat[p] = gradient of parameter p (sum of the partials; b_ih/b_hh from the constant-1 column
  *       of u; LayerNorm / heads / logstd from the head gradient buffer); flat[P..P+3] = a_loss, c_loss, kl, b_loss.
  *   vine_lstm_adam : torch.optim.Adam on the flat vector + in-place update of the packed block + the loss / KL
@@ -619,20 +630,23 @@ int vine_lstm_bwd_gemm(const VineLstmBwdGemm* args, void* stream);
  * Minibatch assembly of the recurrent update in one launch: envs [env_begin, env_begin+env_count) x all horizon steps of
  * the [T, N] rollout buffers -> rows ordered [step in chunk][chunk, env] (T = chunks * seq_len; sequences = chunks *
  * env_count), plus the initial cell state and the masked initial hidden-state tiles of every sequence from the snapshots the
- * rollout took at the chunk starts.  num_envs, env_begin and env_count must be multiples of 128.
+ * rollout took at the chunk starts.  Each step's rows are padded to step_rows (the minibatch layout of the recurrent update:
+ * sequences rounded up to whole 128-row tiles); a padded sequence gets zero observations, scalars, not_done, c0 and hm0.
  */
 typedef struct VineLstmGather {
   const float* obs;              /* [T, N, O] */
   const float* scalars;          /* [T, N, 8] */
   const float* not_done;         /* [T, N] */
   const float* c_saved;          /* [chunks, N, 256] */
-  const void* hh_saved;          /* [chunks][N/128][2][128 x 128] bf16 */
-  float* mb_obs;                 /* [L, S, O] out */
-  float* mb_scalars;             /* [L, S, 8] out */
-  float* mb_not_done;            /* [L, S] out */
-  float* c0;                     /* [S, 256] out */
-  void* hm0;                     /* [S/128][2][128 x 128] bf16 out: not_done[first step] * h */
+  const void* hh_saved;          /* [chunks][ceil(N/128)][2][128 x 128] bf16 */
+  float* mb_obs;                 /* [L, R, O] out */
+  float* mb_scalars;             /* [L, R, 8] out */
+  float* mb_not_done;            /* [L, R] out */
+  float* c0;                     /* [R, 256] out */
+  void* hm0;                     /* [ceil(R/128)][2][128 x 128] bf16 out: not_done[first step] * h */
   int32_t seq_len, chunks, num_envs, env_begin, env_count, num_obs;
+  int32_t step_rows;             /* R = rows per step of the outputs, >= S = chunks * env_count; 0: R = S */
+  int32_t reserved;              /* 0 */
 } VineLstmGather;
 int vine_lstm_gather(const VineLstmGather* args, void* stream);
 
@@ -722,9 +736,10 @@ typedef struct VinePpoMinibatch {
   int32_t horizon, num_envs, env_begin, env_count, num_obs, workspace_ctas, adaptive_lr;
   int32_t reserved;              /* 0; 2 selects two (instead of four) epilogue threads per row, an A/B switch for profiling */
   float e_clip, critic_coef, entropy_coef, bounds_loss_coef, kl_threshold, lr_min, lr_max, reserved_f;
-  const float* dh3_ext;          /* NULL, or f32 [T*env_count, 64]: d(loss)/d(MLP output) supplied by the LSTM backward
-                                    (vine_lstm_bwd_gemm); the heads and losses are skipped and the loss pointers may be
-                                    NULL -- the kernel recomputes the MLP forward and back-propagates from there */
+  const float* dh3_ext;          /* NULL, or f32 [T, N, 64] (rows like obs; only the minibatch's rows are read): d(loss)/d(MLP
+                                    output) supplied by the LSTM backward (vine_lstm_bwd_gemm); the heads and losses are
+                                    skipped and the loss pointers may be NULL -- the kernel recomputes the MLP forward and
+                                    back-propagates from there */
   int32_t lr_linear;             /* 1: linear schedule (adaptive_lr must be 0; max_epochs > 0) */
   int32_t schedule_standard;     /* 0: rl_games schedule_type legacy, 1: standard (see above) */
   int32_t epoch_begin;           /* 1: this launch opens a training iteration */

@@ -1,7 +1,10 @@
 """Time one PPO iteration of the reference network (MLP -> LSTM 256 -> LayerNorm) at FSTR, N envs, CUDA-graph replay:
-python tools/ppo_time.py [N] [--mlp] [--no-pdl] [--no-arena] [--pad K] [--truncate-grads [--grad-norm X]]
-Prints ms per iteration / rollout / update (CUDA events, best of 3 x 20).  --truncate-grads also builds a second agent with
-gradient-norm clipping (truncate_grads=True, grad_norm X, default 1.0) and times the two update graphs alternately."""
+python tools/ppo_time.py [N] [--minibatch M] [--mlp] [--no-pdl] [--no-arena] [--pad K] [--truncate-grads [--grad-norm X]]
+Prints ms per iteration / rollout / update (CUDA events, best of 3 x 20) and the card with its power limit.  --minibatch sets
+minibatch_size (default: the config's 32768, which needs N * horizon to be a multiple of it; e.g. N = 4000 wants 32000).
+--truncate-grads also builds a second agent with gradient-norm clipping (truncate_grads=True, grad_norm X, default 1.0) and
+times the two update graphs alternately."""
+import subprocess
 import sys
 
 import torch
@@ -14,6 +17,8 @@ from vine_robot_isaacgymenvs_b200.ppo.ppo import PPOAgent  # noqa: E402
 args = [a for a in sys.argv[1:]]
 n = int(args[0]) if args and args[0].isdigit() else 4096
 extra = ["train.params.network.rnn=null"] if "--mlp" in args else []
+if "--minibatch" in args:
+    extra.append(f"train.params.config.minibatch_size={int(args[args.index('--minibatch') + 1])}")
 if "--no-pdl" in args:
     PPOAgent.PDL_MAX_ENVS = 0
 if "--no-arena" in args:
@@ -58,10 +63,11 @@ it = best(agent.train_epoch)
 ro = best(agent.play_steps)
 up = best(agent._g_update.replay if agent._g_update is not None else agent._update_any)
 st = agent.pop_stats()
+_q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader", "-i", "0"], capture_output=True, text=True)
 print(f"n={n} {' '.join(args[1:])}: iteration {it:.3f} ms  rollout {ro:.3f}  update {up:.3f}  frames/s {n * agent.T / it * 1e3:.4g}  "
-      f"kl {st['kl']:.4g} a_loss {st['a_loss']:.4g} c_loss {st['c_loss']:.4g}", flush=True)
+      f"kl {st['kl']:.4g} a_loss {st['a_loss']:.4g} c_loss {st['c_loss']:.4g}  "
+      f"[{_q.stdout.strip() or torch.cuda.get_device_name(0)}]", flush=True)
 if clip_agent is not None:   # update graph without / with clipping, alternating; the card and its power limit of this run
-    import subprocess
     off, on = [], []
     for _ in range(5):
         off.append(best(agent._g_update.replay))

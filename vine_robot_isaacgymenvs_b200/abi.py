@@ -12,7 +12,7 @@ NUM_ACTIONS = 2
 NUM_REWARDS = 13
 NUM_OBJECT_INFO = 2
 MAX_ACTION_DELAY = 8
-ABI_VERSION = 5
+ABI_VERSION = 6
 
 OK = 0
 ERR_INVALID_ARG = -1
@@ -166,12 +166,12 @@ class VinePolicyAct(C.Structure):
         "packed", "obs", "obs_mean", "obs_inv_std", "value_stats", "mu", "value", "logstd", "rng_counter", "actions",
         "neglogp", "obs_copy", "env_actions")]
         + [("n", C.c_int64), ("num_obs", C.c_int32), ("reserved", C.c_int32), ("seed", C.c_uint64),
-           ("global_env_offset", C.c_int64), ("u_out", C.c_void_p)])
+           ("global_env_offset", C.c_int64), ("u_out", C.c_void_p), ("u_step_rows", C.c_int32), ("u_step_seqs", C.c_int32)])
 
 
 class VineLstmStep(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in ("params", "u", "hm", "c_prev", "not_done", "not_done_next", "c", "hh", "hm_next",
-                                          "act")] + [("n", C.c_int64)]
+                                          "act")] + [("n", C.c_int64), ("hm_next_rows", C.c_int64)]
 
 
 class VineLstmHead(C.Structure):
@@ -183,10 +183,10 @@ class VineLstmHead(C.Structure):
 class VineLstmHeadTrain(C.Structure):
     _fields_ = ([(n, C.c_void_p) for n in ("params", "hh", "scalars", "logstd", "logstd_old", "dh", "grads", "debug_out")]
                 + [("n", C.c_int64)]
-                + [(n, C.c_float) for n in ("e_clip", "critic_coef", "entropy_coef", "bounds_loss_coef", "inv_B", "reserved_f")]
-                + [("mu_writeback", C.c_void_p)]
+                + [(n, C.c_float) for n in ("e_clip", "critic_coef", "entropy_coef", "bounds_loss_coef", "inv_B")]
+                + [("step_rows", C.c_int32), ("mu_writeback", C.c_void_p)]
                 + [(n, C.c_int64) for n in ("wb_seq_len", "wb_chunks", "wb_num_envs", "wb_env_begin", "wb_env_count")]
-                + [("value_loss_unclipped", C.c_int32), ("reserved2", C.c_int32)])
+                + [("value_loss_unclipped", C.c_int32), ("step_seqs", C.c_int32)])
 
 
 class VineLstmCellBwd(C.Structure):
@@ -194,13 +194,14 @@ class VineLstmCellBwd(C.Structure):
 
 
 class VineLstmBwdGemm(C.Structure):
-    _fields_ = [(n, C.c_void_p) for n in ("params", "dg", "not_done", "dh3", "dh_rec")] + [("n", C.c_int64)]
+    _fields_ = [(n, C.c_void_p) for n in ("params", "dg", "not_done", "dh3", "dh_rec")] + [("n", C.c_int64), ("dh3_rows", C.c_int64)]
 
 
 class VineLstmGather(C.Structure):
     _fields_ = ([(n, C.c_void_p) for n in ("obs", "scalars", "not_done", "c_saved", "hh_saved", "mb_obs", "mb_scalars", "mb_not_done",
                                            "c0", "hm0")]
-                + [(n, C.c_int32) for n in ("seq_len", "chunks", "num_envs", "env_begin", "env_count", "num_obs")])
+                + [(n, C.c_int32) for n in ("seq_len", "chunks", "num_envs", "env_begin", "env_count", "num_obs",
+                                             "step_rows", "reserved")])
 
 
 class VineLstmWgrad(C.Structure):

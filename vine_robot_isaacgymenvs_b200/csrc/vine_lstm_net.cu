@@ -212,8 +212,11 @@ __global__ void __launch_bounds__(STEP_THREADS, 1) vine_lstm_step_kernel(const V
       fence_before_sync();
       __syncwarp();
       if ((tid & 31) == 0) mbar_arrive(acc_empty(b));   // this warp's lanes hold their accumulator values in registers
-      if (!valid) continue;
       const int piece = piece0 + p, unit0 = 16 * piece + 8 * sub;
+      if (!valid) {   // a padded row of a minibatch: hm_next is an operand of vine_lstm_wgrad, so it gets zeros, never stale bytes
+        if (hm_t && s < a.hm_next_rows) *reinterpret_cast<uint4*>(hm_t + tile_offset(row, unit0 % UK, UK)) = make_uint4(0u, 0u, 0u, 0u);
+        continue;
+      }
       const float* sb = reinterpret_cast<const float*>(smem + SO_BIAS) + p * PIECE_ROWS + 8 * sub;
       const float cp[8] = {c0.x, c0.y, c0.z, c0.w, c1.x, c1.y, c1.z, c1.w};
       float cn[8], hn[8], ai[8], af[8], ag[8], ao[8];
@@ -358,6 +361,9 @@ static_assert(HG_FLOATS == VINE_LSTM_HEAD_GRAD_FLOATS, "header constant out of d
 // LayerNorm gain/bias and of the head weights are linear in those sums and are assembled once per block at the end.
 constexpr int HT_ROWS = 2;
 
+// PADDED: the minibatch has padded rows (step_rows != 0).  A separate instantiation, so that the dense rows of an aligned
+// minibatch run the same code as before padding existed (the padded-row tests cost registers in this 128-register kernel).
+template <bool PADDED>
 __global__ void __launch_bounds__(256, 2) vine_lstm_head_train_kernel(const VineLstmHeadTrain a) {
   vine_launch::grid_dependency_sync();
   __shared__ float red[HG_FLOATS];
@@ -391,6 +397,9 @@ __global__ void __launch_bounds__(256, 2) vine_lstm_head_train_kernel(const Vine
   const float klq0 = 1.f / (2.f * (sigo0 * sigo0 + 1e-5f)), klq1 = 1.f / (2.f * (sigo1 * sigo1 + 1e-5f));
   const float lo = 1.f - a.e_clip, hi = 1.f + a.e_clip;
   const bool clip_value = !a.value_loss_unclipped;   // rl_games clip_value
+  // rows come in steps of step_rows, of which the first step_seqs are real; the rest pad each step to whole tiles
+  // (32-bit: the host keeps n below 2^31 when step_rows is set; a 64-bit remainder is a call that spills the row state)
+  auto real = [&](int64_t s) { return !PADDED || (uint32_t)s % (uint32_t)a.step_rows < (uint32_t)a.step_seqs; };
   __syncthreads();
   auto load8 = [&](int arr, float* v) {
     const float4 x = prm[arr][0][lane], y = prm[arr][1][lane];
@@ -405,8 +414,8 @@ __global__ void __launch_bounds__(256, 2) vine_lstm_head_train_kernel(const Vine
 #pragma unroll
     for (int r = 0; r < HT_ROWS; ++r) {   // every load of the rows in flight is issued before anything waits on one
       const int64_t s = s0 + r * nwarps;
-      ok[r] = s < a.n;
-      srow[r] = ok[r] ? s : s0;
+      ok[r] = s < a.n && real(s);
+      srow[r] = ok[r] ? s : (real(s0) ? s0 : 0);   // a row that is not real computes on a real row's (finite) data, weight 0
       const int64_t tile = srow[r] / TILE;
       const int row = (int)(srow[r] % TILE), unit = 8 * lane;
       off[r] = ((size_t)tile * 2 + unit / UK) * TILE_BYTES + tile_offset(row, unit % UK, UK);
@@ -487,7 +496,7 @@ __global__ void __launch_bounds__(256, 2) vine_lstm_head_train_kernel(const Vine
       dmu1 += a.bounds_loss_coef * 2.f * (bh1 + bl1);
       const float m0 = mu0 - muo0, m1 = mu1 - muo1;
       const float kl = klc0 + (sig0 * sig0 + m0 * m0) * klq0 + klc1 + (sig1 * sig1 + m1 * m1) * klq1;
-      const float w = ok[r] ? a.inv_B : 0.f;   // a row past the end contributes nothing
+      const float w = ok[r] ? a.inv_B : 0.f;   // a row past the end or a padded row contributes nothing
       dmu0 *= w, dmu1 *= w, dv *= w;
       gr[r][0] = dmu0, gr[r][1] = dmu1, gr[r][2] = dv;
       sc[0] += dmu0, sc[1] += dmu1, sc[2] += dv;
@@ -497,7 +506,7 @@ __global__ void __launch_bounds__(256, 2) vine_lstm_head_train_kernel(const Vine
       if (lane == 0 && ok[r]) {
         const int64_t s = srow[r];
         if (a.mu_writeback) {   // dataset.update_mu_sigma: row s = [step l][chunk c][env e] of the minibatch -> row (c L + l, e0 + e) of [T, N, 8]
-          const int64_t per_step = a.wb_chunks * a.wb_env_count;
+          const int64_t per_step = PADDED ? a.step_rows : a.wb_chunks * a.wb_env_count;
           const int64_t l = s / per_step, rem = s - l * per_step, c = rem / a.wb_env_count, e = rem - c * a.wb_env_count;
           float* dst = a.mu_writeback + ((c * a.wb_seq_len + l) * a.wb_num_envs + a.wb_env_begin + e) * 8 + 2;
           *reinterpret_cast<float2*>(dst) = make_float2(mu0, mu1);
@@ -543,6 +552,12 @@ __global__ void __launch_bounds__(256, 2) vine_lstm_head_train_kernel(const Vine
         o[k] = pack_bf16(rstd[r] * (dyh[r][2 * k] - mean1 - yh[r][2 * k] * mean2),
                          rstd[r] * (dyh[r][2 * k + 1] - mean1 - yh[r][2 * k + 1] * mean2));
       if (ok[r]) *reinterpret_cast<uint4*>(reinterpret_cast<uint8_t*>(a.dh) + off[r]) = make_uint4(o[0], o[1], o[2], o[3]);
+      else if (PADDED && s0 + r * nwarps < a.n) {   // padded row: dh = 0 (at its own offset; off[r] is that of the row it computed on)
+        const int64_t s = s0 + r * nwarps;
+        const int unit = 8 * lane;
+        *reinterpret_cast<uint4*>(reinterpret_cast<uint8_t*>(a.dh) + ((size_t)(s / TILE) * 2 + unit / UK) * TILE_BYTES +
+                                  tile_offset((int)(s % TILE), unit % UK, UK)) = make_uint4(0u, 0u, 0u, 0u);
+      }
     }
   }
   // ---- the parameter gradients from the sums: with y = yh g + b and dy = sum_j d_j w_j,
@@ -586,10 +601,14 @@ __global__ void __launch_bounds__(CB_THREADS) vine_lstm_cell_bwd_tiles_kernel(co
   vine_launch::grid_dependency_sync();
   const int tile = blockIdx.x, piece = blockIdx.y, row = threadIdx.x >> 2, q = threadIdx.x & 3;
   const int64_t s = (int64_t)tile * TILE + row;
-  if (s >= a.n) return;
   const int col = 4 * q, unit0 = 16 * piece + col;
-  const uint8_t* at = reinterpret_cast<const uint8_t*>(a.act) + ((size_t)tile * NPIECE + piece) * ACT_BYTES;
   uint8_t* dg = reinterpret_cast<uint8_t*>(a.dg) + ((size_t)tile * NPIECE + piece) * ACT_BYTES;
+  if (s >= a.n) {   // a padded row of the last tile: dG = 0, so it adds nothing to vine_lstm_bwd_gemm and vine_lstm_wgrad
+#pragma unroll
+    for (int j = 0; j < 4; ++j) *reinterpret_cast<uint2*>(dg + tile_offset(row, 16 * j + col, PIECE_ROWS)) = make_uint2(0u, 0u);
+    return;
+  }
+  const uint8_t* at = reinterpret_cast<const uint8_t*>(a.act) + ((size_t)tile * NPIECE + piece) * ACT_BYTES;
   auto ld4 = [&](const uint8_t* p, float (&o)[4]) {
     const uint2 v = __ldg(reinterpret_cast<const uint2*>(p));
     const float2 f0 = unpack_bf16(v.x), f1 = unpack_bf16(v.y);
@@ -707,11 +726,15 @@ __global__ void __launch_bounds__(THREADS, 1) vine_lstm_bwd_gemm_kernel(const Vi
   mbar_wait(fin, 0);
   fence_after_sync();
   const int64_t s = (int64_t)tile * TILE + row;
-  const float m = (s < a.n && a.not_done) ? a.not_done[s] : 1.f;
+  const bool valid = s < a.n;   // a padded row's dh3 and dh_rec are written as zeros
+  const float m = (valid && a.not_done) ? a.not_done[s] : 1.f;
   if (part == 0) {
     uint32_t r[32];
     tmem_ld32(lane_base + BG_TM_DU + half * 32, r);
-    if (s < a.n) {
+    if (!valid)
+#pragma unroll
+      for (int i = 0; i < 32; ++i) r[i] = 0u;
+    if (s < (a.dh3_rows ? a.dh3_rows : a.n)) {
       float4* dst = reinterpret_cast<float4*>(a.dh3 + s * H3 + half * 32);
 #pragma unroll
       for (int i = 0; i < 8; ++i)
@@ -722,7 +745,10 @@ __global__ void __launch_bounds__(THREADS, 1) vine_lstm_bwd_gemm_kernel(const Vi
   for (int c0 = half * 64; c0 < half * 64 + 64; c0 += 32) {   // this thread: hidden units 128*part + c0 .. +31 of its row
     uint32_t r[32];
     tmem_ld32(lane_base + BG_TM_DH + c0, r);
-    if (a.dh_rec && s < a.n) {
+    if (!valid)
+#pragma unroll
+      for (int i = 0; i < 32; ++i) r[i] = 0u;
+    if (a.dh_rec) {
       uint8_t* dst = reinterpret_cast<uint8_t*>(a.dh_rec) + ((size_t)tile * 2 + part) * TILE_BYTES;
 #pragma unroll
       for (int q = 0; q < 4; ++q)
@@ -992,52 +1018,63 @@ __global__ void vine_lstm_adam_kernel(const float* __restrict__ flat, float scal
 // ---------------------------------------------------------------------------------------------------------------
 // Minibatch assembly for the recurrent update in ONE launch: rows ordered [step in chunk][chunk, env] gathered from the
 // [T, N] rollout buffers (observations, loss scalars, not_done), the initial cell state and the masked initial hidden-state
-// tiles of every sequence (saved at the chunk starts of the rollout).
+// tiles of every sequence (saved at the chunk starts of the rollout).  Each step holds R rows: the S sequences, then R - S
+// padded ones (zero observations, scalars, not_done and initial state), so that every step starts on a whole tile.
 __global__ void __launch_bounds__(256) vine_lstm_gather_kernel(const VineLstmGather a) {
   vine_launch::grid_dependency_sync();
-  const int64_t S = (int64_t)a.chunks * a.env_count;
+  const int64_t S = (int64_t)a.chunks * a.env_count, R = a.step_rows ? a.step_rows : S;
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   // one piece of (obs | scalars | not_done) per thread: obs in float2 pieces when the width is even (8-byte aligned rows),
   // scalars as two float4, not_done as one float; the host checked that rows * pieces fits 32 bits
   const bool even = (a.num_obs & 1) == 0;
   const unsigned OP = even ? a.num_obs / 2 : a.num_obs, W = OP + 3;
-  const unsigned rows = (unsigned)(a.seq_len * S);
+  const unsigned rows = (unsigned)(a.seq_len * R);
   if (i < (int64_t)rows * W) {
-    const unsigned iu = (unsigned)i, r = iu / W, c = iu - r * W, Su = (unsigned)S, t = r / Su, sq = r - t * Su;
-    const unsigned ck = sq / (unsigned)a.env_count, e = (unsigned)a.env_begin + (sq - ck * (unsigned)a.env_count);
+    const unsigned iu = (unsigned)i, r = iu / W, c = iu - r * W, Ru = (unsigned)R, t = r / Ru, sq = r - t * Ru;
+    const bool real = sq < (unsigned)S;
+    const unsigned ck = real ? sq / (unsigned)a.env_count : 0u, e = real ? (unsigned)a.env_begin + (sq - ck * (unsigned)a.env_count) : 0u;
     const int64_t src = ((int64_t)ck * a.seq_len + t) * a.num_envs + e;
     if (c < OP) {
-      if (even) reinterpret_cast<float2*>(a.mb_obs + (int64_t)r * a.num_obs)[c] = __ldg(reinterpret_cast<const float2*>(a.obs + src * a.num_obs) + c);
-      else a.mb_obs[(int64_t)r * a.num_obs + c] = __ldg(a.obs + src * a.num_obs + c);
+      if (even) reinterpret_cast<float2*>(a.mb_obs + (int64_t)r * a.num_obs)[c] =
+          real ? __ldg(reinterpret_cast<const float2*>(a.obs + src * a.num_obs) + c) : make_float2(0.f, 0.f);
+      else a.mb_obs[(int64_t)r * a.num_obs + c] = real ? __ldg(a.obs + src * a.num_obs + c) : 0.f;
     } else if (c < OP + 2) {
-      reinterpret_cast<float4*>(a.mb_scalars + (int64_t)r * 8)[c - OP] = __ldg(reinterpret_cast<const float4*>(a.scalars + src * 8) + (c - OP));
+      reinterpret_cast<float4*>(a.mb_scalars + (int64_t)r * 8)[c - OP] =
+          real ? __ldg(reinterpret_cast<const float4*>(a.scalars + src * 8) + (c - OP)) : make_float4(0.f, 0.f, 0.f, 0.f);
     } else {
-      a.mb_not_done[r] = __ldg(a.not_done + src);
+      a.mb_not_done[r] = real ? __ldg(a.not_done + src) : 0.f;
     }
   }
   // initial state: thread -> one 16-byte chunk (8 hidden units) of one sequence
-  const int64_t nchunks = S * (HID / 8);
+  const int64_t nchunks = R * (HID / 8);
   if (i < nchunks) {
     const int64_t sq = i / (HID / 8);
-    const int ug = (int)(i % (HID / 8)), unit0 = 8 * ug;
-    const int ck = (int)(sq / a.env_count), el = (int)(sq % a.env_count), e = a.env_begin + el;
-    const float m = a.not_done[((int64_t)ck * a.seq_len) * a.num_envs + e];
-    // cell state rows
-    const float4* cs = reinterpret_cast<const float4*>(a.c_saved + ((int64_t)ck * a.num_envs + e) * HID + unit0);
+    const int ug = (int)(i % (HID / 8)), unit0 = 8 * ug, half = unit0 / UK;
     float4* cd = reinterpret_cast<float4*>(a.c0 + sq * HID + unit0);
-    cd[0] = cs[0], cd[1] = cs[1];
-    // hidden state: saved tiles [chunk][N/128][2] -> masked tiles [S/128][2]
-    const int64_t st = (int64_t)ck * (a.num_envs / TILE) + e / TILE, dt = sq / TILE;
-    const int half = unit0 / UK, off_s = tile_offset(e % TILE, unit0 % UK, UK), off_d = tile_offset((int)(sq % TILE), unit0 % UK, UK);
-    const uint4 v = *reinterpret_cast<const uint4*>(reinterpret_cast<const uint8_t*>(a.hh_saved) + (st * 2 + half) * TILE_BYTES + off_s);
-    const uint32_t w[4] = {v.x, v.y, v.z, v.w};
-    uint32_t o[4];
+    uint4* hd = reinterpret_cast<uint4*>(reinterpret_cast<uint8_t*>(a.hm0) + ((sq / TILE) * 2 + half) * TILE_BYTES +
+                                         tile_offset((int)(sq % TILE), unit0 % UK, UK));
+    if (sq >= S) {   // padded sequence
+      cd[0] = cd[1] = make_float4(0.f, 0.f, 0.f, 0.f);
+      *hd = make_uint4(0u, 0u, 0u, 0u);
+    } else {
+      const int ck = (int)(sq / a.env_count), el = (int)(sq % a.env_count), e = a.env_begin + el;
+      const float m = a.not_done[((int64_t)ck * a.seq_len) * a.num_envs + e];
+      // cell state rows
+      const float4* cs = reinterpret_cast<const float4*>(a.c_saved + ((int64_t)ck * a.num_envs + e) * HID + unit0);
+      cd[0] = cs[0], cd[1] = cs[1];
+      // hidden state: saved tiles [chunk][ceil(N/128)][2] -> masked tiles [ceil(R/128)][2]
+      const int64_t st = (int64_t)ck * ((a.num_envs + TILE - 1) / TILE) + e / TILE;
+      const uint4 v = *reinterpret_cast<const uint4*>(reinterpret_cast<const uint8_t*>(a.hh_saved) + (st * 2 + half) * TILE_BYTES +
+                                                      tile_offset(e % TILE, unit0 % UK, UK));
+      const uint32_t w[4] = {v.x, v.y, v.z, v.w};
+      uint32_t o[4];
 #pragma unroll
-    for (int k = 0; k < 4; ++k) {
-      const float2 f = unpack_bf16(w[k]);
-      o[k] = pack_bf16(f.x * m, f.y * m);
+      for (int k = 0; k < 4; ++k) {
+        const float2 f = unpack_bf16(w[k]);
+        o[k] = pack_bf16(f.x * m, f.y * m);
+      }
+      *hd = make_uint4(o[0], o[1], o[2], o[3]);
     }
-    *reinterpret_cast<uint4*>(reinterpret_cast<uint8_t*>(a.hm0) + (dt * 2 + half) * TILE_BYTES + off_d) = make_uint4(o[0], o[1], o[2], o[3]);
   }
 }
 
@@ -1059,6 +1096,7 @@ int vine_lstm_pack(const float* w_ih, const float* w_hh, const float* b_ih, cons
 
 int vine_lstm_step(const VineLstmStep* a, void* stream) {
   if (!a || !a->params || !a->u || !a->hm || !a->c_prev || !a->c || !a->hh || a->n <= 0) return VINE_ERR_INVALID_ARG;
+  if (a->hm_next_rows != 0 && (a->hm_next_rows < a->n || a->hm_next_rows > (a->n + TILE - 1) / TILE * TILE)) return VINE_ERR_INVALID_ARG;
   if ((((uintptr_t)a->params) | ((uintptr_t)a->u) | ((uintptr_t)a->hm) | ((uintptr_t)a->hh) | ((uintptr_t)a->c_prev) |
        ((uintptr_t)a->c)) & 15u)
     return VINE_ERR_INVALID_ARG;
@@ -1092,6 +1130,7 @@ int vine_lstm_cell_bwd_tiles(const VineLstmCellBwd* a, void* stream) {
 
 int vine_lstm_bwd_gemm(const VineLstmBwdGemm* a, void* stream) {
   if (!a || !a->params || !a->dg || !a->dh3 || a->n <= 0) return VINE_ERR_INVALID_ARG;
+  if (a->dh3_rows != 0 && (a->dh3_rows < a->n || a->dh3_rows > (a->n + TILE - 1) / TILE * TILE)) return VINE_ERR_INVALID_ARG;
   static int configured = -1;
   int dev = 0;
   if (cudaGetDevice(&dev) != cudaSuccess) return VINE_ERR_CUDA;
@@ -1124,13 +1163,14 @@ int vine_abi_struct_size(int which) {
 int vine_lstm_gather(const VineLstmGather* a, void* stream) {
   if (!a || !a->obs || !a->scalars || !a->not_done || !a->c_saved || !a->hh_saved || !a->mb_obs || !a->mb_scalars || !a->mb_not_done ||
       !a->c0 || !a->hm0 || a->seq_len < 1 || a->chunks < 1 || a->env_count < 1 || a->env_begin < 0 ||
-      a->env_begin + a->env_count > a->num_envs || a->num_envs % TILE || a->env_count % TILE || a->env_begin % TILE || a->num_obs < 1)
+      a->env_begin + a->env_count > a->num_envs || a->num_obs < 1)
     return VINE_ERR_INVALID_ARG;
-  const int64_t S = (int64_t)a->chunks * a->env_count, rows = (int64_t)a->seq_len * S;
+  const int64_t S = (int64_t)a->chunks * a->env_count, R = a->step_rows ? a->step_rows : S, rows = (int64_t)a->seq_len * R;
+  if (a->step_rows < 0 || R < S) return VINE_ERR_INVALID_ARG;
   const int64_t pieces = ((a->num_obs & 1) ? a->num_obs : a->num_obs / 2) + 3;
   if (rows * pieces >= (int64_t)1 << 31) return VINE_ERR_INVALID_ARG;
   int64_t work = rows * pieces;
-  if (S * (HID / 8) > work) work = S * (HID / 8);
+  if (R * (HID / 8) > work) work = R * (HID / 8);
   vine_launch::launch(vine_lstm_gather_kernel, (unsigned)((work + 255) / 256), 256, 0, (cudaStream_t)stream, *a);
   return cudaGetLastError() == cudaSuccess ? VINE_OK : VINE_ERR_CUDA;
 }
@@ -1186,9 +1226,14 @@ int vine_lstm_adam(const float* flat, float grad_scale, float* params, float* ex
 int vine_lstm_head_train(const VineLstmHeadTrain* a, void* stream) {
   if (!a || !a->params || !a->hh || !a->scalars || !a->logstd || !a->logstd_old || !a->dh || !a->grads || a->n <= 0)
     return VINE_ERR_INVALID_ARG;
+  if (a->step_rows != 0 && (a->step_rows < 0 || a->step_seqs < 1 || a->step_seqs > a->step_rows || a->n % a->step_rows ||
+                            a->n >= ((int64_t)1 << 31)))
+    return VINE_ERR_INVALID_ARG;
+  if (a->step_rows != 0 && a->mu_writeback && a->wb_chunks * a->wb_env_count != a->step_seqs) return VINE_ERR_INVALID_ARG;
   int64_t blocks = (a->n + 7) / 8;
   if (blocks > 296) blocks = 296;   // 2 resident blocks per SM (128 registers per thread), one wave; <= VINE_LSTM_HEAD_GRAD_PARTS
-  vine_launch::launch(vine_lstm_head_train_kernel, (unsigned)blocks, 256, 0, (cudaStream_t)stream, *a);
+  if (a->step_rows) vine_launch::launch(vine_lstm_head_train_kernel<true>, (unsigned)blocks, 256, 0, (cudaStream_t)stream, *a);
+  else vine_launch::launch(vine_lstm_head_train_kernel<false>, (unsigned)blocks, 256, 0, (cudaStream_t)stream, *a);
   return cudaGetLastError() == cudaSuccess ? (int)blocks : VINE_ERR_CUDA;   // number of gradient partials written
 }
 

@@ -295,11 +295,11 @@ __global__ void __launch_bounds__(128 * Q, 1) vine_ppo_minibatch_kernel(const Mb
              });
     bwd_epilogue<H3>(lane_base + TM_DATA + part * C64, C64, part * C64, a3_t, row);   // dz3 over h3
     } else {
-      // dz3 = dh3 (from the LSTM backward, f32 [B, 64]) * ELU'(h3), written over h3 in place
+      // dz3 = dh3 (from the LSTM backward, f32 [T, N, 64], rows like obs) * ELU'(h3), written over h3 in place
       __syncthreads();   // every thread is past its h3 stores / the layer-3 accumulator reads
       uint32_t r[C64];
       if (valid) {
-        const float4* src = reinterpret_cast<const float4*>(a.dh3_ext + s * H3 + part * C64);
+        const float4* src = reinterpret_cast<const float4*>(a.dh3_ext + grow * H3 + part * C64);
 #pragma unroll
         for (int i = 0; i < C64 / 4; ++i) {
           const float4 v = src[i];

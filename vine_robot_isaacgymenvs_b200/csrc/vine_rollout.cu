@@ -78,7 +78,8 @@ __global__ void __launch_bounds__(THREADS, 1) vine_policy_act_kernel(const VineP
 
   for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
     const int64_t e = tile * TILE + row;
-    const bool valid = e < a.n;
+    // a padded row of a recurrent minibatch (u_step_*) reads no observation: its U row is that of a zero input, finite
+    const bool valid = e < a.n && (a.u_step_rows == 0 || e % a.u_step_rows < a.u_step_seqs);
     build_x_tile(x_t, row, half, valid, a.obs + e * O, a.obs_mean, a.obs_inv_std, O, a.u_out != nullptr,
                  (valid && a.obs_copy) ? a.obs_copy + e * O : nullptr);
 #pragma unroll 1
@@ -275,6 +276,8 @@ int vine_policy_act(const VinePolicyAct* a, void* stream) {
   if (a->actions && !a->logstd) return VINE_ERR_INVALID_ARG;
   if (!a->actions && !a->mu && !a->value && !a->u_out) return VINE_ERR_INVALID_ARG;
   if (a->u_out && (a->num_obs >= K1 || (((uintptr_t)a->u_out) & 15u))) return VINE_ERR_INVALID_ARG;
+  if (a->u_step_rows != 0 && (!a->u_out || a->u_step_rows < 0 || a->u_step_seqs < 1 || a->u_step_seqs > a->u_step_rows))
+    return VINE_ERR_INVALID_ARG;
   static int configured = -1;
   int dev = 0, sms = 0;
   if (cudaGetDevice(&dev) != cudaSuccess) return VINE_ERR_CUDA;

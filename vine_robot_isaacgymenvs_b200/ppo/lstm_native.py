@@ -2,7 +2,8 @@
 which kernel runs when, on which buffers.  All arithmetic is in csrc/ (vine_rollout.cu, vine_lstm_net.cu, vine_ppo.cu);
 this module only owns the HBM buffers (activation tiles, cell states, gradient workspaces) and issues the launches.
 
-One minibatch (S sequences x L steps, rows ordered [step][sequence]) = 1 MLP forward launch (U tiles), L LSTM steps,
+One minibatch (S sequences x L steps, rows ordered [step][sequence]; every step padded to R = round_up(S, 128) rows, see
+NativeLstmPath.step_rows) = 1 MLP forward launch (U tiles), L LSTM steps,
 1 head forward/loss/backward, L x (cell backward + backward-data GEMM), 1 MLP backward launch (recompute + weight
 gradients), 1 LSTM weight-gradient GEMM, 2 reductions, [all-reduce], [gradient-norm clip over both vectors, with
 truncate_grads], 2 Adam launches.
@@ -24,12 +25,21 @@ def _ptr(t, off_elems=0):
 class NativeLstmPath:
     ARENA = True
 
+    @staticmethod
+    def step_rows(num_seqs):
+        """Rows per time step of a minibatch of ``num_seqs`` sequences: rounded up to whole 128-row tiles, so that every step
+        starts on a tile and the per-step kernels see a ragged last tile at most.  Rows [num_seqs, step_rows) of each step are
+        padded sequences: the gather gives them zero inputs and state, and the kernels keep them out of every loss term and
+        gradient."""
+        return -(-num_seqs // 128) * 128
+
     def __init__(self, num_obs, seq_len, num_seqs, device, hyper, wgrad_splits=12):
-        assert num_seqs % 128 == 0, "sequences per minibatch must be a multiple of the 128-row tile"
+        assert num_seqs >= 1
         self.lib = abi.load_library()
         self.O, self.L, self.S, self.dev = num_obs, seq_len, num_seqs, device
-        self.tiles = num_seqs // 128
-        L, S, tl = seq_len, num_seqs, self.tiles
+        self.R = self.step_rows(num_seqs)
+        self.tiles = self.R // 128
+        L, S, tl = seq_len, self.R, self.tiles      # every per-step buffer holds R rows
         # every activation / scratch buffer of the path is a view into ONE allocation (ARENA): their relative placement then
         # does not depend on what the caching allocator freed before the agent was built
         elems = lambda s: int(torch.Size(s).numel())  # noqa: E731
@@ -69,30 +79,32 @@ class NativeLstmPath:
     # ------------------------------------------------------------------ forward + backward of one minibatch
     def gradients(self, packed_mlp, packed_lstm, obs, scalars, not_done, obs_mean, obs_inv_std, value_stats, logstd, logstd_old,
                   state, debug_out=None, writeback=None, p2p=(None, None), position=(0, 0)):
-        """obs f32 [L, S, O], scalars f32 [L, S, 8], not_done f32 [L, S]; self.HM[0] (masked initial hidden state tiles) and
-        self.C0 must already hold the initial LSTM state.  Leaves the gradients in flat_g_mlp / flat_g_lstm.
+        """obs f32 [L, R, O], scalars f32 [L, R, 8], not_done f32 [L, R] (R = self.R; rows [S, R) of each step are padding
+        and never read); self.HM[0] (masked initial hidden state tiles) and self.C0 must already hold the initial LSTM state.  Leaves the gradients in flat_g_mlp / flat_g_lstm.
         ``writeback`` = (scalars_src [T, N, 8], seq_len, chunks, num_envs, env_begin, env_count): rl_games'
         dataset.update_mu_sigma -- this pass's mu goes back into the source rows and ``logstd_old`` receives ``logstd``.
         ``p2p`` = (MLP channel, LSTM channel) device pointers: multi-GPU, the two gradient sums go into this rank's peer-visible
         buffers instead of flat_g_* (distributed.P2PChannel).  ``position`` = (mini-epoch, minibatch slot) of this minibatch
         in the iteration: what the learning-rate schedule of vine_ppo_minibatch needs to know, passed to hyper["schedule"]
         (PPOAgent._schedule_fields); without that entry the launch runs the adaptive legacy schedule."""
-        lib, L, S, tl, st = self.lib, self.L, self.S, self.tiles, self._stream()
-        n = L * S
+        lib, L, S, R, tl, st = self.lib, self.L, self.S, self.R, self.tiles, self._stream()
+        n = L * R
         act = abi.VinePolicyAct(packed=_ptr(packed_mlp), obs=_ptr(obs), obs_mean=_ptr(obs_mean), obs_inv_std=_ptr(obs_inv_std),
-                                value_stats=_ptr(value_stats), n=n, num_obs=self.O, u_out=_ptr(self.U))
+                                value_stats=_ptr(value_stats), n=n, num_obs=self.O, u_out=_ptr(self.U), u_step_rows=R,
+                                u_step_seqs=S)
         assert lib.vine_policy_act(C.byref(act), st) == 0
         for t in range(L):
             last = t == L - 1
             a = abi.VineLstmStep(params=_ptr(packed_lstm), u=_ptr(self.U[t]), hm=_ptr(self.HM[t]),
                                  c_prev=_ptr(self.Cs[t - 1] if t else self.C0), not_done=_ptr(not_done[t]),
                                  not_done_next=None if last else _ptr(not_done[t + 1]), c=_ptr(self.Cs[t]), hh=_ptr(self.HH[t]),
-                                 hm_next=None if last else _ptr(self.HM[t + 1]), act=_ptr(self.ACT[t]), n=S)
+                                 hm_next=None if last else _ptr(self.HM[t + 1]), act=_ptr(self.ACT[t]), n=S, hm_next_rows=R)
             assert lib.vine_lstm_step(C.byref(a), st) == 0
         h = self.hyper
         ht = abi.VineLstmHeadTrain(params=_ptr(packed_lstm), hh=_ptr(self.HH), scalars=_ptr(scalars), logstd=_ptr(logstd),
                                    logstd_old=_ptr(logstd_old), dh=_ptr(self.DH), grads=_ptr(self.head_grads),
-                                   debug_out=_ptr(debug_out) if debug_out is not None else None, n=n, inv_B=1.0 / n,
+                                   debug_out=_ptr(debug_out) if debug_out is not None else None, n=n, inv_B=1.0 / (L * S),
+                                   step_rows=R if R != S else 0, step_seqs=S,   # 0: no padded rows (the dense kernel)
                                    e_clip=h["e_clip"], critic_coef=h["critic_coef"], entropy_coef=h["entropy_coef"],
                                    bounds_loss_coef=h["bounds_loss_coef"], value_loss_unclipped=int(not h.get("clip_value", True)))
         if writeback is not None:
@@ -108,13 +120,13 @@ class NativeLstmPath:
                                      dc_prev=_ptr(self.DC[t & 1]), n=S)
             assert lib.vine_lstm_cell_bwd_tiles(C.byref(cb), st) == 0
             bg = abi.VineLstmBwdGemm(params=_ptr(packed_lstm), dg=_ptr(self.DG[t]), not_done=_ptr(not_done[t]), dh3=_ptr(self.DH3[t]),
-                                     dh_rec=_ptr(self.DHREC[t - 1]) if t else None, n=S)
+                                     dh_rec=_ptr(self.DHREC[t - 1]) if t else None, n=S, dh3_rows=R)
             assert lib.vine_lstm_bwd_gemm(C.byref(bg), st) == 0
         sched = h["schedule"](*position) if "schedule" in h else dict(
             adaptive_lr=int(h.get("adaptive_lr", 1)), kl_threshold=h.get("kl_threshold", 0.008), lr_min=1e-6, lr_max=1e-2)
         mb = abi.VinePpoMinibatch(packed=_ptr(packed_mlp), obs=_ptr(obs), obs_mean=_ptr(obs_mean), obs_inv_std=_ptr(obs_inv_std),
                                   logstd=_ptr(logstd), logstd_old=_ptr(logstd_old), workspace=_ptr(self.mlp_ws), state=_ptr(state),
-                                  horizon=1, num_envs=n, env_begin=0, env_count=n, num_obs=self.O, workspace_ctas=self.mlp_ctas,
+                                  horizon=L, num_envs=R, env_begin=0, env_count=S, num_obs=self.O, workspace_ctas=self.mlp_ctas,
                                   e_clip=h["e_clip"], critic_coef=h["critic_coef"], entropy_coef=h["entropy_coef"],
                                   bounds_loss_coef=h["bounds_loss_coef"], dh3_ext=_ptr(self.DH3), **sched)
         n_part = lib.vine_ppo_minibatch(C.byref(mb), st)

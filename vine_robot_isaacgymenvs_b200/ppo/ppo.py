@@ -346,9 +346,6 @@ class PPOAgent:
         if self.has_rnn:
             if int(rnn_cfg.get("units", 0)) != 256 or not rnn_cfg.get("concat_input") or not rnn_cfg.get("layer_norm"):
                 why.append("network.rnn must be the reference's block: units 256, concat_input True, layer_norm True")
-            if self.n % 128 or self.mb_envs % 128:
-                why.append(f"num_envs ({self.n}) and minibatch_size / horizon_length ({self.mb_envs}) must be multiples of 128 "
-                           "for the recurrent kernels (128-row tensor-core tiles)")
         return why
 
     def _param_order(self):
@@ -426,7 +423,7 @@ class PPOAgent:
         self._moments = torch.zeros(2 * self.O + 4, dtype=torch.float64, device=dev)
         self._adv_stats = z(2)
         self._clip_ws = z(abi.GRAD_CLIP_WS_FLOATS) if self.truncate_grads else None
-        L, chunks, tiles_n = self.seq_len, self.T // self.seq_len, self.n // 128
+        L, chunks, tiles_n = self.seq_len, self.T // self.seq_len, -(-self.n // 128)
         hyper = dict(e_clip=self.e_clip, critic_coef=self.critic_coef, entropy_coef=self.entropy_coef,
                      bounds_loss_coef=self.bounds_coef, clip_value=self.clip_value, schedule=self._schedule_fields)
         self._path = NativeLstmPath(self.O, L, chunks * self.mb_envs, dev, hyper)
@@ -440,8 +437,8 @@ class PPOAgent:
         self._nd_ext = torch.zeros(self.T + 1, self.n, device=dev)       # 1 - dones before step t
         self._ones_n = torch.ones(self.n, device=dev)
         self._scal = z(self.T, self.n, 8)
-        self._mb_obs, self._mb_scal = z(L, chunks * self.mb_envs, self.O), z(L, chunks * self.mb_envs, 8)
-        self._mb_nd = z(L, chunks * self.mb_envs)
+        R = self._path.R                                                 # minibatch rows per step (padded to whole tiles)
+        self._mb_obs, self._mb_scal, self._mb_nd = z(L, R, self.O), z(L, R, 8), z(L, R)
 
     @torch.no_grad()
     def _rollout_native_lstm(self):
@@ -532,7 +529,7 @@ class PPOAgent:
                                         c_saved=ptr(self._C_saved), hh_saved=ptr(self._HH_saved), mb_obs=ptr(self._mb_obs),
                                         mb_scalars=ptr(self._mb_scal), mb_not_done=ptr(self._mb_nd), c0=ptr(path.C0),
                                         hm0=ptr(path.HM[0]), seq_len=L, chunks=chunks, num_envs=n, env_begin=e0, env_count=E,
-                                        num_obs=self.O)
+                                        num_obs=self.O, step_rows=path.R)
                 assert lib.vine_lstm_gather(C.byref(ga), stream) == 0
                 path.gradients(self._packed, self._lpacked, self._mb_obs, self._mb_scal, self._mb_nd, self._obs_mean_f,
                                self._obs_inv_std_f, self._val_stats, self.model.sigma, self._logstd_old[e0 // E], self.ppo_state,
