@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define VINE_ABI_VERSION 6
+#define VINE_ABI_VERSION 7
 
 #define VINE_NUM_DOFS 6          /* 1 prismatic rail cart + 5 revolute links (V5:54,83) */
 #define VINE_NUM_ACTIONS 2       /* u_rail_velocity, u_fpam (V5:171) */
@@ -395,6 +395,8 @@ int vine_gae(const float* rewards, const float* values, const float* dones,
  *   x = clamp((obs - obs_mean) * obs_inv_std, +-5);  mu f32[N,2];  value f32[N] de-normalised as
  *   clamp(v, +-5) * value_stats[1] + value_stats[0]  (rl_games RunningMeanStd, normalize_input /
  *   normalize_value; value_stats = device pointer to {mean, std} so a captured CUDA graph sees updates).
+ * vine_mlp_forward expresses a normaliser that is off (normalize_input / normalize_value False) by NULL statistics:
+ * obs_mean == obs_inv_std == NULL gives x = obs (no clamp), value_stats == NULL gives value = v (no clamp).
  */
 #define VINE_MLP_PACKED_BYTES 102208
 int vine_mlp_pack(const float* w1, const float* b1, const float* w2, const float* b2, const float* w3,
@@ -416,11 +418,11 @@ int vine_mlp_forward(const void* packed, const float* obs, const float* obs_mean
 typedef struct VinePolicyAct {
   const void* packed;            /* VINE_MLP_PACKED_BYTES */
   const float* obs;              /* [n, O] */
-  const float* obs_mean;         /* [O] */
-  const float* obs_inv_std;      /* [O] */
-  const float* value_stats;      /* {mean, std} */
+  const float* obs_mean;         /* [O]; not read (may be NULL) with raw_obs */
+  const float* obs_inv_std;      /* [O]; not read (may be NULL) with raw_obs */
+  const float* value_stats;      /* {mean, std}; not read (may be NULL) with raw_value */
   float* mu;                     /* [n, 2] */
-  float* value;                  /* [n] de-normalised */
+  float* value;                  /* [n] de-normalised (raw_value: the value head's output) */
   const float* logstd;           /* [2]; required when sampling */
   const uint32_t* rng_counter;   /* device word, advanced by vine_rollout_post */
   float* actions;                /* [n, 2] raw sampled actions; NULL = no sampling */
@@ -428,15 +430,18 @@ typedef struct VinePolicyAct {
   float* obs_copy;               /* [n, O] */
   float* env_actions;            /* [n, 2] clamped to [-1, 1] */
   int64_t n;
-  int32_t num_obs, reserved;
+  int32_t num_obs;
+  int32_t raw_obs;               /* 1: normalize_input off: x = bf16(obs), no mean / std and no +-5 clamp */
   uint64_t seed;
   int64_t global_env_offset;
   void* u_out;                   /* NULL, or [ceil(n/128)] tiles [128 x 128] bf16 (UMMA row-blocked): the LSTM input
-                                    [MLP output (64) | normalised obs (32, col 31 == 1) | 0]; heads and sampling are
+                                    [MLP output (64) | x (32, col 31 == 1) | 0]; heads and sampling are
                                     skipped (they follow the LSTM: vine_lstm_step / vine_lstm_head) */
   int32_t u_step_rows, u_step_seqs;   /* with u_out: rows come in groups of u_step_rows (one time step of a minibatch padded to
                                     whole tiles), of which the first u_step_seqs are real; the rest read no observation and
                                     get the U row of a zero input.  0, 0: every row is real */
+  int32_t raw_value;             /* 1: normalize_value off: value = the value head's output (no clamp, no de-normalisation) */
+  int32_t reserved;              /* 0 */
 } VinePolicyAct;
 int vine_policy_act(const VinePolicyAct* args, void* stream);
 
@@ -477,6 +482,9 @@ int vine_rollout_post(const VineRolloutPost* args, void* stream);
  * statistics into `moments` (2*O + 4 doubles, zero on first use; all-reduce it across ranks and set `world`),
  * vine_ppo_finalize merges them into the running statistics (f64, in place), writes the f32 copies the
  * kernels read, normalises, and clears `moments`.
+ * raw_obs (normalize_input off): the observation moments stay zero and obs, obs_mean/var/count and their f32 copies are not
+ * read or written (may be NULL).  raw_value (normalize_value off): val_mean/var/count and value_stats are not read or
+ * written (may be NULL) and values_n / returns_n are exact copies of values / returns.  Advantages are unaffected.
  */
 typedef struct VinePpoPrologue {
   const float* obs;              /* [count, O] */
@@ -489,7 +497,10 @@ typedef struct VinePpoPrologue {
   float *value_stats, *adv_stats;             /* {mean, std}, {mean, 1/(std+1e-8)} out */
   float *values_n, *returns_n, *advantages_n; /* [count] out */
   int64_t count;
-  int32_t num_obs, world, normalize_advantage, reserved;
+  int32_t num_obs, world, normalize_advantage;
+  int32_t raw_obs;               /* 1: normalize_input off */
+  int32_t raw_value;             /* 1: normalize_value off */
+  int32_t reserved;              /* 0 */
 } VinePpoPrologue;
 int vine_ppo_moments(const VinePpoPrologue* args, void* stream);
 int vine_ppo_finalize(const VinePpoPrologue* args, void* stream);
@@ -527,9 +538,9 @@ typedef struct VineLstmStep {
 typedef struct VineLstmHead {
   const void* params;
   const void* hh;
-  const float* value_stats;      /* {mean, std} */
+  const float* value_stats;      /* {mean, std}; not read (may be NULL) with raw_value */
   float* mu;                     /* [n, 2] or NULL */
-  float* value;                  /* [n] de-normalised, or NULL */
+  float* value;                  /* [n] de-normalised (raw_value: the value head's output), or NULL */
   const float* logstd;           /* [2]; required when sampling */
   const uint32_t* rng_counter;
   float* actions;                /* [n, 2] or NULL (no sampling) */
@@ -538,6 +549,8 @@ typedef struct VineLstmHead {
   int64_t n;
   uint64_t seed;
   int64_t global_env_offset;
+  int32_t raw_value;             /* 1: normalize_value off: value = the value head's output (no clamp, no de-normalisation) */
+  int32_t reserved;              /* 0 */
 } VineLstmHead;
 int vine_lstm_pack(const float* w_ih, const float* w_hh, const float* b_ih, const float* b_hh, const float* ln_gamma,
                    const float* ln_beta, const float* w_mu, const float* b_mu, const float* w_v, const float* b_v,
@@ -549,8 +562,8 @@ int vine_lstm_head(const VineLstmHead* args, void* stream);
 /*
  * Training counterpart of vine_lstm_head over all rows of a minibatch (rows = [step][sequence]): LayerNorm + heads,
  * the PPO losses of vine_ppo_minibatch (same formulas), and the backward down to dh (bf16 tiles like hh).
- * scalars f32 [n, 8] per row: action0, action1, mu_old0, mu_old1, neglogp_old, value_old (normalised), return
- * (normalised), advantage (normalised).  grads f32 [VINE_LSTM_HEAD_GRAD_PARTS + 1][VINE_LSTM_HEAD_GRAD_FLOATS] receives one
+ * scalars f32 [n, 8] per row: action0, action1, mu_old0, mu_old1, neglogp_old, value_old (normalised; raw with
+ * normalize_value off), return (likewise), advantage (normalised).  grads f32 [VINE_LSTM_HEAD_GRAD_PARTS + 1][VINE_LSTM_HEAD_GRAD_FLOATS] receives one
  * partial per thread block (the call returns how many; vine_lstm_reduce sums them): d(LayerNorm gamma)[256],
  * d(beta)[256], d(W_mu0, W_mu1, W_v)[3][256], d(b)[3] (+1 pad), d(logstd)[2], loss statistics a_loss, c_loss, kl,
  * b_loss (means), padding.
@@ -698,8 +711,9 @@ int vine_lstm_cell_bwd(const void* acts_bf16, const float* c_prev, const float* 
  * vine_ppo_adam rewrites in place, so vine_mlp_forward always sees the current policy.
  *
  * A minibatch is rl_games' env-major slice: envs [env_begin, env_begin+env_count) x all `horizon` steps of the
- * [T, N] rollout buffers.  values_old / returns are value-normalised, advantages are batch-normalised (both
- * done by the caller once per iteration), obs is raw and normalised inside like vine_mlp_forward.
+ * [T, N] rollout buffers.  values_old / returns are value-normalised (raw with normalize_value off), advantages are
+ * batch-normalised (both done by the caller once per iteration), obs is raw and normalised inside like vine_mlp_forward
+ * (with raw_obs: used as it is).
  *
  * state (device, >= 16 floats): [0] learning rate, [1] Adam step count, [2] KL of the last minibatch,
  * [3] "KL pending" flag, [4..7] running sums of a_loss, c_loss, kl, b_loss, [8] minibatches summed,
@@ -723,11 +737,11 @@ typedef struct VinePpoMinibatch {
   float* mu_old;                 /* [T, N, 2] in: mean of the policy the row was last evaluated with (rollout, or the previous
                                     mini-epoch); out: this pass's mean (rl_games dataset.update_mu_sigma) */
   const float* neglogp_old;      /* [T, N] */
-  const float* values_old;       /* [T, N] normalised */
-  const float* returns;          /* [T, N] normalised */
+  const float* values_old;       /* [T, N] normalised (or raw, see above) */
+  const float* returns;          /* [T, N] normalised (or raw, see above) */
   const float* advantages;       /* [T, N] normalised */
-  const float* obs_mean;         /* [O] */
-  const float* obs_inv_std;      /* [O] */
+  const float* obs_mean;         /* [O]; not read (may be NULL) with raw_obs */
+  const float* obs_inv_std;      /* [O]; not read (may be NULL) with raw_obs */
   const float* logstd;           /* [2] current (points into the flat parameter vector) */
   const float* logstd_old;       /* [2] log-std these rows were last evaluated with (see vine_ppo_reduce) */
   float* workspace;              /* [workspace_ctas][VINE_PPO_WS_FLOATS] gradient partials, 16-B aligned */
@@ -747,7 +761,7 @@ typedef struct VinePpoMinibatch {
   int32_t max_epochs;            /* lr_linear: the schedule's length in iterations */
   int32_t value_loss_unclipped;  /* 0: clipped value loss (rl_games clip_value True); 1: c_loss = (return - v)^2 */
   float lr0;                     /* lr_linear: the initial learning rate */
-  float reserved_f2;             /* 0 */
+  int32_t raw_obs;               /* 1: normalize_input off: x = bf16(obs), no mean / std and no +-5 clamp */
 } VinePpoMinibatch;
 
 int vine_ppo_num_params(int num_obs);

@@ -1,6 +1,7 @@
 """Time one PPO iteration of the reference network (MLP -> LSTM 256 -> LayerNorm) at FSTR, N envs, CUDA-graph replay:
-python tools/ppo_time.py [N] [--minibatch M] [--mlp] [--no-pdl] [--no-arena] [--pad K] [--truncate-grads [--grad-norm X]]
-Prints ms per iteration / rollout / update (CUDA events, best of 3 x 20) and the card with its power limit.  --minibatch sets
+python tools/ppo_time.py [N] [--minibatch M] [--mlp] [--raw-obs] [--raw-value] [--no-pdl] [--no-arena] [--pad K]
+                         [--truncate-grads [--grad-norm X]]
+--raw-obs / --raw-value switch the input / value normaliser off (normalize_input / normalize_value False).  Prints ms per iteration / rollout / update (CUDA events, best of 3 x 20) and the card with its power limit.  --minibatch sets
 minibatch_size (default: the config's 32768, which needs N * horizon to be a multiple of it; e.g. N = 4000 wants 32000).
 --truncate-grads also builds a second agent with gradient-norm clipping (truncate_grads=True, grad_norm X, default 1.0) and
 times the two update graphs alternately."""
@@ -19,6 +20,10 @@ n = int(args[0]) if args and args[0].isdigit() else 4096
 extra = ["train.params.network.rnn=null"] if "--mlp" in args else []
 if "--minibatch" in args:
     extra.append(f"train.params.config.minibatch_size={int(args[args.index('--minibatch') + 1])}")
+if "--raw-obs" in args:
+    extra.append("train.params.config.normalize_input=False")
+if "--raw-value" in args:
+    extra.append("train.params.config.normalize_value=False")
 if "--no-pdl" in args:
     PPOAgent.PDL_MAX_ENVS = 0
 if "--no-arena" in args:
@@ -74,7 +79,7 @@ if clip_agent is not None:   # update graph without / with clipping, alternating
         on.append(best(clip_agent._g_update.replay))
     q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader", "-i", "0"], capture_output=True, text=True)
     coef = float(clip_agent.ppo_state[9])
-    print(f"n={n} {'mlp' if extra else 'reference network'}: update {min(off):.3f} ms without clipping, {min(on):.3f} ms with "
+    print(f"n={n} {'mlp' if '--mlp' in args else 'reference network'}: update {min(off):.3f} ms without clipping, {min(on):.3f} ms with "
           f"(+{(min(on) - min(off)) * 1e3:.1f} us per update, {(min(on) - min(off)) * 1e3 / (agent.mini_epochs * (agent.n // agent.mb_envs)):.2f} "
           f"us per minibatch; spread off {min(off):.3f}-{max(off):.3f}, on {min(on):.3f}-{max(on):.3f}); last coefficient {coef:.4g}; "
           f"{q.stdout.strip() or torch.cuda.get_device_name(0)}", flush=True)

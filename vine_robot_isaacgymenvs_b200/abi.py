@@ -12,7 +12,7 @@ NUM_ACTIONS = 2
 NUM_REWARDS = 13
 NUM_OBJECT_INFO = 2
 MAX_ACTION_DELAY = 8
-ABI_VERSION = 6
+ABI_VERSION = 7
 
 OK = 0
 ERR_INVALID_ARG = -1
@@ -165,8 +165,9 @@ class VinePolicyAct(C.Structure):
     _fields_ = ([(n, C.c_void_p) for n in (
         "packed", "obs", "obs_mean", "obs_inv_std", "value_stats", "mu", "value", "logstd", "rng_counter", "actions",
         "neglogp", "obs_copy", "env_actions")]
-        + [("n", C.c_int64), ("num_obs", C.c_int32), ("reserved", C.c_int32), ("seed", C.c_uint64),
-           ("global_env_offset", C.c_int64), ("u_out", C.c_void_p), ("u_step_rows", C.c_int32), ("u_step_seqs", C.c_int32)])
+        + [("n", C.c_int64), ("num_obs", C.c_int32), ("raw_obs", C.c_int32), ("seed", C.c_uint64),
+           ("global_env_offset", C.c_int64), ("u_out", C.c_void_p), ("u_step_rows", C.c_int32), ("u_step_seqs", C.c_int32),
+           ("raw_value", C.c_int32), ("reserved", C.c_int32)])
 
 
 class VineLstmStep(C.Structure):
@@ -177,7 +178,8 @@ class VineLstmStep(C.Structure):
 class VineLstmHead(C.Structure):
     _fields_ = ([(n, C.c_void_p) for n in ("params", "hh", "value_stats", "mu", "value", "logstd", "rng_counter", "actions",
                                            "neglogp", "env_actions")]
-                + [("n", C.c_int64), ("seed", C.c_uint64), ("global_env_offset", C.c_int64)])
+                + [("n", C.c_int64), ("seed", C.c_uint64), ("global_env_offset", C.c_int64), ("raw_value", C.c_int32),
+                   ("reserved", C.c_int32)])
 
 
 class VineLstmHeadTrain(C.Structure):
@@ -222,7 +224,7 @@ class VinePpoPrologue(C.Structure):
         "obs", "values", "returns", "moments", "obs_mean", "obs_var", "obs_count", "val_mean", "val_var", "val_count",
         "obs_mean_f", "obs_inv_std_f", "value_stats", "adv_stats", "values_n", "returns_n", "advantages_n")]
         + [("count", C.c_int64), ("num_obs", C.c_int32), ("world", C.c_int32), ("normalize_advantage", C.c_int32),
-           ("reserved", C.c_int32)])
+           ("raw_obs", C.c_int32), ("raw_value", C.c_int32), ("reserved", C.c_int32)])
 
 
 class VinePpoMinibatch(C.Structure):
@@ -236,7 +238,7 @@ class VinePpoMinibatch(C.Structure):
         + [("dh3_ext", C.c_void_p)]
         + [(n, C.c_int32) for n in ("lr_linear", "schedule_standard", "epoch_begin", "mini_epoch_begin", "max_epochs",
                                     "value_loss_unclipped")]
-        + [("lr0", C.c_float), ("reserved_f2", C.c_float)])
+        + [("lr0", C.c_float), ("raw_obs", C.c_int32)])
 
 # argument structs of the PPO entry points in the order of vine_abi_struct_size()
 PPO_STRUCTS = [VinePolicyAct, VineRolloutPost, VinePpoPrologue, VinePpoMinibatch, VineLstmStep, VineLstmHead, VineLstmHeadTrain,

@@ -286,6 +286,7 @@ __device__ __forceinline__ float wsum(float v) {
   return v;
 }
 
+template <bool RAW_VALUE>   // VineLstmHead.raw_value (normalize_value off)
 __global__ void __launch_bounds__(256) vine_lstm_head_kernel(const VineLstmHead a) {
   vine_launch::grid_dependency_sync();
   const int lane = threadIdx.x & 31;
@@ -301,7 +302,7 @@ __global__ void __launch_bounds__(256) vine_lstm_head_kernel(const VineLstmHead 
   const bool sample = a.actions != nullptr;
   const uint32_t ctr = (sample && a.rng_counter) ? *a.rng_counter : 0u;
   const float ls0 = sample ? a.logstd[0] : 0.f, ls1 = sample ? a.logstd[1] : 0.f;
-  const float vmean = a.value_stats[0], vstd = a.value_stats[1];
+  const float vmean = RAW_VALUE ? 0.f : a.value_stats[0], vstd = RAW_VALUE ? 1.f : a.value_stats[1];
   for (int64_t s = warp0; s < a.n; s += nwarps) {
     const int64_t tile = s / TILE;
     const int row = (int)(s % TILE), unit = 8 * lane;
@@ -330,7 +331,7 @@ __global__ void __launch_bounds__(256) vine_lstm_head_kernel(const VineLstmHead 
     }
     const float mu0 = wsum(d0) + bh[0], mu1 = wsum(d1) + bh[1], v = wsum(d2) + bh[2];
     if (lane == 0) {
-      const float value = fminf(fmaxf(v, -5.f), 5.f) * vstd + vmean;
+      const float value = RAW_VALUE ? v : fminf(fmaxf(v, -5.f), 5.f) * vstd + vmean;
       if (a.mu) *reinterpret_cast<float2*>(a.mu + 2 * s) = make_float2(mu0, mu1);
       if (a.value) a.value[s] = value;
       if (sample) {
@@ -1238,11 +1239,12 @@ int vine_lstm_head_train(const VineLstmHeadTrain* a, void* stream) {
 }
 
 int vine_lstm_head(const VineLstmHead* a, void* stream) {
-  if (!a || !a->params || !a->hh || !a->value_stats || a->n <= 0) return VINE_ERR_INVALID_ARG;
+  if (!a || !a->params || !a->hh || (!a->raw_value && !a->value_stats) || a->n <= 0) return VINE_ERR_INVALID_ARG;
   if (a->actions && !a->logstd) return VINE_ERR_INVALID_ARG;
   int64_t blocks = (a->n + 7) / 8;
   if (blocks > 148 * 8) blocks = 148 * 8;
-  vine_launch::launch(vine_lstm_head_kernel, (unsigned)blocks, 256, 0, (cudaStream_t)stream, *a);
+  if (a->raw_value) vine_launch::launch(vine_lstm_head_kernel<true>, (unsigned)blocks, 256, 0, (cudaStream_t)stream, *a);
+  else vine_launch::launch(vine_lstm_head_kernel<false>, (unsigned)blocks, 256, 0, (cudaStream_t)stream, *a);
   return cudaGetLastError() == cudaSuccess ? VINE_OK : VINE_ERR_CUDA;
 }
 

@@ -180,8 +180,10 @@ __device__ __forceinline__ float bf16_at(const uint8_t* tile, int row, int col, 
 }
 
 // normalised observation row -> bf16 x tile (this thread: 16 of the 32 padded columns of its row); optionally copies
-// the raw observation out (rollout buffer) and plants the constant 1 in column 31 (bias gradient through dW1)
-template <int CPT = 16>   // columns per thread: 16 (two threads per row) or 8 (four threads per row)
+// the raw observation out (rollout buffer) and plants the constant 1 in column 31 (bias gradient through dW1).
+// RAW (normalize_input off): x = obs as it is, mean / inv_std are not read and there is no clamp.  A template parameter, so
+// the normalising instantiation is the same code whether or not the raw one exists.
+template <int CPT = 16, bool RAW = false>   // columns per thread: 16 (two threads per row) or 8 (four threads per row)
 __device__ __forceinline__ void build_x_tile(uint8_t* x_t, int row, int part, bool valid, const float* __restrict__ obs_row,
                                              const float* __restrict__ mean, const float* __restrict__ inv_std, int O,
                                              bool ones_column, float* __restrict__ obs_copy_row) {
@@ -194,7 +196,7 @@ __device__ __forceinline__ void build_x_tile(uint8_t* x_t, int row, int part, bo
     if (valid && k < O) {
       const float raw = obs_row[k];
       if (obs_copy_row) obs_copy_row[k] = raw;
-      v = fminf(fmaxf((raw - mean[k]) * inv_std[k], -5.f), 5.f);
+      v = RAW ? raw : fminf(fmaxf((raw - mean[k]) * inv_std[k], -5.f), 5.f);
     }
     if (ones_column && valid && k == K1 - 1) v = 1.f;
     x[i] = v;

@@ -82,7 +82,8 @@ __device__ __forceinline__ void lr_schedule_rule(const MbArgs& a, float kl) {
 
 // Q = epilogue threads per row (2 or 4): thread (row, part) owns the columns [part * N/Q, (part+1) * N/Q) of every N-wide
 // accumulator; with Q = 4 the SM has 4 warps per sub-partition to hide the TMEM/shared-memory latencies of the epilogues.
-template <int Q>
+// RAW_OBS: normalize_input off (VinePpoMinibatch.raw_obs), the observations enter as they are.
+template <int Q, bool RAW_OBS>
 __global__ void __launch_bounds__(128 * Q, 1) vine_ppo_minibatch_kernel(const MbArgs a) {
   vine_launch::grid_dependency_sync();
   extern __shared__ __align__(1024) uint8_t smem[];
@@ -185,7 +186,7 @@ __global__ void __launch_bounds__(128 * Q, 1) vine_ppo_minibatch_kernel(const Mb
       nlpo = a.nlp_old[grow], vo = a.val_old[grow], ret = a.ret[grow], adv = a.adv[grow];
     }
     // ---- x tile: normalised observation, bf16, zero padded to K1; column 31 is the constant 1 (bias gradient) ----
-    build_x_tile<K1 / Q>(x_t, row, part, valid, a.obs + grow * a.O, a.obs_mean, a.obs_inv_std, a.O, true, nullptr);
+    build_x_tile<K1 / Q, RAW_OBS>(x_t, row, part, valid, a.obs + grow * a.O, a.obs_mean, a.obs_inv_std, a.O, true, nullptr);
     // =============================== forward ===============================
 #pragma unroll 1
     for (int h = 0; h < 2; ++h) {   // layer 1 in two halves of 128 output features (working accumulator = 128 columns)
@@ -617,7 +618,8 @@ int vine_ppo_max_ctas(void) {
 }
 
 int vine_ppo_minibatch(const VinePpoMinibatch* b, void* stream) {
-  if (!b || !b->packed || !b->obs || !b->obs_mean || !b->obs_inv_std || !b->logstd || !b->logstd_old || !b->workspace || !b->state)
+  if (!b || !b->packed || !b->obs || (!b->raw_obs && (!b->obs_mean || !b->obs_inv_std)) || !b->logstd || !b->logstd_old ||
+      !b->workspace || !b->state)
     return VINE_ERR_INVALID_ARG;
   if (!b->dh3_ext && (!b->actions || !b->mu_old || !b->neglogp_old || !b->values_old || !b->returns || !b->advantages))
     return VINE_ERR_INVALID_ARG;
@@ -629,8 +631,10 @@ int vine_ppo_minibatch(const VinePpoMinibatch* b, void* stream) {
   int dev = 0, sms = 0;
   if (cudaGetDevice(&dev) != cudaSuccess) return VINE_ERR_CUDA;
   if (configured != dev) {
-    if (cudaFuncSetAttribute(vine_ppo_minibatch_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES) != cudaSuccess ||
-        cudaFuncSetAttribute(vine_ppo_minibatch_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES) != cudaSuccess)
+    if (cudaFuncSetAttribute(vine_ppo_minibatch_kernel<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES) != cudaSuccess ||
+        cudaFuncSetAttribute(vine_ppo_minibatch_kernel<4, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES) != cudaSuccess ||
+        cudaFuncSetAttribute(vine_ppo_minibatch_kernel<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES) != cudaSuccess ||
+        cudaFuncSetAttribute(vine_ppo_minibatch_kernel<4, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES) != cudaSuccess)
       return VINE_ERR_CUDA;
     configured = dev;
   }
@@ -651,8 +655,14 @@ int vine_ppo_minibatch(const VinePpoMinibatch* b, void* stream) {
   a.inv_B = 1.0f / (float)B, a.kl_threshold = b->kl_threshold, a.lr_min = b->lr_min, a.lr_max = b->lr_max, a.adaptive = b->adaptive_lr;
   a.lr0 = b->lr0, a.linear = b->lr_linear, a.standard = b->schedule_standard, a.epoch_begin = b->epoch_begin;
   a.mini_epoch_begin = b->mini_epoch_begin, a.max_epochs = b->max_epochs, a.clip_value = !b->value_loss_unclipped;
-  if (q4) vine_launch::launch(vine_ppo_minibatch_kernel<4>, grid, 512, SMEM_BYTES, (cudaStream_t)stream, a);
-  else vine_launch::launch(vine_ppo_minibatch_kernel<2>, grid, 256, SMEM_BYTES, (cudaStream_t)stream, a);
+  const cudaStream_t st = (cudaStream_t)stream;
+  if (b->raw_obs) {
+    if (q4) vine_launch::launch(vine_ppo_minibatch_kernel<4, true>, grid, 512, SMEM_BYTES, st, a);
+    else vine_launch::launch(vine_ppo_minibatch_kernel<2, true>, grid, 256, SMEM_BYTES, st, a);
+  } else {
+    if (q4) vine_launch::launch(vine_ppo_minibatch_kernel<4, false>, grid, 512, SMEM_BYTES, st, a);
+    else vine_launch::launch(vine_ppo_minibatch_kernel<2, false>, grid, 256, SMEM_BYTES, st, a);
+  }
   if (cudaGetLastError() != cudaSuccess) return VINE_ERR_CUDA;
   return grid;   // number of gradient partials written (>= 1)
 }

@@ -24,6 +24,8 @@ constexpr int OFF_BAR = OFF_END;
 constexpr int ACT_SMEM_BYTES = OFF_BAR + 64;
 constexpr uint32_t VINE_SITE_POLICY = 16;   // Philox "site" of the policy's action noise (env sites: vine_params.h:20)
 
+// RAW_OBS / RAW_VALUE: VinePolicyAct.raw_obs / raw_value (normalize_input / normalize_value off), one instantiation each
+template <bool RAW_OBS, bool RAW_VALUE>
 __global__ void __launch_bounds__(THREADS, 1) vine_policy_act_kernel(const VinePolicyAct a) {
   vine_launch::grid_dependency_sync();
   extern __shared__ __align__(1024) uint8_t smem[];
@@ -72,7 +74,7 @@ __global__ void __launch_bounds__(THREADS, 1) vine_policy_act_kernel(const VineP
   const uint32_t ctr = (sample && a.rng_counter) ? *a.rng_counter : 0u;
   float ls0 = 0.f, ls1 = 0.f;
   if (sample) ls0 = a.logstd[0], ls1 = a.logstd[1];
-  const float vmean = a.value_stats[0], vstd = a.value_stats[1];
+  const float vmean = RAW_VALUE ? 0.f : a.value_stats[0], vstd = RAW_VALUE ? 1.f : a.value_stats[1];
   const int O = a.num_obs;
   const int64_t ntiles = (a.n + TILE - 1) / TILE;
 
@@ -80,7 +82,7 @@ __global__ void __launch_bounds__(THREADS, 1) vine_policy_act_kernel(const VineP
     const int64_t e = tile * TILE + row;
     // a padded row of a recurrent minibatch (u_step_*) reads no observation: its U row is that of a zero input, finite
     const bool valid = e < a.n && (a.u_step_rows == 0 || e % a.u_step_rows < a.u_step_seqs);
-    build_x_tile(x_t, row, half, valid, a.obs + e * O, a.obs_mean, a.obs_inv_std, O, a.u_out != nullptr,
+    build_x_tile<16, RAW_OBS>(x_t, row, half, valid, a.obs + e * O, a.obs_mean, a.obs_inv_std, O, a.u_out != nullptr,
                  (valid && a.obs_copy) ? a.obs_copy + e * O : nullptr);
 #pragma unroll 1
     for (int h = 0; h < 2; ++h) {
@@ -113,7 +115,7 @@ __global__ void __launch_bounds__(THREADS, 1) vine_policy_act_kernel(const VineP
       if (valid) {
         const float* bh = biases + H1 + H2 + H3;
         const float mu0 = __uint_as_float(r[0]) + bh[0], mu1 = __uint_as_float(r[1]) + bh[1], v = __uint_as_float(r[2]) + bh[2];
-        const float value = fminf(fmaxf(v, -5.f), 5.f) * vstd + vmean;   // RunningMeanStd(unnorm=True)
+        const float value = RAW_VALUE ? v : fminf(fmaxf(v, -5.f), 5.f) * vstd + vmean;   // RunningMeanStd(unnorm=True)
         if (a.mu) *reinterpret_cast<float2*>(a.mu + 2 * e) = make_float2(mu0, mu1);
         if (a.value) a.value[e] = value;
         if (sample) {
@@ -181,11 +183,12 @@ __global__ void __launch_bounds__(256) vine_rollout_post_kernel(const VineRollou
 
 // ---------------------------------------------------------------------------------------------------------------
 // moments layout (f64): [0,O) sum obs, [O,2O) sum obs^2, then sum v, sum v^2 (values and returns pooled), sum adv, sum adv^2
+// raw_obs: the observation columns are skipped (they stay zero; the layout, and with it the all-reduce, does not change)
 __global__ void __launch_bounds__(256) vine_ppo_moments_kernel(const VinePpoPrologue a) {
   __shared__ double red[8][2 * 32];
   const int tid = threadIdx.x, f = tid & 31, lane8 = tid >> 5, O = a.num_obs;
   double s = 0.0, q = 0.0;
-  if (f < O)
+  if (f < O && !a.raw_obs)
     for (int64_t i = (int64_t)blockIdx.x * 8 + lane8; i < a.count; i += (int64_t)gridDim.x * 8) {
       const double x = a.obs[i * O + f];
       s += x, q += x * x;
@@ -196,7 +199,7 @@ __global__ void __launch_bounds__(256) vine_ppo_moments_kernel(const VinePpoProl
     double t = 0.0;
     for (int w = 0; w < 8; ++w) t += red[w][tid];
     const int ff = tid & 31;
-    if (ff < O) atomicAdd(a.moments + (tid < 32 ? ff : O + ff), t);
+    if (ff < O && !a.raw_obs) atomicAdd(a.moments + (tid < 32 ? ff : O + ff), t);
   }
   __syncthreads();
   double m[4] = {0.0, 0.0, 0.0, 0.0};
@@ -231,7 +234,7 @@ __device__ inline void rms_merge(double sum, double sumsq, double n, double* mea
 __global__ void vine_ppo_finalize_kernel(const VinePpoPrologue a) {
   const int tid = threadIdx.x, O = a.num_obs;
   const double n = (double)a.count * a.world;   // moments were summed over ranks
-  if (tid < O) {
+  if (tid < O && !a.raw_obs) {   // normalize_input off: the observation statistics are not touched
     double mean = a.obs_mean[tid], var = a.obs_var[tid], cnt;
     rms_merge(a.moments[tid], a.moments[O + tid], n, &mean, &var, *a.obs_count, &cnt);
     a.obs_mean[tid] = mean, a.obs_var[tid] = var;
@@ -240,12 +243,14 @@ __global__ void vine_ppo_finalize_kernel(const VinePpoPrologue a) {
   }
   __syncthreads();   // every thread has read the old obs count
   if (tid == 0) {
-    *a.obs_count += n;
-    double mean = *a.val_mean, var = *a.val_var, cnt;
-    rms_merge(a.moments[2 * O], a.moments[2 * O + 1], 2.0 * n, &mean, &var, *a.val_count, &cnt);
-    *a.val_mean = mean, *a.val_var = var, *a.val_count = cnt;
-    a.value_stats[0] = (float)mean;
-    a.value_stats[1] = sqrtf((float)var + 1e-5f);
+    if (!a.raw_obs) *a.obs_count += n;
+    if (!a.raw_value) {   // normalize_value off: the value statistics are not touched
+      double mean = *a.val_mean, var = *a.val_var, cnt;
+      rms_merge(a.moments[2 * O], a.moments[2 * O + 1], 2.0 * n, &mean, &var, *a.val_count, &cnt);
+      *a.val_mean = mean, *a.val_var = var, *a.val_count = cnt;
+      a.value_stats[0] = (float)mean;
+      a.value_stats[1] = sqrtf((float)var + 1e-5f);
+    }
     const double am = a.moments[2 * O + 2] / n;
     const double astd = sqrt(fmax((a.moments[2 * O + 3] - n * am * am) / (n - 1.0), 0.0));
     a.adv_stats[0] = a.normalize_advantage ? (float)am : 0.f;
@@ -258,10 +263,15 @@ __global__ void vine_ppo_finalize_kernel(const VinePpoPrologue a) {
 __global__ void __launch_bounds__(256) vine_ppo_normalize_kernel(const VinePpoPrologue a) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= a.count) return;
-  const float vm = a.value_stats[0], vinv = 1.f / a.value_stats[1];
   const float v = a.values[i], r = a.returns[i];
-  a.values_n[i] = fminf(fmaxf((v - vm) * vinv, -5.f), 5.f);
-  a.returns_n[i] = fminf(fmaxf((r - vm) * vinv, -5.f), 5.f);
+  if (a.raw_value) {   // normalize_value off: the value targets enter the loss as they are
+    a.values_n[i] = v;
+    a.returns_n[i] = r;
+  } else {
+    const float vm = a.value_stats[0], vinv = 1.f / a.value_stats[1];
+    a.values_n[i] = fminf(fmaxf((v - vm) * vinv, -5.f), 5.f);
+    a.returns_n[i] = fminf(fmaxf((r - vm) * vinv, -5.f), 5.f);
+  }
   a.advantages_n[i] = ((r - v) - a.adv_stats[0]) * a.adv_stats[1];
 }
 
@@ -270,35 +280,38 @@ __global__ void __launch_bounds__(256) vine_ppo_normalize_kernel(const VinePpoPr
 extern "C" {
 
 int vine_policy_act(const VinePolicyAct* a, void* stream) {
-  if (!a || !a->packed || !a->obs || !a->obs_mean || !a->obs_inv_std || !a->value_stats || a->n <= 0 || a->num_obs < 1 ||
-      a->num_obs > K1 || (((uintptr_t)a->packed) & 15u))
+  if (!a || !a->packed || !a->obs || (!a->raw_obs && (!a->obs_mean || !a->obs_inv_std)) || (!a->raw_value && !a->value_stats) ||
+      a->n <= 0 || a->num_obs < 1 || a->num_obs > K1 || (((uintptr_t)a->packed) & 15u))
     return VINE_ERR_INVALID_ARG;
   if (a->actions && !a->logstd) return VINE_ERR_INVALID_ARG;
   if (!a->actions && !a->mu && !a->value && !a->u_out) return VINE_ERR_INVALID_ARG;
   if (a->u_out && (a->num_obs >= K1 || (((uintptr_t)a->u_out) & 15u))) return VINE_ERR_INVALID_ARG;
   if (a->u_step_rows != 0 && (!a->u_out || a->u_step_rows < 0 || a->u_step_seqs < 1 || a->u_step_seqs > a->u_step_rows))
     return VINE_ERR_INVALID_ARG;
+  static void (*const kernels[4])(const VinePolicyAct) = {vine_policy_act_kernel<false, false>, vine_policy_act_kernel<false, true>,
+                                                          vine_policy_act_kernel<true, false>, vine_policy_act_kernel<true, true>};
   static int configured = -1;
   int dev = 0, sms = 0;
   if (cudaGetDevice(&dev) != cudaSuccess) return VINE_ERR_CUDA;
   if (configured != dev) {
-    if (cudaFuncSetAttribute(vine_policy_act_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, ACT_SMEM_BYTES) != cudaSuccess)
-      return VINE_ERR_CUDA;
+    for (auto k : kernels)
+      if (cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, ACT_SMEM_BYTES) != cudaSuccess) return VINE_ERR_CUDA;
     configured = dev;
   }
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   const int64_t ntiles = (a->n + TILE - 1) / TILE;
   const int grid = (int)(ntiles < sms ? ntiles : sms);
-  vine_launch::launch(vine_policy_act_kernel, grid, THREADS, ACT_SMEM_BYTES, (cudaStream_t)stream, *a);
+  vine_launch::launch(kernels[2 * (a->raw_obs != 0) + (a->raw_value != 0)], grid, THREADS, ACT_SMEM_BYTES, (cudaStream_t)stream, *a);
   return cudaGetLastError() == cudaSuccess ? VINE_OK : VINE_ERR_CUDA;
 }
 
 int vine_mlp_forward(const void* packed, const float* obs, const float* obs_mean, const float* obs_inv_std, int64_t n,
                      int num_obs, const float* value_stats, float* mu, float* value, void* stream) {
-  if (!mu || !value) return VINE_ERR_INVALID_ARG;
+  if (!mu || !value || (!obs_mean) != (!obs_inv_std)) return VINE_ERR_INVALID_ARG;
   VinePolicyAct a = {};
   a.packed = packed, a.obs = obs, a.obs_mean = obs_mean, a.obs_inv_std = obs_inv_std, a.value_stats = value_stats;
   a.mu = mu, a.value = value, a.n = n, a.num_obs = num_obs;
+  a.raw_obs = !obs_mean, a.raw_value = !value_stats;   // NULL statistics: that normaliser is off
   return vine_policy_act(&a, stream);
 }
 
@@ -311,9 +324,11 @@ int vine_rollout_post(const VineRolloutPost* a, void* stream) {
 }
 
 static int prologue_ok(const VinePpoPrologue* a) {
-  return a && a->obs && a->values && a->returns && a->moments && a->obs_mean && a->obs_var && a->obs_count && a->val_mean &&
-         a->val_var && a->val_count && a->obs_mean_f && a->obs_inv_std_f && a->value_stats && a->adv_stats && a->values_n &&
-         a->returns_n && a->advantages_n && a->count > 1 && a->num_obs >= 1 && a->num_obs <= 32 && a->world >= 1;
+  if (!a) return 0;
+  const bool obs_ok = a->raw_obs || (a->obs && a->obs_mean && a->obs_var && a->obs_count && a->obs_mean_f && a->obs_inv_std_f);
+  const bool val_ok = a->raw_value || (a->val_mean && a->val_var && a->val_count && a->value_stats);
+  return obs_ok && val_ok && a->values && a->returns && a->moments && a->adv_stats && a->values_n && a->returns_n &&
+         a->advantages_n && a->count > 1 && a->num_obs >= 1 && a->num_obs <= 32 && a->world >= 1;
 }
 
 int vine_ppo_moments(const VinePpoPrologue* a, void* stream) {

@@ -6,6 +6,8 @@ LSTM state between calls -- without rl_games.
 ``VineRobotControlModel.get_action(q, qd, tip_pos, tip_vel, target_pos)`` == vine_robot_test_model.py:143-177
 
 Checkpoints: the rl_games layout ``PPOAgent.state_dict`` writes (``model`` -> ``a2c_network.*``, ``running_mean_std.*``).
+A file without ``running_mean_std.*`` comes from a run with ``normalize_input: False``: the policy then acts on the raw
+observations (no mean, std or +-5 clamp), as it did in training.
 Runs wherever torch runs (the robot-side host may have no GPU); on a B200 the batched MLP policy can instead go through
 ``vine_policy_act``.
 """
@@ -17,10 +19,15 @@ REFERENCE_RNN = {"name": "lstm", "units": 256, "layers": 1, "before_mlp": False,
 
 
 class PolicyPlayer:
-    def __init__(self, num_obs, num_actions=2, units=(256, 128, 64), rnn="auto", device="cpu", clip_actions=True):
+    def __init__(self, num_obs, num_actions=2, units=(256, 128, 64), rnn="auto", device="cpu", clip_actions=True,
+                 normalize_input="auto"):
+        """``normalize_input``: "auto" = whether the checkpoint has the input normaliser (``running_mean_std.*``), or the
+        training config's bool (then a file that disagrees is refused)."""
         self.device, self.clip_actions, self._rnn_arg = torch.device(device), clip_actions, rnn
         self.num_obs, self.num_actions, self.units = num_obs, num_actions, tuple(units)
+        self._norm_arg = normalize_input
         self.model = self.obs_rms = self.states = None
+        self.normalize_input = True
 
     def _build(self, has_rnn):
         rnn = REFERENCE_RNN if has_rnn else None
@@ -37,6 +44,9 @@ class PolicyPlayer:
         rms = {k[len("running_mean_std."):]: v for k, v in model.items() if k.startswith("running_mean_std.")}
         if not rms and "running_mean_std" in ck:          # vine_robot_test_model.py:137-139
             rms = ck["running_mean_std"]
+        self.normalize_input = bool(rms) if self._norm_arg == "auto" else bool(self._norm_arg)
+        if bool(rms) != self.normalize_input:
+            raise ValueError(f"normalize_input={self.normalize_input} but the checkpoint {'has' if rms else 'lacks'} running_mean_std.*")
         if rms:
             self.obs_rms.load_state_dict({k: v.to(torch.float64) for k, v in rms.items()})
         return self
@@ -56,7 +66,8 @@ class PolicyPlayer:
         obs = obs.reshape(-1, self.num_obs)
         if self.states is not None and self.states[0].shape[0] != obs.shape[0]:
             self.reset(obs.shape[0])
-        mu, logstd, _, self.states = self.model(self.obs_rms(obs), self.states)
+        x = self.obs_rms(obs) if self.normalize_input else obs
+        mu, logstd, _, self.states = self.model(x, self.states)
         action = mu if is_deterministic else mu + torch.exp(logstd) * torch.randn_like(mu)
         if self.clip_actions:
             action = torch.clamp(action, -1.0, 1.0)

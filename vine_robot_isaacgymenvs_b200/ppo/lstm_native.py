@@ -81,6 +81,8 @@ class NativeLstmPath:
                   state, debug_out=None, writeback=None, p2p=(None, None), position=(0, 0)):
         """obs f32 [L, R, O], scalars f32 [L, R, 8], not_done f32 [L, R] (R = self.R; rows [S, R) of each step are padding
         and never read); self.HM[0] (masked initial hidden state tiles) and self.C0 must already hold the initial LSTM state.  Leaves the gradients in flat_g_mlp / flat_g_lstm.
+        obs_mean = obs_inv_std = None: normalize_input is off and the MLP reads the observations as they are; value_stats = None:
+        normalize_value is off (the scalars' value_old / return are then raw).
         ``writeback`` = (scalars_src [T, N, 8], seq_len, chunks, num_envs, env_begin, env_count): rl_games'
         dataset.update_mu_sigma -- this pass's mu goes back into the source rows and ``logstd_old`` receives ``logstd``.
         ``p2p`` = (MLP channel, LSTM channel) device pointers: multi-GPU, the two gradient sums go into this rank's peer-visible
@@ -89,9 +91,11 @@ class NativeLstmPath:
         (PPOAgent._schedule_fields); without that entry the launch runs the adaptive legacy schedule."""
         lib, L, S, R, tl, st = self.lib, self.L, self.S, self.R, self.tiles, self._stream()
         n = L * R
-        act = abi.VinePolicyAct(packed=_ptr(packed_mlp), obs=_ptr(obs), obs_mean=_ptr(obs_mean), obs_inv_std=_ptr(obs_inv_std),
-                                value_stats=_ptr(value_stats), n=n, num_obs=self.O, u_out=_ptr(self.U), u_step_rows=R,
-                                u_step_seqs=S)
+        raw_obs = int(obs_mean is None)
+        stats = dict(obs_mean=None, obs_inv_std=None) if raw_obs else dict(obs_mean=_ptr(obs_mean), obs_inv_std=_ptr(obs_inv_std))
+        act = abi.VinePolicyAct(packed=_ptr(packed_mlp), obs=_ptr(obs), n=n, num_obs=self.O, u_out=_ptr(self.U), u_step_rows=R,
+                                u_step_seqs=S, raw_obs=raw_obs, raw_value=int(value_stats is None),
+                                value_stats=_ptr(value_stats) if value_stats is not None else None, **stats)
         assert lib.vine_policy_act(C.byref(act), st) == 0
         for t in range(L):
             last = t == L - 1
@@ -124,8 +128,8 @@ class NativeLstmPath:
             assert lib.vine_lstm_bwd_gemm(C.byref(bg), st) == 0
         sched = h["schedule"](*position) if "schedule" in h else dict(
             adaptive_lr=int(h.get("adaptive_lr", 1)), kl_threshold=h.get("kl_threshold", 0.008), lr_min=1e-6, lr_max=1e-2)
-        mb = abi.VinePpoMinibatch(packed=_ptr(packed_mlp), obs=_ptr(obs), obs_mean=_ptr(obs_mean), obs_inv_std=_ptr(obs_inv_std),
-                                  logstd=_ptr(logstd), logstd_old=_ptr(logstd_old), workspace=_ptr(self.mlp_ws), state=_ptr(state),
+        mb = abi.VinePpoMinibatch(packed=_ptr(packed_mlp), obs=_ptr(obs), **stats, raw_obs=raw_obs, logstd=_ptr(logstd),
+                                  logstd_old=_ptr(logstd_old), workspace=_ptr(self.mlp_ws), state=_ptr(state),
                                   horizon=L, num_envs=R, env_begin=0, env_count=S, num_obs=self.O, workspace_ctas=self.mlp_ctas,
                                   e_clip=h["e_clip"], critic_coef=h["critic_coef"], entropy_coef=h["entropy_coef"],
                                   bounds_loss_coef=h["bounds_loss_coef"], dh3_ext=_ptr(self.DH3), **sched)

@@ -159,12 +159,19 @@ def policy_kl(p0_mu, p0_sigma, p1_mu, p1_sigma):
 LR_MIN, LR_MAX = 1e-6, 1e-2   # rl_games AdaptiveScheduler's bounds; LinearScheduler's min_lr is LR_MIN too
 
 
+NORMALISER_KEYS = ("running_mean_std", "value_mean_std")   # checkpoint prefixes of the input / value normaliser
+
+
 def rlgames_model_state(model, obs_rms, val_rms):
     """The ``model`` entry of an rl-games 1.5.2 checkpoint (``A2CBase.get_full_state_weights`` -> ``model.state_dict()`` of
     ``ModelA2CContinuousLogStd.Network``): the network under ``a2c_network.*``, the input normaliser under
-    ``running_mean_std.*`` ([O], [O], []) and the value normaliser under ``value_mean_std.*`` ([1], [1], [])."""
+    ``running_mean_std.*`` ([O], [O], []) and the value normaliser under ``value_mean_std.*`` ([1], [1], []).
+    A normaliser passed as None is off (normalize_input / normalize_value False): rl_games builds no such sub-module, so the
+    file has none of its keys."""
     sd = {"a2c_network." + k: v.detach().clone() for k, v in model.state_dict().items()}
-    for name, rms in (("running_mean_std", obs_rms), ("value_mean_std", val_rms)):
+    for name, rms in zip(NORMALISER_KEYS, (obs_rms, val_rms)):
+        if rms is None:
+            continue
         for k, v in rms.state_dict().items():
             sd[f"{name}.{k}"] = v.detach().clone()
     return sd
@@ -201,6 +208,8 @@ class PPOAgent:
         self.value_bootstrap = bool(c.get("value_bootstrap", False))
         self.normalize_input, self.normalize_value = bool(c["normalize_input"]), bool(c["normalize_value"])
         self.normalize_advantage = bool(c["normalize_advantage"])
+        # the kernels' flags of a normaliser that is off (named for the off state: 0 = rl_games' default, normaliser on)
+        self._raw_flags = dict(raw_obs=int(not self.normalize_input), raw_value=int(not self.normalize_value))
         self.truncate_grads, self.grad_norm = bool(c.get("truncate_grads", False)), float(c.get("grad_norm", 1.0))
         self.bf16 = bool(c.get("mixed_precision", False))
         # an episode counts as a success when the "Position Success" term (1000 x its weight, V5:1507, V5:186-203) fired in
@@ -341,8 +350,6 @@ class PPOAgent:
             why.append(f"{self.A} actions (kernels: 2)")
         if self.O > (30 if self.has_rnn else 31):
             why.append(f"{self.O} observations (kernels: <= {30 if self.has_rnn else 31})")
-        if not (self.normalize_input and self.normalize_value):
-            why.append("normalize_input / normalize_value must both be True")
         if self.has_rnn:
             if int(rnn_cfg.get("units", 0)) != 256 or not rnn_cfg.get("concat_input") or not rnn_cfg.get("layer_norm"):
                 why.append("network.rnn must be the reference's block: units 256, concat_input True, layer_norm True")
@@ -447,9 +454,10 @@ class PPOAgent:
         env, lib, T, n, L = self.env, self._lib, self.T, self.n, self.seq_len
         ptr = lambda x: x.data_ptr()  # noqa: E731
         stream = C.c_void_p(torch.cuda.current_stream().cuda_stream)
-        common = dict(packed=ptr(self._packed), obs=ptr(env._obs_clamped), obs_mean=ptr(self._obs_mean_f),
-                      obs_inv_std=ptr(self._obs_inv_std_f), value_stats=ptr(self._val_stats), n=n, num_obs=self.O)
+        common = dict(packed=ptr(self._packed), obs=ptr(env._obs_clamped), n=n, num_obs=self.O, **self._stat_ptrs(),
+                      **self._raw_flags)
         seed, goff = int(env._seed) ^ 0x5DEECE66D, int(env._global_env_offset)
+        vstats = common["value_stats"]
         self._done_ext[0].copy_(self._done_ext[T])
         torch.sub(self._ones_n, self._done_ext[0], out=self._nd_ext[0])   # later rows are written by vine_rollout_post
         for t in range(T + 1):
@@ -466,14 +474,15 @@ class PPOAgent:
                                   not_done=ptr(self._nd_ext[t]), c=ptr(self._r_C[nxt]), hh=ptr(self._r_HH[nxt]), n=n)
             assert lib.vine_lstm_step(C.byref(st), stream) == 0
             if last:   # bootstrap value of the final observation: the persistent state is NOT advanced
-                hd = abi.VineLstmHead(params=ptr(self._lpacked), hh=ptr(self._r_HH[nxt]), value_stats=ptr(self._val_stats),
-                                      value=ptr(self.last_value), n=n)
+                hd = abi.VineLstmHead(params=ptr(self._lpacked), hh=ptr(self._r_HH[nxt]), value_stats=vstats,
+                                      value=ptr(self.last_value), n=n, raw_value=self._raw_flags["raw_value"])
                 assert lib.vine_lstm_head(C.byref(hd), stream) == 0
                 break
-            hd = abi.VineLstmHead(params=ptr(self._lpacked), hh=ptr(self._r_HH[nxt]), value_stats=ptr(self._val_stats),
+            hd = abi.VineLstmHead(params=ptr(self._lpacked), hh=ptr(self._r_HH[nxt]), value_stats=vstats,
                                   mu=ptr(self.b_mu[t]), value=ptr(self.b_val[t]), logstd=ptr(self.model.sigma),
                                   rng_counter=ptr(self._rng_counter), actions=ptr(self.b_act[t]), neglogp=ptr(self.b_nlp[t]),
-                                  env_actions=ptr(env.actions), n=n, seed=seed, global_env_offset=goff)
+                                  env_actions=ptr(env.actions), n=n, seed=seed, global_env_offset=goff,
+                                  raw_value=self._raw_flags["raw_value"])
             assert lib.vine_lstm_head(C.byref(hd), stream) == 0
             self._r_cur = nxt
             env.step_device()
@@ -502,15 +511,7 @@ class PPOAgent:
         ptr = lambda x: x.data_ptr()  # noqa: E731
         p = lambda x: C.c_void_p(x.data_ptr())  # noqa: E731
         if self._mb_structs is None:
-            self._prologue = abi.VinePpoPrologue(
-                obs=ptr(self.b_obs), values=ptr(self.b_val), returns=ptr(self.b_ret), moments=ptr(self._moments),
-                obs_mean=ptr(self.obs_rms.running_mean), obs_var=ptr(self.obs_rms.running_var),
-                obs_count=ptr(self.obs_rms.count), val_mean=ptr(self.val_rms.running_mean),
-                val_var=ptr(self.val_rms.running_var), val_count=ptr(self.val_rms.count),
-                obs_mean_f=ptr(self._obs_mean_f), obs_inv_std_f=ptr(self._obs_inv_std_f), value_stats=ptr(self._val_stats),
-                adv_stats=ptr(self._adv_stats), values_n=ptr(self._val_old_n), returns_n=ptr(self._ret_n),
-                advantages_n=ptr(self._adv_n), count=T * n, num_obs=self.O, world=self.world,
-                normalize_advantage=int(self.normalize_advantage))
+            self._prologue = self._prologue_struct()
             self._mb_structs = True
         assert lib.vine_ppo_moments(C.byref(self._prologue), stream) == 0
         self._allreduce_moments(stream)
@@ -531,9 +532,10 @@ class PPOAgent:
                                         hm0=ptr(path.HM[0]), seq_len=L, chunks=chunks, num_envs=n, env_begin=e0, env_count=E,
                                         num_obs=self.O, step_rows=path.R)
                 assert lib.vine_lstm_gather(C.byref(ga), stream) == 0
-                path.gradients(self._packed, self._lpacked, self._mb_obs, self._mb_scal, self._mb_nd, self._obs_mean_f,
-                               self._obs_inv_std_f, self._val_stats, self.model.sigma, self._logstd_old[e0 // E], self.ppo_state,
-                               writeback=(self._scal, L, chunks, n, e0, E), p2p=(pm, pl), position=(k, e0 // E))
+                obs_stats = (self._obs_mean_f, self._obs_inv_std_f) if self.normalize_input else (None, None)   # None: off
+                path.gradients(self._packed, self._lpacked, self._mb_obs, self._mb_scal, self._mb_nd, *obs_stats,
+                               self._val_stats if self.normalize_value else None, self.model.sigma, self._logstd_old[e0 // E],
+                               self.ppo_state, writeback=(self._scal, L, chunks, n, e0, E), p2p=(pm, pl), position=(k, e0 // E))
                 if self.grad_allreduce == "nccl":   # baseline: ONE NCCL all-reduce per minibatch (gradients + loss statistics)
                     torch.distributed.all_reduce(path.flat_g)
                 sc = 1.0 / self.world                # p2p: the Adam kernels add the ranks' buffers themselves (vine_p2p.cuh)
@@ -561,6 +563,30 @@ class PPOAgent:
         assert lib.vine_lstm_adam_clipped(p(path.flat_g_lstm), sc, p(self.flat_l), p(self.adam_ml), p(self.adam_vl), p(self._lpacked),
                                           p(self.ppo_state), self.O, 0.9, 0.999, 1e-8, coef, None, stream) == 0
 
+    def _stat_ptrs(self, value=True):
+        """Device pointers of the normalisation statistics the kernels read, as struct fields; a normaliser that is off passes
+        None (its kernel flag is set, nothing is read).  value=False: only the observation statistics."""
+        ptrs = dict(obs_mean=self._obs_mean_f.data_ptr() if self.normalize_input else None,
+                    obs_inv_std=self._obs_inv_std_f.data_ptr() if self.normalize_input else None)
+        if value:
+            ptrs["value_stats"] = self._val_stats.data_ptr() if self.normalize_value else None
+        return ptrs
+
+    def _prologue_struct(self):
+        """VinePpoPrologue of the kernel update: running statistics, normalised value targets and advantages."""
+        ptr = lambda x: x.data_ptr()  # noqa: E731
+        io, iv = self.normalize_input, self.normalize_value
+        obs_fields = dict(obs=ptr(self.b_obs), obs_mean=ptr(self.obs_rms.running_mean), obs_var=ptr(self.obs_rms.running_var),
+                          obs_count=ptr(self.obs_rms.count), obs_mean_f=ptr(self._obs_mean_f),
+                          obs_inv_std_f=ptr(self._obs_inv_std_f)) if io else {}
+        val_fields = dict(val_mean=ptr(self.val_rms.running_mean), val_var=ptr(self.val_rms.running_var),
+                          val_count=ptr(self.val_rms.count), value_stats=ptr(self._val_stats)) if iv else {}
+        return abi.VinePpoPrologue(
+            values=ptr(self.b_val), returns=ptr(self.b_ret), moments=ptr(self._moments), adv_stats=ptr(self._adv_stats),
+            values_n=ptr(self._val_old_n), returns_n=ptr(self._ret_n), advantages_n=ptr(self._adv_n), count=self.T * self.n,
+            num_obs=self.O, world=self.world, normalize_advantage=int(self.normalize_advantage), **obs_fields, **val_fields,
+            **self._raw_flags)
+
     def _allreduce_moments(self, stream):
         """Sum over the ranks of the f64 running-statistics moments (observations, values, advantages), once per iteration:
         over the peer-memory channel (one single-block launch) or, baseline, one NCCL all-reduce."""
@@ -576,10 +602,12 @@ class PPOAgent:
     def _refresh_fused(self, pack=False):
         """Refresh the normalisation statistics the kernels read; ``pack``: also re-pack the weights (bf16, tensor-core
         operand layout) -- only needed when something other than vine_ppo_adam changed them."""
-        self._obs_mean_f.copy_(self.obs_rms.running_mean.float())
-        self._obs_inv_std_f.copy_(torch.rsqrt(self.obs_rms.running_var.float() + self.obs_rms.eps))
-        self._val_stats.copy_(torch.cat([self.val_rms.running_mean.float().reshape(1),
-                                         torch.sqrt(self.val_rms.running_var.float() + self.val_rms.eps).reshape(1)]))
+        if self.normalize_input:   # a normaliser that is off has no statistics the kernels read
+            self._obs_mean_f.copy_(self.obs_rms.running_mean.float())
+            self._obs_inv_std_f.copy_(torch.rsqrt(self.obs_rms.running_var.float() + self.obs_rms.eps))
+        if self.normalize_value:
+            self._val_stats.copy_(torch.cat([self.val_rms.running_mean.float().reshape(1),
+                                             torch.sqrt(self.val_rms.running_var.float() + self.val_rms.eps).reshape(1)]))
         if pack:
             p = lambda x: C.c_void_p(x.data_ptr())  # noqa: E731
             st = C.c_void_p(torch.cuda.current_stream().cuda_stream)
@@ -603,8 +631,9 @@ class PPOAgent:
         """mu, logstd, de-normalised value and the next LSTM state for one observation per env."""
         if self.fused and obs.shape[0] == self.n:
             p = lambda x: C.c_void_p(x.data_ptr())  # noqa: E731
-            rc = self._lib.vine_mlp_forward(p(self._packed), p(obs), p(self._obs_mean_f), p(self._obs_inv_std_f), self.n,
-                                            self.O, p(self._val_stats), p(self._mu_buf), p(self._val_buf),
+            s = self._stat_ptrs()   # NULL statistics: that normaliser is off
+            rc = self._lib.vine_mlp_forward(p(self._packed), p(obs), s["obs_mean"], s["obs_inv_std"], self.n, self.O,
+                                            s["value_stats"], p(self._mu_buf), p(self._val_buf),
                                             C.c_void_p(torch.cuda.current_stream().cuda_stream))
             assert rc == 0
             return self._mu_buf, self.model.sigma.detach().expand(self.n, -1), self._val_buf, None
@@ -623,9 +652,9 @@ class PPOAgent:
         env, lib, T, n = self.env, self._lib, self.T, self.n
         if self._roll_structs is None:
             ptr = lambda x: x.data_ptr()  # noqa: E731
-            common = dict(packed=ptr(self._packed), obs=ptr(env._obs_clamped), obs_mean=ptr(self._obs_mean_f),
-                          obs_inv_std=ptr(self._obs_inv_std_f), value_stats=ptr(self._val_stats), n=n, num_obs=self.O,
-                          seed=int(env._seed) ^ 0x5DEECE66D, global_env_offset=int(env._global_env_offset))
+            common = dict(packed=ptr(self._packed), obs=ptr(env._obs_clamped), n=n, num_obs=self.O,
+                          seed=int(env._seed) ^ 0x5DEECE66D, global_env_offset=int(env._global_env_offset),
+                          **self._stat_ptrs(), **self._raw_flags)
             acts = [abi.VinePolicyAct(mu=ptr(self.b_mu[t]), value=ptr(self.b_val[t]), logstd=ptr(self.model.sigma),
                                       rng_counter=ptr(self._rng_counter), actions=ptr(self.b_act[t]),
                                       neglogp=ptr(self.b_nlp[t]), obs_copy=ptr(self.b_obs[t]), env_actions=ptr(env.actions),
@@ -847,16 +876,7 @@ class PPOAgent:
         T, n, lib = self.T, self.n, self._lib
         stream = C.c_void_p(torch.cuda.current_stream().cuda_stream)
         if self._mb_structs is None:
-            ptr = lambda x: x.data_ptr()  # noqa: E731
-            self._prologue = abi.VinePpoPrologue(
-                obs=ptr(self.b_obs), values=ptr(self.b_val), returns=ptr(self.b_ret), moments=ptr(self._moments),
-                obs_mean=ptr(self.obs_rms.running_mean), obs_var=ptr(self.obs_rms.running_var),
-                obs_count=ptr(self.obs_rms.count), val_mean=ptr(self.val_rms.running_mean),
-                val_var=ptr(self.val_rms.running_var), val_count=ptr(self.val_rms.count),
-                obs_mean_f=ptr(self._obs_mean_f), obs_inv_std_f=ptr(self._obs_inv_std_f), value_stats=ptr(self._val_stats),
-                adv_stats=ptr(self._adv_stats), values_n=ptr(self._val_old_n), returns_n=ptr(self._ret_n),
-                advantages_n=ptr(self._adv_n), count=T * n, num_obs=self.O, world=self.world,
-                normalize_advantage=int(self.normalize_advantage))
+            self._prologue = self._prologue_struct()
         # running statistics + normalised targets: f64 sufficient statistics, [one all-reduce], finalize
         assert lib.vine_ppo_moments(C.byref(self._prologue), stream) == 0
         self._allreduce_moments(stream)
@@ -867,7 +887,7 @@ class PPOAgent:
             self._mb_structs = [[abi.VinePpoMinibatch(
                 packed=ptr(self._packed), obs=ptr(self.b_obs), actions=ptr(self.b_act), mu_old=ptr(self.b_mu),
                 neglogp_old=ptr(self.b_nlp), values_old=ptr(self._val_old_n), returns=ptr(self._ret_n),
-                advantages=ptr(self._adv_n), obs_mean=ptr(self._obs_mean_f), obs_inv_std=ptr(self._obs_inv_std_f),
+                advantages=ptr(self._adv_n), **self._stat_ptrs(value=False), raw_obs=self._raw_flags["raw_obs"],
                 logstd=ptr(self.model.sigma), logstd_old=ptr(self._logstd_old[e0 // self.mb_envs]), workspace=ptr(self._ws),
                 state=ptr(self.ppo_state), debug_out=None, horizon=T, num_envs=n, env_begin=e0, env_count=self.mb_envs,
                 num_obs=self.O, workspace_ctas=self._ctas, e_clip=self.e_clip, critic_coef=self.critic_coef,
@@ -976,9 +996,11 @@ class PPOAgent:
     # ------------------------------------------------------------------ checkpoints
     # Layout of rl-games 1.5.2 ``A2CBase.get_full_state_weights`` -- what the reference's train.py saves under
     # runs/<name>/nn/*.pth and what isaacgymenvs/vine_robot_test_model.py:135-139 reads back: ``model`` holds the
-    # network under ``a2c_network.*`` plus the input/value normalisers as ``running_mean_std.*`` / ``value_mean_std.*``.
+    # network under ``a2c_network.*`` plus the input/value normalisers as ``running_mean_std.*`` / ``value_mean_std.*``
+    # (each only when it is on, like rl_games' Network).
     def rlgames_model_state(self):
-        return rlgames_model_state(self.model, self.obs_rms, self.val_rms)
+        return rlgames_model_state(self.model, self.obs_rms if self.normalize_input else None,
+                                   self.val_rms if self.normalize_value else None)
 
     def _optimizer_state(self):
         if self.fused_update:
@@ -1003,10 +1025,14 @@ class PPOAgent:
             assert set(own) == set(net), (sorted(set(own) ^ set(net)))
             for k, v in own.items():
                 v.copy_(net[k])
-        for name, rms in (("running_mean_std", self.obs_rms), ("value_mean_std", self.val_rms)):
+        for name, rms, on, key in zip(NORMALISER_KEYS, (self.obs_rms, self.val_rms), (self.normalize_input, self.normalize_value),
+                                      ("normalize_input", "normalize_value")):
             sub = {k[len(name) + 1:]: v for k, v in model.items() if k.startswith(name + ".")}
             if not sub and name in sd:          # older layout: normalisers stored beside 'model'
                 sub = sd[name]
+            if bool(sub) != on:   # rl_games' strict load: a surplus or missing normaliser is an error, not a silent default
+                raise ValueError(f"checkpoint {'has' if sub else 'lacks'} {name}.* but {key} is {on}: it was written by a run "
+                                 f"with {key} {not on}")
             if sub:   # value_mean_std is [1] in rl_games files; older files of this trainer stored it 0-dim
                 own = rms.state_dict()
                 rms.load_state_dict({k: v.to(own[k].dtype).reshape(own[k].shape) for k, v in sub.items()})
