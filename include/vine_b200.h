@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define VINE_ABI_VERSION 7
+#define VINE_ABI_VERSION 8
 
 #define VINE_NUM_DOFS 6          /* 1 prismatic rail cart + 5 revolute links (V5:54,83) */
 #define VINE_NUM_ACTIONS 2       /* u_rail_velocity, u_fpam (V5:171) */
@@ -436,12 +436,14 @@ typedef struct VinePolicyAct {
   int64_t global_env_offset;
   void* u_out;                   /* NULL, or [ceil(n/128)] tiles [128 x 128] bf16 (UMMA row-blocked): the LSTM input
                                     [MLP output (64) | x (32, col 31 == 1) | 0]; heads and sampling are
-                                    skipped (they follow the LSTM: vine_lstm_step / vine_lstm_head) */
+                                    skipped (they follow the LSTM: vine_lstm_step / vine_lstm_head).  With u_no_obs the
+                                    x columns 0..30 are 0 (col 31 is still 1) */
   int32_t u_step_rows, u_step_seqs;   /* with u_out: rows come in groups of u_step_rows (one time step of a minibatch padded to
                                     whole tiles), of which the first u_step_seqs are real; the rest read no observation and
                                     get the U row of a zero input.  0, 0: every row is real */
   int32_t raw_value;             /* 1: normalize_value off: value = the value head's output (no clamp, no de-normalisation) */
-  int32_t reserved;              /* 0 */
+  int32_t u_no_obs;              /* 1 (needs u_out): rnn concat_input off: U carries no observation, only the MLP output and
+                                    the constant-1 column.  Every other output is unchanged */
 } VinePolicyAct;
 int vine_policy_act(const VinePolicyAct* args, void* stream);
 
@@ -507,7 +509,9 @@ int vine_ppo_finalize(const VinePpoPrologue* args, void* stream);
 
 /*
  * The recurrent half of the reference's network (Vine5LinkMovingBasePPO.yaml:32-40: lstm 256, concat_input,
- * layer_norm; rl_games A2CBuilder.Network.forward) on hand-written kernels.  Activations live in HBM as 128-row
+ * layer_norm; rl_games A2CBuilder.Network.forward) on hand-written kernels.  Either switch may be off: concat_input off is
+ * VinePolicyAct.u_no_obs (U without the observation, the W_ih observation columns stay 0), layer_norm off is
+ * VineLstmHead / VineLstmHeadTrain.no_layer_norm (the heads act on h; gamma / beta are not read).  Activations live in HBM as 128-row
  * tiles in the UMMA row-blocked layout (one bulk-TMA copy per GEMM operand): u / hm / hh = [tiles][...] as described
  * in csrc/vine_lstm_net.cu; c = f32 [n, 256] row-major.
  *   vine_lstm_pack : torch-layout f32 parameters (W_ih [1024, 64+O], W_hh [1024, 256], b_ih, b_hh, LayerNorm gamma/beta,
@@ -516,8 +520,8 @@ int vine_ppo_finalize(const VinePpoPrologue* args, void* stream);
  *                    h = o tanh(c); writes c, hh (bf16 tiles), optionally hm_next = hh * not_done_next and the activated
  *                    gates (for backward).  Grid = (tiles, 8 slices of 32 hidden units).
  *   vine_lstm_mask : hm = hh * not_done (rollout: the done flag arrives after the step has run).
- *   vine_lstm_head : LayerNorm + mu/value heads per row (+ Philox Gaussian sampling, neglogp, clamped env action: the
- *                    same outputs and Philox keying as vine_policy_act).
+ *   vine_lstm_head : LayerNorm (unless no_layer_norm) + mu/value heads per row (+ Philox Gaussian sampling, neglogp,
+ *                    clamped env action: the same outputs and Philox keying as vine_policy_act).
  */
 #define VINE_LSTM_PACKED_BYTES 795664
 typedef struct VineLstmStep {
@@ -550,7 +554,7 @@ typedef struct VineLstmHead {
   uint64_t seed;
   int64_t global_env_offset;
   int32_t raw_value;             /* 1: normalize_value off: value = the value head's output (no clamp, no de-normalisation) */
-  int32_t reserved;              /* 0 */
+  int32_t no_layer_norm;         /* 1: rnn layer_norm off: the heads act on y = h; LayerNorm gamma / beta are not read */
 } VineLstmHead;
 int vine_lstm_pack(const float* w_ih, const float* w_hh, const float* b_ih, const float* b_hh, const float* ln_gamma,
                    const float* ln_beta, const float* w_mu, const float* b_mu, const float* w_v, const float* b_v,
@@ -566,7 +570,8 @@ int vine_lstm_head(const VineLstmHead* args, void* stream);
  * normalize_value off), return (likewise), advantage (normalised).  grads f32 [VINE_LSTM_HEAD_GRAD_PARTS + 1][VINE_LSTM_HEAD_GRAD_FLOATS] receives one
  * partial per thread block (the call returns how many; vine_lstm_reduce sums them): d(LayerNorm gamma)[256],
  * d(beta)[256], d(W_mu0, W_mu1, W_v)[3][256], d(b)[3] (+1 pad), d(logstd)[2], loss statistics a_loss, c_loss, kl,
- * b_loss (means), padding.
+ * b_loss (means), padding.  With no_layer_norm there is no LayerNorm (y = h, dh = sum_j d_j w_j) and the gamma / beta
+ * slots are exactly 0.
  */
 #define VINE_LSTM_HEAD_GRAD_FLOATS 1296
 #define VINE_LSTM_HEAD_GRAD_PARTS 1184  /* max per-block gradient partials one vine_lstm_head_train call writes */
@@ -589,6 +594,8 @@ typedef struct VineLstmHeadTrain {
   int32_t value_loss_unclipped;  /* 0: clipped value loss (rl_games clip_value True); 1: c_loss = (return - v)^2 */
   int32_t step_seqs;             /* with step_rows: the real sequences at the start of every step; the other (padded) rows
                                     add nothing to the losses, statistics and gradients, get dh = 0 and no mu write-back */
+  int32_t no_layer_norm;         /* 1: rnn layer_norm off (as VineLstmHead.no_layer_norm) */
+  int32_t reserved;              /* 0 */
 } VineLstmHeadTrain;
 int vine_lstm_head_train(const VineLstmHeadTrain* args, void* stream);
 
@@ -629,6 +636,9 @@ int vine_lstm_bwd_gemm(const VineLstmBwdGemm* args, void* stream);
  * Weight gradients and optimiser of the recurrent half.  Flat f32 parameter vector (torch layouts, this order):
  *   W_ih[1024, 64+O] W_hh[1024, 256] b_ih[1024] b_hh[1024] ln_gamma[256] ln_beta[256] W_mu[2,256] b_mu[2] W_v[1,256]
  *   b_v[1] logstd[2]                                   (vine_lstm_num_params(O) floats)
+ *   The layout is the same with either switch of the rnn block off.  Parameters the network then lacks keep their slots
+ *   and get a gradient of exactly 0: W_ih's observation columns (concat_input off: u's observation columns are 0) and
+ *   ln_gamma / ln_beta (layer_norm off), so Adam leaves them where they are.
  *   vine_lstm_wgrad : dW^T = in^T dG over all (step, sequence) rows of the minibatch (tcgen05, both operands MN-major,
  *       rows streamed through a 2-stage bulk-TMA ring); grid = 12 output blocks x `splits` K ranges; partials go to
  *       workspace f32 [splits][12][128][256].  ntiles = number of 128-row tiles of u / hm / dg (all steps).  A padded row

@@ -1,7 +1,8 @@
 """Time one PPO iteration of the reference network (MLP -> LSTM 256 -> LayerNorm) at FSTR, N envs, CUDA-graph replay:
-python tools/ppo_time.py [N] [--minibatch M] [--mlp] [--raw-obs] [--raw-value] [--no-pdl] [--no-arena] [--pad K]
-                         [--truncate-grads [--grad-norm X]]
---raw-obs / --raw-value switch the input / value normaliser off (normalize_input / normalize_value False).  Prints ms per iteration / rollout / update (CUDA events, best of 3 x 20) and the card with its power limit.  --minibatch sets
+python tools/ppo_time.py [N] [--minibatch M] [--mlp] [--raw-obs] [--raw-value] [--no-layer-norm] [--no-concat-input]
+                         [--no-pdl] [--no-arena] [--pad K] [--truncate-grads [--grad-norm X]]
+--raw-obs / --raw-value switch the input / value normaliser off (normalize_input / normalize_value False).
+--no-layer-norm / --no-concat-input switch the rnn block's layer_norm / concat_input off.  Prints ms per iteration / rollout / update (CUDA events, best of 3 x 20) and the card with its power limit.  --minibatch sets
 minibatch_size (default: the config's 32768, which needs N * horizon to be a multiple of it; e.g. N = 4000 wants 32000).
 --truncate-grads also builds a second agent with gradient-norm clipping (truncate_grads=True, grad_norm X, default 1.0) and
 times the two update graphs alternately."""
@@ -24,6 +25,10 @@ if "--raw-obs" in args:
     extra.append("train.params.config.normalize_input=False")
 if "--raw-value" in args:
     extra.append("train.params.config.normalize_value=False")
+if "--no-layer-norm" in args:
+    extra.append("train.params.network.rnn.layer_norm=False")
+if "--no-concat-input" in args:
+    extra.append("train.params.network.rnn.concat_input=False")
 if "--no-pdl" in args:
     PPOAgent.PDL_MAX_ENVS = 0
 if "--no-arena" in args:

@@ -12,7 +12,7 @@ NUM_ACTIONS = 2
 NUM_REWARDS = 13
 NUM_OBJECT_INFO = 2
 MAX_ACTION_DELAY = 8
-ABI_VERSION = 7
+ABI_VERSION = 8
 
 OK = 0
 ERR_INVALID_ARG = -1
@@ -167,7 +167,7 @@ class VinePolicyAct(C.Structure):
         "neglogp", "obs_copy", "env_actions")]
         + [("n", C.c_int64), ("num_obs", C.c_int32), ("raw_obs", C.c_int32), ("seed", C.c_uint64),
            ("global_env_offset", C.c_int64), ("u_out", C.c_void_p), ("u_step_rows", C.c_int32), ("u_step_seqs", C.c_int32),
-           ("raw_value", C.c_int32), ("reserved", C.c_int32)])
+           ("raw_value", C.c_int32), ("u_no_obs", C.c_int32)])
 
 
 class VineLstmStep(C.Structure):
@@ -179,7 +179,7 @@ class VineLstmHead(C.Structure):
     _fields_ = ([(n, C.c_void_p) for n in ("params", "hh", "value_stats", "mu", "value", "logstd", "rng_counter", "actions",
                                            "neglogp", "env_actions")]
                 + [("n", C.c_int64), ("seed", C.c_uint64), ("global_env_offset", C.c_int64), ("raw_value", C.c_int32),
-                   ("reserved", C.c_int32)])
+                   ("no_layer_norm", C.c_int32)])
 
 
 class VineLstmHeadTrain(C.Structure):
@@ -188,7 +188,8 @@ class VineLstmHeadTrain(C.Structure):
                 + [(n, C.c_float) for n in ("e_clip", "critic_coef", "entropy_coef", "bounds_loss_coef", "inv_B")]
                 + [("step_rows", C.c_int32), ("mu_writeback", C.c_void_p)]
                 + [(n, C.c_int64) for n in ("wb_seq_len", "wb_chunks", "wb_num_envs", "wb_env_begin", "wb_env_count")]
-                + [("value_loss_unclipped", C.c_int32), ("step_seqs", C.c_int32)])
+                + [("value_loss_unclipped", C.c_int32), ("step_seqs", C.c_int32), ("no_layer_norm", C.c_int32),
+                   ("reserved", C.c_int32)])
 
 
 class VineLstmCellBwd(C.Structure):

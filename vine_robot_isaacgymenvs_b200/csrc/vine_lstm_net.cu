@@ -1,6 +1,8 @@
 // vine_lstm_net.cu — the recurrent half of the reference's actor-critic on hand-written sm_100a kernels:
 //   u = [MLP(x) (64) | x (32, padded)]  ->  LSTM 256 (gates = u W_ih^T + h W_hh^T + b, torch order i,f,g,o)  ->  LayerNorm
 //   ->  mu (2), value (1)                                   (cfg/train/Vine5LinkMovingBasePPO.yaml:10-40, rl_games A2CBuilder)
+// Either switch of the block may be off: concat_input off leaves x's columns of U at 0 (vine_policy_act u_no_obs; W_ih keeps
+// its 64+O columns, the observation ones stay 0), layer_norm off makes the heads act on h (no_layer_norm instantiations).
 //
 // Data lives in HBM as 128-row tiles in the UMMA row-blocked layout (vine_umma.cuh), so every GEMM operand is one bulk-TMA
 // copy and the same bytes serve forward (K-major) and backward/weight-gradient (MN-major) GEMMs:
@@ -16,7 +18,7 @@
 // vine_lstm_step  : one LSTM time step for every 128-sequence tile; CTA = (tile, half of the hidden units): resident A tile,
 //                   weight pieces streamed through a bulk-TMA ring, tcgen05.mma into ping-pong TMEM accumulators, cell
 //                   epilogue per row overlapped with the next piece (warp-specialised).
-// vine_lstm_head  : LayerNorm + heads per row (one warp per row) + Gaussian sampling / neglogp (rollout).
+// vine_lstm_head  : LayerNorm (unless no_layer_norm) + heads per row (one warp per row) + Gaussian sampling / neglogp (rollout).
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -286,7 +288,9 @@ __device__ __forceinline__ float wsum(float v) {
   return v;
 }
 
-template <bool RAW_VALUE>   // VineLstmHead.raw_value (normalize_value off)
+// RAW_VALUE: VineLstmHead.raw_value (normalize_value off); NO_LN: VineLstmHead.no_layer_norm (layer_norm off: the heads act on
+// y = h, gamma / beta are not read)
+template <bool RAW_VALUE, bool NO_LN>
 __global__ void __launch_bounds__(256) vine_lstm_head_kernel(const VineLstmHead a) {
   vine_launch::grid_dependency_sync();
   const int lane = threadIdx.x & 31;
@@ -298,7 +302,10 @@ __global__ void __launch_bounds__(256) vine_lstm_head_kernel(const VineLstmHead 
   const float* bh = reinterpret_cast<const float*>(P + LP_BH);
   float g[8], b[8], w0[8], w1[8], w2[8];
 #pragma unroll
-  for (int k = 0; k < 8; ++k) g[k] = lng[k], b[k] = lnb[k], w0[k] = wh[k], w1[k] = wh[HID + k], w2[k] = wh[2 * HID + k];
+  for (int k = 0; k < 8; ++k) {
+    if (!NO_LN) g[k] = lng[k], b[k] = lnb[k];
+    w0[k] = wh[k], w1[k] = wh[HID + k], w2[k] = wh[2 * HID + k];
+  }
   const bool sample = a.actions != nullptr;
   const uint32_t ctr = (sample && a.rng_counter) ? *a.rng_counter : 0u;
   const float ls0 = sample ? a.logstd[0] : 0.f, ls1 = sample ? a.logstd[1] : 0.f;
@@ -316,17 +323,20 @@ __global__ void __launch_bounds__(256) vine_lstm_head_kernel(const VineLstmHead 
       h[2 * k] = f.x, h[2 * k + 1] = f.y;
     }
     // same summation order as vine_lstm_head_train_kernel: the first training pass reproduces the rollout's mu bit for bit
-    const float sm = ((h[0] + h[1]) + (h[2] + h[3])) + ((h[4] + h[5]) + (h[6] + h[7]));
-    const float mean = wsum(sm) * (1.f / HID);
-    float t[8];
+    float rstd = 1.f;
+    if (!NO_LN) {
+      const float sm = ((h[0] + h[1]) + (h[2] + h[3])) + ((h[4] + h[5]) + (h[6] + h[7]));
+      const float mean = wsum(sm) * (1.f / HID);
+      float t[8];
 #pragma unroll
-    for (int k = 0; k < 8; ++k) h[k] -= mean, t[k] = h[k] * h[k];
-    const float sq = ((t[0] + t[1]) + (t[2] + t[3])) + ((t[4] + t[5]) + (t[6] + t[7]));
-    const float rstd = rsqrtf(wsum(sq) * (1.f / HID) + 1e-5f);     // torch.nn.LayerNorm: biased variance, eps 1e-5
+      for (int k = 0; k < 8; ++k) h[k] -= mean, t[k] = h[k] * h[k];
+      const float sq = ((t[0] + t[1]) + (t[2] + t[3])) + ((t[4] + t[5]) + (t[6] + t[7]));
+      rstd = rsqrtf(wsum(sq) * (1.f / HID) + 1e-5f);     // torch.nn.LayerNorm: biased variance, eps 1e-5
+    }
     float d0 = 0.f, d1 = 0.f, d2 = 0.f;
 #pragma unroll
     for (int k = 0; k < 8; ++k) {
-      const float y = fmaf(h[k] * rstd, g[k], b[k]);
+      const float y = NO_LN ? h[k] : fmaf(h[k] * rstd, g[k], b[k]);
       d0 = fmaf(y, w0[k], d0), d1 = fmaf(y, w1[k], d1), d2 = fmaf(y, w2[k], d2);
     }
     const float mu0 = wsum(d0) + bh[0], mu1 = wsum(d1) + bh[1], v = wsum(d2) + bh[2];
@@ -364,7 +374,9 @@ constexpr int HT_ROWS = 2;
 
 // PADDED: the minibatch has padded rows (step_rows != 0).  A separate instantiation, so that the dense rows of an aligned
 // minibatch run the same code as before padding existed (the padded-row tests cost registers in this 128-register kernel).
-template <bool PADDED>
+// NO_LN: VineLstmHeadTrain.no_layer_norm (layer_norm off): forward y = h, backward dh = sum_j d_j w_j, d(w_j) = A_j with
+// A_j[k] = sum_rows d_j h[k]; gamma / beta are not read and their gradient slots stay 0.
+template <bool PADDED, bool NO_LN>
 __global__ void __launch_bounds__(256, 2) vine_lstm_head_train_kernel(const VineLstmHeadTrain a) {
   vine_launch::grid_dependency_sync();
   __shared__ float red[HG_FLOATS];
@@ -372,7 +384,7 @@ __global__ void __launch_bounds__(256, 2) vine_lstm_head_train_kernel(const Vine
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int64_t warp0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5, nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
   const uint8_t* P = reinterpret_cast<const uint8_t*>(a.params);
-  for (int i = threadIdx.x; i < 5 * 64; i += blockDim.x) {
+  for (int i = (NO_LN ? 2 * 64 : 0) + threadIdx.x; i < 5 * 64; i += blockDim.x) {
     const int arr = i / 64, r = i % 64, l = r >> 1, half = r & 1;
     const float* src = arr == 0 ? reinterpret_cast<const float*>(P + LP_LNG)
                      : arr == 1 ? reinterpret_cast<const float*>(P + LP_LNB)
@@ -433,36 +445,39 @@ __global__ void __launch_bounds__(256, 2) vine_lstm_head_train_kernel(const Vine
         const float2 f = unpack_bf16(hw[k]);
         yh[r][2 * k] = f.x, yh[r][2 * k + 1] = f.y;
       }
-      mean[r] = ((yh[r][0] + yh[r][1]) + (yh[r][2] + yh[r][3])) + ((yh[r][4] + yh[r][5]) + (yh[r][6] + yh[r][7]));
+      if (!NO_LN) mean[r] = ((yh[r][0] + yh[r][1]) + (yh[r][2] + yh[r][3])) + ((yh[r][4] + yh[r][5]) + (yh[r][6] + yh[r][7]));
     }
+    if (!NO_LN) {
 #pragma unroll
-    for (int o = 16; o > 0; o >>= 1)
+      for (int o = 16; o > 0; o >>= 1)
 #pragma unroll
-      for (int r = 0; r < HT_ROWS; ++r) mean[r] += __shfl_xor_sync(0xffffffffu, mean[r], o);
+        for (int r = 0; r < HT_ROWS; ++r) mean[r] += __shfl_xor_sync(0xffffffffu, mean[r], o);
 #pragma unroll
-    for (int r = 0; r < HT_ROWS; ++r) {
-      mean[r] *= (1.f / HID);
-      float t[8];
+      for (int r = 0; r < HT_ROWS; ++r) {
+        mean[r] *= (1.f / HID);
+        float t[8];
 #pragma unroll
-      for (int k = 0; k < 8; ++k) yh[r][k] -= mean[r], t[k] = yh[r][k] * yh[r][k];
-      sq[r] = ((t[0] + t[1]) + (t[2] + t[3])) + ((t[4] + t[5]) + (t[6] + t[7]));
+        for (int k = 0; k < 8; ++k) yh[r][k] -= mean[r], t[k] = yh[r][k] * yh[r][k];
+        sq[r] = ((t[0] + t[1]) + (t[2] + t[3])) + ((t[4] + t[5]) + (t[6] + t[7]));
+      }
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1)
+#pragma unroll
+        for (int r = 0; r < HT_ROWS; ++r) sq[r] += __shfl_xor_sync(0xffffffffu, sq[r], o);
     }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1)
-#pragma unroll
-      for (int r = 0; r < HT_ROWS; ++r) sq[r] += __shfl_xor_sync(0xffffffffu, sq[r], o);
     float d[HT_ROWS][3];
     {
       float g[8], b[8], w0[8], w1[8], w2[8];
-      load8(0, g), load8(1, b), load8(2, w0), load8(3, w1), load8(4, w2);
+      if (!NO_LN) load8(0, g), load8(1, b);
+      load8(2, w0), load8(3, w1), load8(4, w2);
 #pragma unroll
       for (int r = 0; r < HT_ROWS; ++r) {
-        rstd[r] = rsqrtf(sq[r] * (1.f / HID) + 1e-5f);   // torch.nn.LayerNorm: biased variance, eps 1e-5
+        if (!NO_LN) rstd[r] = rsqrtf(sq[r] * (1.f / HID) + 1e-5f);   // torch.nn.LayerNorm: biased variance, eps 1e-5
         d[r][0] = d[r][1] = d[r][2] = 0.f;
 #pragma unroll
         for (int k = 0; k < 8; ++k) {
-          yh[r][k] *= rstd[r];
-          const float y = fmaf(yh[r][k], g[k], b[k]);
+          if (!NO_LN) yh[r][k] *= rstd[r];
+          const float y = NO_LN ? yh[r][k] : fmaf(yh[r][k], g[k], b[k]);   // the same order as vine_lstm_head_kernel
           d[r][0] = fmaf(y, w0[k], d[r][0]), d[r][1] = fmaf(y, w1[k], d[r][1]), d[r][2] = fmaf(y, w2[k], d[r][2]);
         }
       }
@@ -522,7 +537,8 @@ __global__ void __launch_bounds__(256, 2) vine_lstm_head_train_kernel(const Vine
     float dyh[HT_ROWS][8], s1[HT_ROWS], s2[HT_ROWS];
     {
       float g[8], w0[8], w1[8], w2[8];
-      load8(0, g), load8(2, w0), load8(3, w1), load8(4, w2);
+      if (!NO_LN) load8(0, g);
+      load8(2, w0), load8(3, w1), load8(4, w2);
 #pragma unroll
       for (int r = 0; r < HT_ROWS; ++r) {
         s1[r] = s2[r] = 0.f;
@@ -532,26 +548,29 @@ __global__ void __launch_bounds__(256, 2) vine_lstm_head_train_kernel(const Vine
           A[0][k] = fmaf(gr[r][0], yh[r][k], A[0][k]);
           A[1][k] = fmaf(gr[r][1], yh[r][k], A[1][k]);
           A[2][k] = fmaf(gr[r][2], yh[r][k], A[2][k]);
-          dyh[r][k] = dy * g[k];
-          s1[r] += dyh[r][k], s2[r] = fmaf(dyh[r][k], yh[r][k], s2[r]);
+          dyh[r][k] = NO_LN ? dy : dy * g[k];
+          if (!NO_LN) s1[r] += dyh[r][k], s2[r] = fmaf(dyh[r][k], yh[r][k], s2[r]);
         }
       }
     }
+    if (!NO_LN) {
 #pragma unroll
-    for (int o = 16; o > 0; o >>= 1)
+      for (int o = 16; o > 0; o >>= 1)
 #pragma unroll
-      for (int r = 0; r < HT_ROWS; ++r) {
-        s1[r] += __shfl_xor_sync(0xffffffffu, s1[r], o);
-        s2[r] += __shfl_xor_sync(0xffffffffu, s2[r], o);
-      }
+        for (int r = 0; r < HT_ROWS; ++r) {
+          s1[r] += __shfl_xor_sync(0xffffffffu, s1[r], o);
+          s2[r] += __shfl_xor_sync(0xffffffffu, s2[r], o);
+        }
+    }
 #pragma unroll
     for (int r = 0; r < HT_ROWS; ++r) {
       const float mean1 = s1[r] * (1.f / HID), mean2 = s2[r] * (1.f / HID);
       uint32_t o[4];
 #pragma unroll
       for (int k = 0; k < 4; ++k)
-        o[k] = pack_bf16(rstd[r] * (dyh[r][2 * k] - mean1 - yh[r][2 * k] * mean2),
-                         rstd[r] * (dyh[r][2 * k + 1] - mean1 - yh[r][2 * k + 1] * mean2));
+        o[k] = NO_LN ? pack_bf16(dyh[r][2 * k], dyh[r][2 * k + 1])
+                     : pack_bf16(rstd[r] * (dyh[r][2 * k] - mean1 - yh[r][2 * k] * mean2),
+                                 rstd[r] * (dyh[r][2 * k + 1] - mean1 - yh[r][2 * k + 1] * mean2));
       if (ok[r]) *reinterpret_cast<uint4*>(reinterpret_cast<uint8_t*>(a.dh) + off[r]) = make_uint4(o[0], o[1], o[2], o[3]);
       else if (PADDED && s0 + r * nwarps < a.n) {   // padded row: dh = 0 (at its own offset; off[r] is that of the row it computed on)
         const int64_t s = s0 + r * nwarps;
@@ -563,14 +582,21 @@ __global__ void __launch_bounds__(256, 2) vine_lstm_head_train_kernel(const Vine
   }
   // ---- the parameter gradients from the sums: with y = yh g + b and dy = sum_j d_j w_j,
   //        d(gain)[k] = sum_j w_j[k] A_j[k]     d(bias)[k] = sum_j w_j[k] S_j     d(w_j)[k] = g[k] A_j[k] + b[k] S_j
-  //      (S_j = sum_rows d_j = sc[0..2]); the 8 warps of the block take turns on the block's partial in shared memory ----
+  //      (S_j = sum_rows d_j = sc[0..2]); NO_LN: y = h, d(w_j)[k] = A_j[k] and the gain / bias slots keep their 0.
+  //      The 8 warps of the block take turns on the block's partial in shared memory ----
   {
     float g[8], b[8], w0[8], w1[8], w2[8];
-    load8(0, g), load8(1, b), load8(2, w0), load8(3, w1), load8(4, w2);
+    if (!NO_LN) load8(0, g), load8(1, b), load8(2, w0), load8(3, w1), load8(4, w2);
     for (int w = 0; w < 8; ++w) {
       if (warp == w) {
 #pragma unroll
         for (int k = 0; k < 8; ++k) {
+          if (NO_LN) {
+            red[HG_WH + 8 * lane + k] += A[0][k];
+            red[HG_WH + HID + 8 * lane + k] += A[1][k];
+            red[HG_WH + 2 * HID + 8 * lane + k] += A[2][k];
+            continue;
+          }
           red[HG_LNG + 8 * lane + k] += fmaf(w0[k], A[0][k], fmaf(w1[k], A[1][k], w2[k] * A[2][k]));
           red[HG_LNB + 8 * lane + k] += fmaf(w0[k], sc[0], fmaf(w1[k], sc[1], w2[k] * sc[2]));
           red[HG_WH + 8 * lane + k] += fmaf(g[k], A[0][k], b[k] * sc[0]);
@@ -1233,8 +1259,9 @@ int vine_lstm_head_train(const VineLstmHeadTrain* a, void* stream) {
   if (a->step_rows != 0 && a->mu_writeback && a->wb_chunks * a->wb_env_count != a->step_seqs) return VINE_ERR_INVALID_ARG;
   int64_t blocks = (a->n + 7) / 8;
   if (blocks > 296) blocks = 296;   // 2 resident blocks per SM (128 registers per thread), one wave; <= VINE_LSTM_HEAD_GRAD_PARTS
-  if (a->step_rows) vine_launch::launch(vine_lstm_head_train_kernel<true>, (unsigned)blocks, 256, 0, (cudaStream_t)stream, *a);
-  else vine_launch::launch(vine_lstm_head_train_kernel<false>, (unsigned)blocks, 256, 0, (cudaStream_t)stream, *a);
+  static void (*const kernels[4])(const VineLstmHeadTrain) = {vine_lstm_head_train_kernel<false, false>, vine_lstm_head_train_kernel<false, true>,
+                                                              vine_lstm_head_train_kernel<true, false>, vine_lstm_head_train_kernel<true, true>};
+  vine_launch::launch(kernels[2 * (a->step_rows != 0) + (a->no_layer_norm != 0)], (unsigned)blocks, 256, 0, (cudaStream_t)stream, *a);
   return cudaGetLastError() == cudaSuccess ? (int)blocks : VINE_ERR_CUDA;   // number of gradient partials written
 }
 
@@ -1243,8 +1270,9 @@ int vine_lstm_head(const VineLstmHead* a, void* stream) {
   if (a->actions && !a->logstd) return VINE_ERR_INVALID_ARG;
   int64_t blocks = (a->n + 7) / 8;
   if (blocks > 148 * 8) blocks = 148 * 8;
-  if (a->raw_value) vine_launch::launch(vine_lstm_head_kernel<true>, (unsigned)blocks, 256, 0, (cudaStream_t)stream, *a);
-  else vine_launch::launch(vine_lstm_head_kernel<false>, (unsigned)blocks, 256, 0, (cudaStream_t)stream, *a);
+  static void (*const kernels[4])(const VineLstmHead) = {vine_lstm_head_kernel<false, false>, vine_lstm_head_kernel<false, true>,
+                                                        vine_lstm_head_kernel<true, false>, vine_lstm_head_kernel<true, true>};
+  vine_launch::launch(kernels[2 * (a->raw_value != 0) + (a->no_layer_norm != 0)], (unsigned)blocks, 256, 0, (cudaStream_t)stream, *a);
   return cudaGetLastError() == cudaSuccess ? VINE_OK : VINE_ERR_CUDA;
 }
 

@@ -24,8 +24,9 @@ constexpr int OFF_BAR = OFF_END;
 constexpr int ACT_SMEM_BYTES = OFF_BAR + 64;
 constexpr uint32_t VINE_SITE_POLICY = 16;   // Philox "site" of the policy's action noise (env sites: vine_params.h:20)
 
-// RAW_OBS / RAW_VALUE: VinePolicyAct.raw_obs / raw_value (normalize_input / normalize_value off), one instantiation each
-template <bool RAW_OBS, bool RAW_VALUE>
+// RAW_OBS / RAW_VALUE: VinePolicyAct.raw_obs / raw_value (normalize_input / normalize_value off), one instantiation each;
+// U_NO_OBS: VinePolicyAct.u_no_obs (concat_input off: U's observation columns are 0)
+template <bool RAW_OBS, bool RAW_VALUE, bool U_NO_OBS>
 __global__ void __launch_bounds__(THREADS, 1) vine_policy_act_kernel(const VinePolicyAct a) {
   vine_launch::grid_dependency_sync();
   extern __shared__ __align__(1024) uint8_t smem[];
@@ -95,14 +96,16 @@ __global__ void __launch_bounds__(THREADS, 1) vine_policy_act_kernel(const VineP
     fwd_epilogue<H3>(lane_base + half * 32, 32, half * 32, biases + H1 + H2, a3_t, row);
     if (a.u_out) {
       // recurrent network: emit the LSTM input tile U = [h3 (64) | x (32) | 0 (32)] (row-blocked [128 x 128] bf16) and stop;
-      // LayerNorm and the heads follow the LSTM (vine_lstm_step / vine_lstm_head)
+      // LayerNorm and the heads follow the LSTM (vine_lstm_step / vine_lstm_head).  U_NO_OBS: x's columns 0..30 are written
+      // as 0 and only its column 31 (the constant 1 of the gate-bias gradient) is kept
       __syncthreads();   // both column halves of h3 are in shared memory
       uint8_t* ut = reinterpret_cast<uint8_t*>(a.u_out) + (size_t)tile * (TILE * 128 * 2);
 #pragma unroll
       for (int q = half * 8; q < half * 8 + 8; ++q) {
         uint4 v = make_uint4(0u, 0u, 0u, 0u);
         if (q < 8) v = *reinterpret_cast<const uint4*>(a3_t + tile_offset(row, 8 * q, H3));
-        else if (q < 12) v = *reinterpret_cast<const uint4*>(x_t + tile_offset(row, 8 * (q - 8), K1));
+        else if (q < 12 && (!U_NO_OBS || q == 11)) v = *reinterpret_cast<const uint4*>(x_t + tile_offset(row, 8 * (q - 8), K1));
+        if (U_NO_OBS && q == 11) v.x = v.y = v.z = 0u, v.w &= 0xFFFF0000u;   // bf16 columns 88..94 -> 0, column 95 kept
         *reinterpret_cast<uint4*>(ut + tile_offset(row, 8 * q, 128)) = v;
       }
       __syncthreads();   // x / h3 tiles are rewritten by the next tile
@@ -286,10 +289,13 @@ int vine_policy_act(const VinePolicyAct* a, void* stream) {
   if (a->actions && !a->logstd) return VINE_ERR_INVALID_ARG;
   if (!a->actions && !a->mu && !a->value && !a->u_out) return VINE_ERR_INVALID_ARG;
   if (a->u_out && (a->num_obs >= K1 || (((uintptr_t)a->u_out) & 15u))) return VINE_ERR_INVALID_ARG;
+  if (a->u_no_obs && !a->u_out) return VINE_ERR_INVALID_ARG;
   if (a->u_step_rows != 0 && (!a->u_out || a->u_step_rows < 0 || a->u_step_seqs < 1 || a->u_step_seqs > a->u_step_rows))
     return VINE_ERR_INVALID_ARG;
-  static void (*const kernels[4])(const VinePolicyAct) = {vine_policy_act_kernel<false, false>, vine_policy_act_kernel<false, true>,
-                                                          vine_policy_act_kernel<true, false>, vine_policy_act_kernel<true, true>};
+  static void (*const kernels[8])(const VinePolicyAct) = {
+      vine_policy_act_kernel<false, false, false>, vine_policy_act_kernel<false, false, true>, vine_policy_act_kernel<false, true, false>,
+      vine_policy_act_kernel<false, true, true>,   vine_policy_act_kernel<true, false, false>, vine_policy_act_kernel<true, false, true>,
+      vine_policy_act_kernel<true, true, false>,   vine_policy_act_kernel<true, true, true>};
   static int configured = -1;
   int dev = 0, sms = 0;
   if (cudaGetDevice(&dev) != cudaSuccess) return VINE_ERR_CUDA;
@@ -301,7 +307,8 @@ int vine_policy_act(const VinePolicyAct* a, void* stream) {
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   const int64_t ntiles = (a->n + TILE - 1) / TILE;
   const int grid = (int)(ntiles < sms ? ntiles : sms);
-  vine_launch::launch(kernels[2 * (a->raw_obs != 0) + (a->raw_value != 0)], grid, THREADS, ACT_SMEM_BYTES, (cudaStream_t)stream, *a);
+  const int k = 4 * (a->raw_obs != 0) + 2 * (a->raw_value != 0) + (a->u_no_obs != 0);
+  vine_launch::launch(kernels[k], grid, THREADS, ACT_SMEM_BYTES, (cudaStream_t)stream, *a);
   return cudaGetLastError() == cudaSuccess ? VINE_OK : VINE_ERR_CUDA;
 }
 

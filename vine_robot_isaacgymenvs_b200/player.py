@@ -7,7 +7,9 @@ LSTM state between calls -- without rl_games.
 
 Checkpoints: the rl_games layout ``PPOAgent.state_dict`` writes (``model`` -> ``a2c_network.*``, ``running_mean_std.*``).
 A file without ``running_mean_std.*`` comes from a run with ``normalize_input: False``: the policy then acts on the raw
-observations (no mean, std or +-5 clamp), as it did in training.
+observations (no mean, std or +-5 clamp), as it did in training.  The rnn block is read from the file too (``rnn="auto"``):
+rl_games' ``concat_input`` and ``layer_norm`` default to False, so a block written ``{name: lstm, units: 256, layers: 1}``
+has neither the observation columns in ``weight_ih_l0`` nor ``layer_norm.*``.
 Runs wherever torch runs (the robot-side host may have no GPU); on a B200 the batched MLP policy can instead go through
 ``vine_policy_act``.
 """
@@ -22,15 +24,43 @@ class PolicyPlayer:
     def __init__(self, num_obs, num_actions=2, units=(256, 128, 64), rnn="auto", device="cpu", clip_actions=True,
                  normalize_input="auto"):
         """``normalize_input``: "auto" = whether the checkpoint has the input normaliser (``running_mean_std.*``), or the
-        training config's bool (then a file that disagrees is refused)."""
+        training config's bool (then a file that disagrees is refused).  ``rnn``: "auto" = the block the checkpoint holds
+        (``rnn_block``), the training config's ``network.rnn`` dict (then a file that disagrees is refused), or a bool: the
+        reference's block / none."""
         self.device, self.clip_actions, self._rnn_arg = torch.device(device), clip_actions, rnn
         self.num_obs, self.num_actions, self.units = num_obs, num_actions, tuple(units)
         self._norm_arg = normalize_input
         self.model = self.obs_rms = self.states = None
         self.normalize_input = True
 
-    def _build(self, has_rnn):
-        rnn = REFERENCE_RNN if has_rnn else None
+    def rnn_block(self, net):
+        """The rnn block of a checkpoint's network (``net``: its ``a2c_network.*`` entries without the prefix) as rl_games'
+        ``network.rnn``, or None when it has none: ``units`` from ``weight_hh_l0``'s width, ``concat_input`` from
+        ``weight_ih_l0``'s (mlp ``units[-1] + num_obs`` or ``units[-1]``), ``layer_norm`` from whether ``layer_norm.weight``
+        is present."""
+        if "rnn.rnn.weight_hh_l0" not in net:
+            return None
+        d, width = self.units[-1], int(net["rnn.rnn.weight_ih_l0"].shape[1])
+        if width not in (d, d + self.num_obs):
+            raise ValueError(f"the checkpoint's rnn.rnn.weight_ih_l0 has {width} columns: neither the MLP output ({d}) nor it "
+                             f"plus {self.num_obs} observations")
+        return dict(REFERENCE_RNN, units=int(net["rnn.rnn.weight_hh_l0"].shape[1]), concat_input=width == d + self.num_obs,
+                    layer_norm="layer_norm.weight" in net)
+
+    def _rnn_for(self, net):
+        found = self.rnn_block(net)
+        if isinstance(self._rnn_arg, dict):   # the training config's block: it must be the file's (rl_games' defaults: False)
+            arg = self._rnn_arg
+            same = found is not None and str(arg.get("name", "lstm")).lower() == "lstm" and all(
+                bool(arg.get(k, False)) == found[k] for k in ("concat_input", "layer_norm")) and int(arg.get("units", 0)) == found["units"]
+            if not same:
+                raise ValueError(f"rnn={arg} but the checkpoint's rnn block is {found}")
+            return arg
+        if self._rnn_arg == "auto":
+            return found
+        return REFERENCE_RNN if self._rnn_arg else None
+
+    def _build(self, rnn):
         self.model = ActorCritic(self.num_obs, self.num_actions, self.units, rnn=rnn).to(self.device).eval()
         self.obs_rms = RunningMeanStd((self.num_obs,)).to(self.device)
         self.reset()
@@ -38,9 +68,9 @@ class PolicyPlayer:
     def restore(self, fn_or_state):
         ck = torch.load(fn_or_state, map_location=self.device) if isinstance(fn_or_state, (str, bytes)) or hasattr(fn_or_state, "__fspath__") else fn_or_state
         model = ck["model"]
-        has_rnn = any(k.startswith("a2c_network.rnn.") for k in model) if self._rnn_arg == "auto" else bool(self._rnn_arg)
-        self._build(has_rnn)
-        self.model.load_state_dict({k[len("a2c_network."):]: v for k, v in model.items() if k.startswith("a2c_network.")})
+        net = {k[len("a2c_network."):]: v for k, v in model.items() if k.startswith("a2c_network.")}
+        self._build(self._rnn_for(net))
+        self.model.load_state_dict(net)
         rms = {k[len("running_mean_std."):]: v for k, v in model.items() if k.startswith("running_mean_std.")}
         if not rms and "running_mean_std" in ck:          # vine_robot_test_model.py:137-139
             rms = ck["running_mean_std"]

@@ -1,4 +1,5 @@
-"""Host-side orchestration of the kernel-only path for the reference network (MLP -> LSTM 256 -> LayerNorm -> heads):
+"""Host-side orchestration of the kernel-only path for the reference network (MLP -> LSTM 256 -> LayerNorm -> heads, or the
+same block with concat_input and / or layer_norm off):
 which kernel runs when, on which buffers.  All arithmetic is in csrc/ (vine_rollout.cu, vine_lstm_net.cu, vine_ppo.cu);
 this module only owns the HBM buffers (activation tiles, cell states, gradient workspaces) and issues the launches.
 
@@ -33,9 +34,12 @@ class NativeLstmPath:
         gradient."""
         return -(-num_seqs // 128) * 128
 
-    def __init__(self, num_obs, seq_len, num_seqs, device, hyper, wgrad_splits=12):
+    def __init__(self, num_obs, seq_len, num_seqs, device, hyper, wgrad_splits=12, layer_norm=True, concat_input=True):
+        """``layer_norm`` / ``concat_input``: the rnn block's switches (rl_games network.rnn); with concat_input off the LSTM
+        input carries no observation, with layer_norm off the heads act on h."""
         assert num_seqs >= 1
         self.lib = abi.load_library()
+        self.no_layer_norm, self.u_no_obs = int(not layer_norm), int(not concat_input)
         self.O, self.L, self.S, self.dev = num_obs, seq_len, num_seqs, device
         self.R = self.step_rows(num_seqs)
         self.tiles = self.R // 128
@@ -94,7 +98,7 @@ class NativeLstmPath:
         raw_obs = int(obs_mean is None)
         stats = dict(obs_mean=None, obs_inv_std=None) if raw_obs else dict(obs_mean=_ptr(obs_mean), obs_inv_std=_ptr(obs_inv_std))
         act = abi.VinePolicyAct(packed=_ptr(packed_mlp), obs=_ptr(obs), n=n, num_obs=self.O, u_out=_ptr(self.U), u_step_rows=R,
-                                u_step_seqs=S, raw_obs=raw_obs, raw_value=int(value_stats is None),
+                                u_step_seqs=S, raw_obs=raw_obs, raw_value=int(value_stats is None), u_no_obs=self.u_no_obs,
                                 value_stats=_ptr(value_stats) if value_stats is not None else None, **stats)
         assert lib.vine_policy_act(C.byref(act), st) == 0
         for t in range(L):
@@ -110,7 +114,8 @@ class NativeLstmPath:
                                    debug_out=_ptr(debug_out) if debug_out is not None else None, n=n, inv_B=1.0 / (L * S),
                                    step_rows=R if R != S else 0, step_seqs=S,   # 0: no padded rows (the dense kernel)
                                    e_clip=h["e_clip"], critic_coef=h["critic_coef"], entropy_coef=h["entropy_coef"],
-                                   bounds_loss_coef=h["bounds_loss_coef"], value_loss_unclipped=int(not h.get("clip_value", True)))
+                                   bounds_loss_coef=h["bounds_loss_coef"], value_loss_unclipped=int(not h.get("clip_value", True)),
+                                   no_layer_norm=self.no_layer_norm)
         if writeback is not None:
             src, wl, wc, wn, wb, we = writeback
             ht.mu_writeback, ht.wb_seq_len, ht.wb_chunks, ht.wb_num_envs, ht.wb_env_begin, ht.wb_env_count = _ptr(src), wl, wc, wn, wb, we

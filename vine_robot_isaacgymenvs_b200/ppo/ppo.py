@@ -221,6 +221,7 @@ class PPOAgent:
         dev = self.device
         self.model = ActorCritic(self.O, self.A, units, rnn=net.get("rnn")).to(dev)
         self.has_rnn = self.model.has_rnn
+        self.layer_norm = self.has_rnn and isinstance(self.model.layer_norm, nn.LayerNorm)   # rnn.layer_norm
         self.seq_len = int(c.get("seq_len", 4)) if self.has_rnn else 1
         assert self.T % self.seq_len == 0, "horizon_length must be a multiple of seq_len"
         self.obs_rms = RunningMeanStd((self.O,)).to(dev)
@@ -350,9 +351,11 @@ class PPOAgent:
             why.append(f"{self.A} actions (kernels: 2)")
         if self.O > (30 if self.has_rnn else 31):
             why.append(f"{self.O} observations (kernels: <= {30 if self.has_rnn else 31})")
-        if self.has_rnn:
-            if int(rnn_cfg.get("units", 0)) != 256 or not rnn_cfg.get("concat_input") or not rnn_cfg.get("layer_norm"):
-                why.append("network.rnn must be the reference's block: units 256, concat_input True, layer_norm True")
+        if self.has_rnn:   # concat_input and layer_norm may each be on or off
+            if int(rnn_cfg.get("units", 0)) != 256:
+                why.append(f"network.rnn.units {rnn_cfg.get('units')} (kernels are built for an LSTM of 256 units)")
+            if int(rnn_cfg.get("layers", 1)) != 1 or rnn_cfg.get("before_mlp", False):
+                why.append("network.rnn with layers != 1 or before_mlp True (kernels: one LSTM layer after the MLP)")
         return why
 
     def _param_order(self):
@@ -390,10 +393,14 @@ class PPOAgent:
 
     # ------------------------------------------------------------------ reference network on kernels only
     def _lstm_param_order(self):
-        """Flat parameter order of the recurrent half (include/vine_b200.h, vine_lstm_*)."""
+        """Flat parameter order of the recurrent half (include/vine_b200.h, vine_lstm_*): the tensors whose storage is the flat
+        vector.  The layout is the same with either switch of the rnn block off; the slots the torch block then lacks hold
+        tensors of their own that start at 0 and get a gradient of exactly 0, so Adam never moves them: LayerNorm gamma / beta
+        with layer_norm off, and with concat_input off the observation columns of W_ih, whose whole [1024, 64 + O] slot is
+        _lstm_wih (the torch weight_ih_l0 [1024, 64] is its first 64 columns)."""
         m, r = self.model, self.model.rnn.rnn
-        return [r.weight_ih_l0, r.weight_hh_l0, r.bias_ih_l0, r.bias_hh_l0, m.layer_norm.weight, m.layer_norm.bias,
-                m.mu.weight, m.mu.bias, m.value.weight, m.value.bias, m.sigma]
+        return [self._lstm_wih, r.weight_hh_l0, r.bias_ih_l0, r.bias_hh_l0, *self._lstm_ln, m.mu.weight, m.mu.bias,
+                m.value.weight, m.value.bias, m.sigma]
 
     @torch.no_grad()
     def _init_native_lstm(self, lr):
@@ -410,6 +417,9 @@ class PPOAgent:
         for p in mlp + self._mlp_dummy:
             p.data = self.flat[o:o + p.numel()].view_as(p)
             o += p.numel()
+        r, H = m.rnn.rnn, m.rnn_units
+        self._lstm_wih = r.weight_ih_l0 if m.concat_input else torch.cat([r.weight_ih_l0.detach(), z(4 * H, self.O)], 1)
+        self._lstm_ln = [m.layer_norm.weight, m.layer_norm.bias] if self.layer_norm else [z(H), z(H)]
         order = self._lstm_param_order()
         self.flat_l = torch.cat([p.detach().reshape(-1) for p in order]).contiguous()
         assert self.flat_l.numel() == lib.vine_lstm_num_params(self.O)
@@ -417,6 +427,8 @@ class PPOAgent:
         for p in order:
             p.data = self.flat_l[o:o + p.numel()].view_as(p)
             o += p.numel()
+        if not m.concat_input:   # the torch weight: a strided view of the MLP columns of the flat W_ih
+            r.weight_ih_l0.data = self._lstm_wih[:, :r.input_size]
         self.adam_m, self.adam_v = torch.zeros_like(self.flat), torch.zeros_like(self.flat)
         self.adam_ml, self.adam_vl = torch.zeros_like(self.flat_l), torch.zeros_like(self.flat_l)
         self.ppo_state = torch.zeros(abi.PPO_STATE_FLOATS, device=dev)
@@ -433,7 +445,8 @@ class PPOAgent:
         L, chunks, tiles_n = self.seq_len, self.T // self.seq_len, -(-self.n // 128)
         hyper = dict(e_clip=self.e_clip, critic_coef=self.critic_coef, entropy_coef=self.entropy_coef,
                      bounds_loss_coef=self.bounds_coef, clip_value=self.clip_value, schedule=self._schedule_fields)
-        self._path = NativeLstmPath(self.O, L, chunks * self.mb_envs, dev, hyper)
+        self._path = NativeLstmPath(self.O, L, chunks * self.mb_envs, dev, hyper, layer_norm=self.layer_norm,
+                                    concat_input=m.concat_input)
         from .lstm_native import TB
         bf = lambda *s: torch.zeros(*s, dtype=torch.bfloat16, device=dev)  # noqa: E731
         self._r_U, self._r_HM = bf(tiles_n, TB), bf(tiles_n, 2, TB)
@@ -455,7 +468,8 @@ class PPOAgent:
         ptr = lambda x: x.data_ptr()  # noqa: E731
         stream = C.c_void_p(torch.cuda.current_stream().cuda_stream)
         common = dict(packed=ptr(self._packed), obs=ptr(env._obs_clamped), n=n, num_obs=self.O, **self._stat_ptrs(),
-                      **self._raw_flags)
+                      **self._raw_flags, u_no_obs=int(not self.model.concat_input))
+        no_ln = int(not self.layer_norm)
         seed, goff = int(env._seed) ^ 0x5DEECE66D, int(env._global_env_offset)
         vstats = common["value_stats"]
         self._done_ext[0].copy_(self._done_ext[T])
@@ -475,14 +489,15 @@ class PPOAgent:
             assert lib.vine_lstm_step(C.byref(st), stream) == 0
             if last:   # bootstrap value of the final observation: the persistent state is NOT advanced
                 hd = abi.VineLstmHead(params=ptr(self._lpacked), hh=ptr(self._r_HH[nxt]), value_stats=vstats,
-                                      value=ptr(self.last_value), n=n, raw_value=self._raw_flags["raw_value"])
+                                      value=ptr(self.last_value), n=n, raw_value=self._raw_flags["raw_value"],
+                                      no_layer_norm=no_ln)
                 assert lib.vine_lstm_head(C.byref(hd), stream) == 0
                 break
             hd = abi.VineLstmHead(params=ptr(self._lpacked), hh=ptr(self._r_HH[nxt]), value_stats=vstats,
                                   mu=ptr(self.b_mu[t]), value=ptr(self.b_val[t]), logstd=ptr(self.model.sigma),
                                   rng_counter=ptr(self._rng_counter), actions=ptr(self.b_act[t]), neglogp=ptr(self.b_nlp[t]),
                                   env_actions=ptr(env.actions), n=n, seed=seed, global_env_offset=goff,
-                                  raw_value=self._raw_flags["raw_value"])
+                                  raw_value=self._raw_flags["raw_value"], no_layer_norm=no_ln)
             assert lib.vine_lstm_head(C.byref(hd), stream) == 0
             self._r_cur = nxt
             env.step_device()
@@ -550,7 +565,9 @@ class PPOAgent:
     def _clip_and_adam_native_lstm(self, path, sc, pm, pl, stream):
         """truncate_grads: ONE norm over both gradient vectors (the MLP half without its unused head slots, the whole
         recurrent half), then both Adam launches with the coefficient.  With peer memory the clip kernel consumes both
-        channels and leaves the rank sums in flat_g_*, so Adam runs without a channel."""
+        channels and leaves the rank sums in flat_g_*, so Adam runs without a channel.  The norm is that of exactly
+        ActorCritic's parameters with either rnn switch off too: the recurrent slots the block then lacks (W_ih's observation
+        columns, LayerNorm gamma / beta; _lstm_param_order) carry a gradient of exactly 0."""
         lib = self._lib
         p = lambda x: C.c_void_p(x.data_ptr())  # noqa: E731
         P, PL = path.P_mlp, path.P_lstm
